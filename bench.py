@@ -2,6 +2,7 @@
 """bench.py -- forward splat-render benchmark (BASELINE.json metric) on N B200s of one node.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config C1|C2|C3|C4|C5] [--shard views|rows]
+                    [--dump-outputs DIR]
 
 Workloads (BASELINE.json:configs; synthetic scenes of SURVEY.md 8d, the release .ply files are not available offline):
 
@@ -35,6 +36,7 @@ One JSON line on rank 0:
 from __future__ import annotations
 
 import argparse
+import atexit
 import json
 import os
 import subprocess
@@ -69,7 +71,14 @@ def parse_args():
     ap.add_argument("--deliver", default="rgb8", choices=["rgb8", "float"],
                     help="sharded workloads: what a rank writes into rank 0's ring -- rgb8: the app's final uint8 HWC image (3 B/pixel over "
                          "NVLink, the float image stays local); float: the planar float32 image as well (15 B/pixel)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed as DIR/<name>.npy (float32 or float64, %d MB at most in all; "
+                         "larger outputs as a seeded sample, see DIR/manifest.json) to compare two builds" % (DUMP_BUDGET_BYTES // 10**6))
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl b200)")
     return args
 
 
@@ -203,6 +212,79 @@ def run_reference(args):
 
 
 # ------------------------------------------------------------------------------------------------
+# --dump-outputs: what the last timed step computed, so that two builds can be compared output for output
+# ------------------------------------------------------------------------------------------------
+
+DUMP_BUDGET_BYTES = 64 * 10**6
+DUMP_SEED = 0
+
+
+def capture_frame(r, n, img=True, rgb8=True):
+    """Device copies of the frame `r` has just rendered, as its caller receives it: num_rendered, the planar image, the
+    uint8 image and the frame buffers of app/main.cpp:232-254 except the two unsorted instance lists (the sort's
+    input).  Returns name -> (array, numpy dtype of its elements)."""
+    import torch
+
+    f32, u32 = np.float32, np.uint32
+    bufs = {"depth": (r.depth, f32), "radii": (r.radii, np.int32), "tiles_touched": (r.tiles_touched, u32),
+            "offsets": (r.point_offsets, u32), "keys_sorted": (r.keys[:n], np.uint64), "vals_sorted": (r.vals[:n], u32),
+            "ranges": (r.ranges[:2 * r.num_tiles].view(-1, 2), u32)}
+    if img:
+        bufs["img"] = (r.img.view(3, r.H, r.W), f32)
+    if rgb8 and r.rgb8 is not None:
+        bufs["rgb8"] = (r.rgb8.view(r.H, r.W, 3), np.uint8)
+    if r.conic is not None:
+        bufs.update(means_2d=(r.means_2d.view(-1, 2), f32), conic=(r.conic.view(-1, 3), f32), color=(r.color.view(-1, 3), f32))
+    out = {k: (t.clone(), dt) for k, (t, dt) in bufs.items()}
+    out["num_rendered"] = (torch.tensor([n], dtype=torch.int64), np.int64)
+    return out
+
+
+def read_device(dev, ptr, shape, dtype):
+    """Host copy of device memory at `ptr` (a ring slot, which may live on another GPU)."""
+    out = np.empty(shape, dtype)
+    dev.check(dev.lib.lcgs_b200_peer_read(dev.ctx, ptr, out.ctypes.data, out.nbytes))
+    return out
+
+
+def write_outputs(out_dir, arrays):
+    """out_dir/<name>.npy for each captured array: float32 for float32 and uint8 data, float64 for integers (checked
+    exact).  If the set exceeds DUMP_BUDGET_BYTES, the arrays that do not fit an equal share of what is left keep the
+    elements at sorted, seeded random flat indices -- the same indices for the same array size on every run.
+    out_dir/manifest.json records each array's source shape and dtype and how it was sampled."""
+    os.makedirs(out_dir, exist_ok=True)
+    host = {}
+    for name, (a, dt) in arrays.items():
+        host[name] = (a if isinstance(a, np.ndarray) else a.cpu().numpy()).view(dt)
+    size_of = lambda a: 4 if a.dtype in (np.float32, np.uint8) else 8  # noqa: E731  stored bytes per element
+    budget = DUMP_BUDGET_BYTES - 2**20                                    # headroom for the .npy headers and the manifest
+    left = len(host)
+    manifest = {}
+    for name, a in sorted(host.items(), key=lambda kv: (kv[1].size * size_of(kv[1]), kv[0])):
+        share = budget // left
+        entry = {"shape": list(a.shape), "dtype": str(a.dtype), "sample": None}
+        if a.size * size_of(a) > share:
+            k = share // size_of(a)
+            idx = np.sort(np.random.default_rng(DUMP_SEED).choice(a.size, k, replace=False))
+            a = a.reshape(-1)[idx]
+            entry["sample"] = {"count": int(k), "seed": DUMP_SEED,
+                               "indices": "np.sort(np.random.default_rng(seed).choice(size, count, replace=False)) into the C-order flattened array"}
+        if size_of(a) == 4:
+            out = a.astype(np.float32)
+        else:
+            out = a.astype(np.float64)
+            if not np.array_equal(out.astype(a.dtype), a):
+                raise ValueError("%s: integer values beyond float64's exact range" % name)
+        budget -= out.nbytes
+        left -= 1
+        entry["stored"] = str(out.dtype)
+        manifest[name] = entry
+        np.save(os.path.join(out_dir, name + ".npy"), out)
+    with open(os.path.join(out_dir, "manifest.json"), "w") as fh:
+        json.dump(manifest, fh, indent=1, sort_keys=True)
+
+
+# ------------------------------------------------------------------------------------------------
 # clocks
 # ------------------------------------------------------------------------------------------------
 
@@ -221,6 +303,7 @@ class ClockSampler:
             self.p = subprocess.Popen(["nvidia-smi", "-i", str(self.index), "--query-gpu=" + self.Q,
                                        "--format=csv,noheader,nounits", "-lms", "100"], stdout=self.f,
                                       stderr=subprocess.DEVNULL)
+            atexit.register(self.p.kill)   # a run that fails before stop() must not leave the sampler behind
         except Exception:
             self.p = None
 
@@ -289,6 +372,7 @@ class Bench:
         resolve_workload(args, self.world)
         self.dev = lcgs.Device(self.local)
         self.launches = 0
+        self.outputs = None   # --dump-outputs: capture of the last timed step (rank 0)
 
     # -- helpers ------------------------------------------------------------------------------
     def barrier(self):
@@ -374,6 +458,8 @@ class Bench:
         torch.cuda.synchronize()
         ms_total = float(ev0.elapsed_time(ev1))
         self.launches += KERNELS_PER_FRAME * args.steps
+        if args.dump_outputs:
+            self.outputs = capture_frame(r, dev.num_rendered())
 
         stage_ms, sort_acc = self.stage_profile(r, [vp], max(3, min(args.steps, 10)))
         clock_info = clocks.stop()
@@ -617,6 +703,14 @@ class Bench:
         ev1.record(render_stream)
         evc.record(consume_stream)
         self.barrier()
+        if args.dump_outputs and rank == 0 and not as_leg:
+            # rank 0's own last view (its float image stays local unless delivered) and every view of the last step as delivered
+            self.outputs = capture_frame(r, dev.num_rendered(), img=not fl, rgb8=False)
+            for w in range(world):
+                sl, f = ((gstep[0] - 1) % SLOTS) * world + w, (steps - 1) * world + w
+                self.outputs["rgb8_frame%d" % f] = (read_device(dev, ring.rgb8_ptr(sl), (H, W, 3), np.uint8), np.uint8)
+                if fl:
+                    self.outputs["img_frame%d" % f] = (read_device(dev, ring.ptr(sl), (3, H, W), np.float32), np.float32)
         ms = float(ev0.elapsed_time(ev1))
         per_rank_render_ms = self.gather_counts(ms / steps)
         consumer_ms = float(ev0.elapsed_time(evc)) / steps if rank == 0 else None
@@ -835,6 +929,13 @@ class Bench:
         ev1.record(render_stream)
         evc.record(consume_stream)
         self.barrier()
+        if args.dump_outputs and rank == 0:
+            # rank 0's band (its float image stays local unless delivered) and the assembled frame of the last step
+            self.outputs = capture_frame(r, dev.num_rendered(), img=not fl, rgb8=False)
+            sl = (gstep[0] - 1) % SLOTS
+            self.outputs["rgb8_frame"] = (read_device(dev, ring.rgb8_ptr(sl), (H, W, 3), np.uint8), np.uint8)
+            if fl:
+                self.outputs["img_frame"] = (read_device(dev, ring.ptr(sl), (3, H, W), np.float32), np.float32)
         ms = float(ev0.elapsed_time(ev1))
         per_rank_ms = self.gather_counts(ms / steps)
         if rank == 0:
@@ -984,6 +1085,8 @@ def run_b200(args):
             line = b.run_single()
         if b.rank == 0 and line is not None:
             print(json.dumps(line), flush=True)
+        if b.outputs is not None:
+            write_outputs(args.dump_outputs, b.outputs)
     finally:
         b.close()
     return 0

@@ -71,7 +71,7 @@ class MemmapRing:
         dist.barrier()
 
 
-def _worker(rank, world, port, mode, q):
+def _worker(rank, world, port, mode, q, ring_path):
     os.environ["MASTER_ADDR"] = "127.0.0.1"
     os.environ["MASTER_PORT"] = str(port)
     dist.init_process_group("gloo", rank=rank, world_size=world)
@@ -80,7 +80,7 @@ def _worker(rank, world, port, mode, q):
         if mode == "rows_empty_band":
             # the last rank owns only the last tile row, which is never binned (Q1): its band has 0 instances and must
             # still overwrite the stale pixels of the slot with the background
-            ring = MemmapRing("/tmp/lcgs_ring_%d.bin" % port, slots=2)
+            ring = MemmapRing(ring_path, slots=2)
             if rank == 0:
                 ring.mem[1][:] = -7.0
             dist.barrier()
@@ -98,7 +98,7 @@ def _worker(rank, world, port, mode, q):
             if rank == 0:
                 q.put((img, bands))
         elif mode in ("views_peer", "rows_peer"):
-            ring = MemmapRing("/tmp/lcgs_ring_%d.bin" % port, slots=5)
+            ring = MemmapRing(ring_path, slots=5)
             if mode == "views_peer":
                 out = D.render_sweep_view_sharded_peer(
                     lambda k, ptr: ring.write(ptr, _frame(sc, scenes.orbit_pose(k * 13)).img), 5, ring)
@@ -128,11 +128,11 @@ def _worker(rank, world, port, mode, q):
         dist.destroy_process_group()
 
 
-def _run(mode, world=2):
+def _run(mode, ring_path=None, world=2):
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
     port = _free_port()
-    procs = [ctx.Process(target=_worker, args=(r, world, port, mode, q)) for r in range(world)]
+    procs = [ctx.Process(target=_worker, args=(r, world, port, mode, q, ring_path)) for r in range(world)]
     for p in procs:
         p.start()
     res = q.get(timeout=240)
@@ -159,23 +159,23 @@ def test_tile_row_sharded_frame_equals_single_device_frame(mode):
     assert np.array_equal(img.view(np.uint32), want.view(np.uint32))
 
 
-def test_peer_drivers_assemble_the_same_frames():
+def test_peer_drivers_assemble_the_same_frames(tmp_path):
     """The drivers of the gather-fused-into-the-render path (every rank writes straight into the destination's
     buffer; on a GPU box that buffer is peer-mapped device memory, here a shared file)."""
-    frames = _run("views_peer")
+    frames = _run("views_peer", str(tmp_path / "views_ring.bin"))
     sc = _scene()
     assert len(frames) == 5
     for k, f in enumerate(frames):
         want = _frame(sc, scenes.orbit_pose(k * 13)).img
         assert np.array_equal(f.view(np.uint32), want.view(np.uint32)), k
-    img, bands = _run("rows_peer")
+    img, bands = _run("rows_peer", str(tmp_path / "rows_ring.bin"))
     want = _frame(sc, (scenes.CAM_POS, scenes.CAM_TARGET, scenes.WORLD_UP_COLMAP)).img
     assert bands[0][0] == 0 and bands[-1][1] == (H + 15) // 16
     assert np.array_equal(img.view(np.uint32), want.view(np.uint32))
 
 
-def test_a_band_without_instances_still_writes_the_background():
-    img, bands = _run("rows_empty_band")
+def test_a_band_without_instances_still_writes_the_background(tmp_path):
+    img, bands = _run("rows_empty_band", str(tmp_path / "ring.bin"))
     sc = _scene()
     vp = orc.view_params(orc.make_camera(scenes.CAM_POS, scenes.CAM_TARGET, scenes.WORLD_UP_COLMAP, W, H))
     want = orc.forward(sc.pos, sc.scale, sc.rotq, sc.sh, sc.opacity, vp, bg=(0.25, 0.5, 0.75))

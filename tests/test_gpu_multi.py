@@ -24,7 +24,7 @@ def _gpus():
         return 0
 
 
-pytestmark = [pytest.mark.gpu_multi, pytest.mark.skipif(_gpus() < 2, reason="needs >= 2 GPUs on one node")]
+pytestmark = [pytest.mark.gpu, pytest.mark.gpu_multi, pytest.mark.skipif(_gpus() < 2, reason="needs >= 2 GPUs on one node")]
 
 
 def _run(extra, port, timeout=900):
