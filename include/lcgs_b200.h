@@ -126,6 +126,20 @@ typedef struct lcgs_b200_frame {
      * (app/main.cpp:322-337): interleaved HWC uint8 [H][W][3], vertically flipped (row i = image row
      * H-1-i), uint8(v * 255) with truncation.  4x fewer bytes to read back than target_img. */
     uint8_t* target_rgb8;
+    /* extension, optional (NULL = off; each plane on its own): per-pixel outputs of the blend, [H][W] in the row order
+     * of target_img (not flipped), 4-byte aligned.  For a pixel whose front-to-back walk blends Gaussians i = 1..n with
+     * weights w_i = T_i * alpha_i and ends with transmittance T (the factor of the background):
+     *   target_alpha     = 1 - T                       (accumulated opacity)
+     *   target_depth     = sum of w_i * depth[i]       (view depth, in blend order, not normalised: the expected
+     *                                                   depth is target_depth / target_alpha where alpha > 0)
+     *   target_n_contrib = n                           (pairs blended; entries skipped by the alpha test and the
+     *                                                   entry that saturates the pixel are not counted)
+     * Pixels no Gaussian reaches get 0.  A band of tile rows writes its own rows of these full-frame planes.  On an
+     * empty whole frame (num_rendered == 0) the image is left untouched, but the planes are written as zeros.
+     * Honoured by lcgs_b200_render and lcgs_b200_splat_forward. */
+    float*    target_alpha;
+    float*    target_depth;
+    uint32_t* target_n_contrib;
 } lcgs_b200_frame;
 
 /* ---- library / context ------------------------------------------------------------------- */

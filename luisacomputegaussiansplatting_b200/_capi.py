@@ -52,7 +52,8 @@ class Frame(C.Structure):
                 ("point_list_unsorted", C.c_void_p), ("point_list_keys", C.c_void_p), ("point_list", C.c_void_p),
                 ("ranges", C.c_void_p), ("list_capacity", C.c_size_t), ("target_img", C.c_void_p),
                 ("radii", C.c_void_p), ("tile_row_begin", C.c_int), ("tile_row_end", C.c_int),
-                ("target_rgb8", C.c_void_p)]
+                ("target_rgb8", C.c_void_p), ("target_alpha", C.c_void_p), ("target_depth", C.c_void_p),
+                ("target_n_contrib", C.c_void_p)]
 
 
 PEER_HANDLE_BYTES = 64

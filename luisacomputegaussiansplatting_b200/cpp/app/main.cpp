@@ -8,7 +8,8 @@
 // (main.cpp:322-339) -- in the fused path that conversion is the blend kernel's epilogue, so 3 bytes per
 // pixel cross PCIe instead of 12.  The camera pose is the reference's hard-coded one (main.cpp:191-202).
 // Extensions: --dump <dir> writes the frame's raw buffers, --fused 0 drives the three reference
-// entry points separately instead of the fused frame call, --capacity sets the instance list size L.
+// entry points separately instead of the fused frame call, --capacity sets the instance list size L,
+// --aux 1 also renders the per-pixel alpha / depth / contributor-count planes (written by --dump).
 // --display (ImGui viewer) is out of scope and rejected.
 #include <chrono>
 #include <cstring>
@@ -90,7 +91,7 @@ int main(int argc, char** argv)
     unsigned    res_w = 1600, res_h = 1063;
     fs::path    ply_path = "gsplat.ply";
     std::string backend = "dx", out_dir = "out", world = "colmap", dump_dir;
-    int         exp_N = 1, fused = 1;
+    int         exp_N = 1, fused = 1, aux = 0;
     long        capacity = 20000000;  // max num rendered (main.cpp:245)
 
     Handlers cmds;
@@ -105,7 +106,9 @@ int main(int argc, char** argv)
                     "  --exp_N <N>              Number of frames to render (default: %d)\n"
                     "  --capacity <L>           Instance list capacity (default: %ld)\n"
                     "  --fused <0|1>            1: fused frame call, 0: SHProcessor/GSProjector/GSTileSplatter (default 1)\n"
-                    "  --dump <dir>             Write raw frame buffers for inspection\n",
+                    "  --dump <dir>             Write raw frame buffers for inspection\n"
+                    "  --aux <0|1>              1: also render per-pixel alpha, depth and contributor count\n"
+                    "                           (alpha.f32, depth_map.f32, n_contrib.u32 under --dump; default 0)\n",
                     argv[0], res_w, res_h, backend.c_str(), out_dir.c_str(), exp_N, capacity);
         std::exit(0);
     };
@@ -136,7 +139,12 @@ int main(int argc, char** argv)
     cmds["capacity"] = [&](const std::string& s) { capacity = std::stol(s); };
     cmds["fused"]    = [&](const std::string& s) { fused = s.empty() ? 1 : std::stoi(s); };
     cmds["dump"]     = [&](const std::string& s) { dump_dir = s; };
+    cmds["aux"]      = [&](const std::string& s) { aux = s.empty() ? 1 : std::stoi(s); };
     parse_command(cmds, argc, argv);
+    if (aux && dump_dir.empty()) {
+        std::fprintf(stderr, "[lcgs-app] --aux 1 needs --dump <dir>: the aux planes are only written there\n");
+        return 2;
+    }
 
     std::string ply_name = ply_path.filename().string();
     {
@@ -217,9 +225,17 @@ int main(int argc, char** argv)
     auto d_ranges         = device.create_buffer<lcgs::uint>((size_t)tw * th * 2);
     auto d_img            = device.create_buffer<float>((size_t)w * h * 3);
     auto d_radii          = device.create_buffer<int>((size_t)P);
+    auto d_alpha          = device.create_buffer<float>(aux ? (size_t)w * h : 1);
+    auto d_depth_map      = device.create_buffer<float>(aux ? (size_t)w * h : 1);
+    auto d_n_contrib      = device.create_buffer<lcgs::uint>(aux ? (size_t)w * h : 1);
     device.check(lcgs_b200_ctx_reserve(device.ctx(), P, L), "reserve");
 
     lcgs::GSSplatForwardOutputProxy output{ h, w, d_img, d_radii };
+    if (aux) {
+        output.target_alpha     = d_alpha.view();
+        output.target_depth     = d_depth_map.view();
+        output.target_n_contrib = d_n_contrib.view();
+    }
     lcgs::GSTileSplatterAccelProxy  accel{ d_tiles_touched, d_points_offset, d_keys_unsorted, d_list_unsorted,
                                           d_keys,          d_list,          d_ranges };
     lcgs::GSTileSplatterInputProxy  input{ P, bg_color, d_means_2d, d_depth_features, d_covs_2d, d_color, d_opacity };
@@ -245,6 +261,11 @@ int main(int argc, char** argv)
     frame.target_img = d_img.view().ptr; frame.radii = d_radii.view().ptr;
     frame.tile_row_begin = 0; frame.tile_row_end = -1;
     frame.target_rgb8 = fused ? d_rgb8.view().ptr : nullptr;
+    if (aux) {
+        frame.target_alpha     = d_alpha.view().ptr;
+        frame.target_depth     = d_depth_map.view().ptr;
+        frame.target_n_contrib = d_n_contrib.view().ptr;
+    }
 
     lcgs::CommandList cmd_list;
     int               num_rendered = 0;
@@ -302,6 +323,11 @@ int main(int argc, char** argv)
         dump(d, "keys_sorted.u64", stream, d_keys.view(), n);
         dump(d, "vals_sorted.u32", stream, d_list.view(), n);
         dump(d, "ranges.u32", stream, d_ranges.view(), (size_t)tw * th * 2);
+        if (aux) {
+            dump(d, "alpha.f32", stream, d_alpha.view(), (size_t)w * h);
+            dump(d, "depth_map.f32", stream, d_depth_map.view(), (size_t)w * h);
+            dump(d, "n_contrib.u32", stream, d_n_contrib.view(), (size_t)w * h);
+        }
         std::ofstream meta(d / "meta.txt");
         meta << "P " << P << "\nW " << w << "\nH " << h << "\nnum_rendered " << num_rendered << "\n";
     }

@@ -52,6 +52,8 @@ public:
         if (accel.point_list.count < cap) cap = accel.point_list.count;
         f.list_capacity = cap;
         f.target_img = output.target_img.ptr; f.radii = output.radii.ptr;
+        f.target_alpha = output.target_alpha.ptr; f.target_depth = output.target_depth.ptr;
+        f.target_n_contrib = output.target_n_contrib.ptr;
         f.tile_row_begin = 0; f.tile_row_end = -1;
         device.check(lcgs_b200_splat_forward(device.ctx(), input.num_gaussians, input.opacity_features.ptr, &f, stream.abi()),
                      "GSTileSplatter::forward");

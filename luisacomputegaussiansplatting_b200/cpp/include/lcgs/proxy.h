@@ -32,6 +32,10 @@ struct GSSplatForwardOutputProxy {
     int               width;
     BufferView<float> target_img;  // planar CHW
     BufferView<int>   radii;       // P
+    // extension, optional (empty = off): per-pixel [H][W] planes, see lcgs_b200_frame::target_alpha
+    BufferView<float> target_alpha;      // 1 - T
+    BufferView<float> target_depth;      // sum of w_i * depth_i (not normalised)
+    BufferView<uint>  target_n_contrib;  // Gaussians blended into the pixel
 };
 
 }  // namespace lcgs

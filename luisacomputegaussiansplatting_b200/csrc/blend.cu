@@ -381,6 +381,10 @@ __device__ __forceinline__ void cp_async_16(uint32_t smem_addr, const void* gptr
 {
     asm volatile("cp.async.ca.shared.global [%0], [%1], 16;" ::"r"(smem_addr), "l"(gptr) : "memory");
 }
+__device__ __forceinline__ void cp_async_4(uint32_t smem_addr, const void* gptr)
+{
+    asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(smem_addr), "l"(gptr) : "memory");
+}
 __device__ __forceinline__ void cp_async_wait_all2() { asm volatile("cp.async.commit_group;\ncp.async.wait_group 0;" ::: "memory"); }
 // index of the highest set bit (FLO), x != 0
 __device__ __forceinline__ int top_bit(unsigned x)
@@ -398,25 +402,35 @@ __device__ __forceinline__ int top_bit(unsigned x)
 // MODE 2 (CPT = 1): as MODE 1, and the records never pass through registers: each thread copies its candidate's three
 //         16-byte planes global -> shared with cp.async (LDGSTS) straight into its slot of the next round's buffer,
 //         waited for before the round's barrier.
-template <int MIN_CTAS, int CPT, int MODE = 0>
-__global__ void __launch_bounds__(kB2Threads, MIN_CTAS)
-    blend2_kernel(int W, int H, uint32_t gx, uint32_t row0, float bg0, float bg1, float bg2,
-                  const uint2* __restrict__ ranges, const uint32_t* __restrict__ order,
-                  const uint32_t* __restrict__ point_list, const float4* __restrict__ records,
-                  const uint32_t* __restrict__ d_num_rendered /* non-null: apply quirk Q10 */, float* __restrict__ img,
-                  uint8_t* __restrict__ rgb8)
+//
+// AUX (blend2_aux_kernel, MODE 2 only): the same walk also accumulates the per-pixel outputs of the frame's optional
+// aux planes -- final alpha 1 - T, depth sum(w_i * z_i) and the number of blended pairs n.  The candidate's view depth
+// z = depth[id] is staged with its record by a fourth, 4-byte cp.async into s_z; the record planes are unchanged.  The
+// colour arithmetic is the same operations in the same order, so the image is bit-identical with AUX on or off.
+// `tid` is threadIdx.x read in the __global__ wrapper: there the compiler knows it is below the launch bound (128) and
+// folds the index arithmetic as it did when this was the kernel's own body; read here, it would not.
+template <int MIN_CTAS, int CPT, int MODE, bool AUX>
+__device__ __forceinline__ void blend2_body(const int tid, int W, int H, uint32_t gx, uint32_t row0, float bg0, float bg1, float bg2,
+                                            const uint2* __restrict__ ranges, const uint32_t* __restrict__ order,
+                                            const uint32_t* __restrict__ point_list, const float4* __restrict__ records,
+                                            const uint32_t* __restrict__ d_num_rendered, float* __restrict__ img,
+                                            uint8_t* __restrict__ rgb8, const float* __restrict__ depth,
+                                            float* __restrict__ out_alpha, float* __restrict__ out_depth,
+                                            uint32_t* __restrict__ out_n)
 {
-    if (d_num_rendered && *d_num_rendered == 0u) return;  // Q10, whole frames only (see blend_kernel)
+    static_assert(!AUX || (MODE == 2 && CPT == 1), "the aux outputs are written for the asynchronous staging only");
 
     constexpr int kB2Round = kB2Threads * CPT, kB2Segs = kB2Round / 32;
     __shared__ float4   s_rec[2][3][kB2Round];  // [buffer][plane][slot], planes as in blend_kernel
     __shared__ uint32_t s_cnt[2][kB2Segs];
+    __shared__ float    s_z[2][AUX ? kB2Round : 1];  // [buffer][slot]: view depth of the candidate (AUX only)
 
-    const int      tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int      lane = tid & 31, warp = tid >> 5;
     const unsigned FULL    = 0xFFFFFFFFu;
     const unsigned lt_mask = (1u << lane) - 1u;
     const uint32_t sbase   = (uint32_t)__cvta_generic_to_shared(&s_rec[0][0][0]);
     constexpr uint32_t kPlane = kB2Round * 16u, kBuf = 3u * kPlane;
+    const uint32_t zbase = AUX ? (uint32_t)__cvta_generic_to_shared(&s_z[0][0]) : 0u;
 
     const uint32_t tile    = __ldg(order + blockIdx.x);  // band-local tile id, longest lists first
     const uint32_t tile_by = tile / gx, tile_bx = tile - tile_by * gx;
@@ -429,6 +443,24 @@ __global__ void __launch_bounds__(kB2Threads, MIN_CTAS)
     const f32x2 npy2 = pack2(-(float)pya, -(float)pyb);            // my - py == my + (-py), exactly
     const float tx0 = (float)tile_x0, ty0 = (float)tile_y0, tx1 = (float)(tile_x0 + 15), ty1 = (float)(tile_y0 + 15);
 
+    // Q10 (whole frames only, see blend_kernel): blend2_kernel returns before it gets here
+    if (AUX && d_num_rendered && *d_num_rendered == 0u) {
+        // Q10 leaves the image of an empty frame untouched; the aux planes have no reference counterpart and are
+        // cleared, so that they never hold a stale frame
+        const size_t pa = (size_t)px + (size_t)W * (size_t)pya, pb = (size_t)px + (size_t)W * (size_t)pyb;
+        if (in_a) {
+            if (out_alpha) out_alpha[pa] = 0.0f;
+            if (out_depth) out_depth[pa] = 0.0f;
+            if (out_n) out_n[pa] = 0u;
+        }
+        if (in_b) {
+            if (out_alpha) out_alpha[pb] = 0.0f;
+            if (out_depth) out_depth[pb] = 0.0f;
+            if (out_n) out_n[pb] = 0u;
+        }
+        return;
+    }
+
     const uint2    range = __ldg(ranges + tile);
     const uint32_t len   = range.y > range.x ? range.y - range.x : 0u;
     const uint32_t nrounds = (len + kB2Round - 1) / kB2Round;
@@ -436,6 +468,8 @@ __global__ void __launch_bounds__(kB2Threads, MIN_CTAS)
     // T < 0 marks a finished pixel, as in blend_kernel
     float Ta = in_a ? 1.0f : -1.0f, Tb = in_b ? 1.0f : -1.0f;
     float c0a = 0.0f, c0b = 0.0f, c1a = 0.0f, c1b = 0.0f, c2a = 0.0f, c2b = 0.0f;
+    float    da_sum = 0.0f, db_sum = 0.0f;  // AUX: sum of w * z
+    uint32_t na = 0u, nb = 0u;              // AUX: blended pairs
 
     // candidate j (0, 1) of a thread is entry j * 128 + tid of the round: warp w's j-th ballot fills segment j * 4 + w,
     // so segment s holds entries [32 s, 32 s + 32) and the consumers meet the list in order
@@ -461,6 +495,7 @@ __global__ void __launch_bounds__(kB2Threads, MIN_CTAS)
             cp_async_16(addr, rec);  // .ca: with .cg (L1 bypass) the blend measured 0.4215 against 0.412 ms
             cp_async_16(addr + kPlane, rec + 1);
             cp_async_16(addr + 2u * kPlane, rec + 2);
+            if constexpr (AUX) cp_async_4(zbase + (buf * kB2Round + (uint32_t)(warp * 32 + 31 - lane)) * 4u, depth + id);
         }
         const unsigned v = __ballot_sync(FULL, valid);
         if (lane == 0) s_cnt[buf][warp] = __popc(v);
@@ -537,7 +572,7 @@ __global__ void __launch_bounds__(kB2Threads, MIN_CTAS)
                 unsigned hits = __ballot_sync(FULL, hit);
                 // one Gaussian on this lane's two pixels; blend_power(a, b, c, dx, dy) = fma(b*dx, dy, fma(a*dx, dx, (c*dy)*dy)),
                 // dx is shared by the pair
-                auto evaluate = [&](const float4& ea, const float4& eb, const float4& ec) {
+                auto evaluate = [&](const float4& ea, const float4& eb, const float4& ec, uint32_t zaddr) {
                     const float dx   = ea.x - pxf;
                     const float adx  = ea.z * dx, bdx = ea.w * dx;
                     const f32x2 dy2  = add2(bcast2(ea.y), npy2);
@@ -562,6 +597,11 @@ __global__ void __launch_bounds__(kB2Threads, MIN_CTAS)
                     fma2_acc_s(c0a, c0b, wsa, wsb, ec.x);
                     fma2_acc_s(c1a, c1b, wsa, wsb, ec.y);
                     fma2_acc_s(c2a, c2b, wsa, wsb, ec.z);
+                    if constexpr (AUX) {
+                        fma2_acc_s(da_sum, db_sum, wsa, wsb, lds32(zaddr));
+                        na += bla;
+                        nb += blb;
+                    }
                     Ta = oka ? (bla ? tta : -fabsf(Ta)) : Ta;
                     Tb = okb ? (blb ? ttb : -fabsf(Tb)) : Tb;
                 };
@@ -577,7 +617,7 @@ __global__ void __launch_bounds__(kB2Threads, MIN_CTAS)
                     const float4 ea = lds128(addr);
                     const float4 eb = lds128(addr + kPlane);
                     const float4 ec = lds128(addr + 2u * kPlane);
-                    evaluate(ea, eb, ec);
+                    evaluate(ea, eb, ec, zbase + (buf * kB2Round + (uint32_t)seg * 32u + (uint32_t)top) * 4u);
                 }
                 da = Ta < 0.0f;
                 db = Tb < 0.0f;
@@ -608,6 +648,19 @@ __global__ void __launch_bounds__(kB2Threads, MIN_CTAS)
         const size_t pix = (size_t)px + (size_t)W * (size_t)pyb;
         img[pix] = vb0; img[pix + plane] = vb1; img[pix + 2 * plane] = vb2;
     }
+    if constexpr (AUX) {
+        const size_t pa = (size_t)px + (size_t)W * (size_t)pya, pb = (size_t)px + (size_t)W * (size_t)pyb;
+        if (in_a) {
+            if (out_alpha) out_alpha[pa] = 1.0f - Ta;
+            if (out_depth) out_depth[pa] = da_sum;
+            if (out_n) out_n[pa] = na;
+        }
+        if (in_b) {
+            if (out_alpha) out_alpha[pb] = 1.0f - Tb;
+            if (out_depth) out_depth[pb] = db_sum;
+            if (out_n) out_n[pb] = nb;
+        }
+    }
     if (rgb8) {
         // the app's post-process as in blend_kernel: staged in shared memory, 32-byte runs per warp instruction
         unsigned char* const s_u8 = reinterpret_cast<unsigned char*>(&s_rec[0][0][0]);
@@ -629,6 +682,34 @@ __global__ void __launch_bounds__(kB2Threads, MIN_CTAS)
             if (y < H && col < cols) rgb8[((size_t)(H - 1 - y) * (size_t)W + (size_t)tile_x0) * 3 + col] = s_u8[k];
         }
     }
+}
+
+template <int MIN_CTAS, int CPT, int MODE = 0>
+__global__ void __launch_bounds__(kB2Threads, MIN_CTAS)
+    blend2_kernel(int W, int H, uint32_t gx, uint32_t row0, float bg0, float bg1, float bg2,
+                  const uint2* __restrict__ ranges, const uint32_t* __restrict__ order,
+                  const uint32_t* __restrict__ point_list, const float4* __restrict__ records,
+                  const uint32_t* __restrict__ d_num_rendered /* non-null: apply quirk Q10 */, float* __restrict__ img,
+                  uint8_t* __restrict__ rgb8)
+{
+    if (d_num_rendered && *d_num_rendered == 0u) return;  // Q10, whole frames only (see blend_kernel)
+    blend2_body<MIN_CTAS, CPT, MODE, false>((int)threadIdx.x, W, H, gx, row0, bg0, bg1, bg2, ranges, order, point_list, records, d_num_rendered,
+                                            img, rgb8, nullptr, nullptr, nullptr, nullptr);
+}
+
+// blend2_kernel<MIN_CTAS, 1, 2> plus the aux planes (see blend2_body); each plane pointer may be null on its own.
+// depth: the frame's per-Gaussian view depth [P], indexed like the records.
+template <int MIN_CTAS>
+__global__ void __launch_bounds__(kB2Threads, MIN_CTAS)
+    blend2_aux_kernel(int W, int H, uint32_t gx, uint32_t row0, float bg0, float bg1, float bg2,
+                      const uint2* __restrict__ ranges, const uint32_t* __restrict__ order,
+                      const uint32_t* __restrict__ point_list, const float4* __restrict__ records,
+                      const uint32_t* __restrict__ d_num_rendered /* non-null: apply quirk Q10 */, float* __restrict__ img,
+                      uint8_t* __restrict__ rgb8, const float* __restrict__ depth, float* __restrict__ out_alpha,
+                      float* __restrict__ out_depth, uint32_t* __restrict__ out_n)
+{
+    blend2_body<MIN_CTAS, 1, 2, true>((int)threadIdx.x, W, H, gx, row0, bg0, bg1, bg2, ranges, order, point_list, records, d_num_rendered, img,
+                                      rgb8, depth, out_alpha, out_depth, out_n);
 }
 
 // Display::_transpose_shader (app/display.cpp:30-39): planar CHW float -> RGBA8 unorm framebuffer, no flip.
@@ -657,7 +738,7 @@ int launch_tile_order(lcgs_b200_ctx* ctx, const uint32_t* ranges, int num_tiles,
 // `ranges` must have been ordered by launch_tile_order on the same stream.
 int launch_blend(lcgs_b200_ctx* ctx, int W, int H, const float* bg, const uint32_t* ranges, const uint32_t* point_list,
                  const float4* records, const uint32_t* d_num_rendered, float* img, uint8_t* rgb8, int row0, int row1,
-                 cudaStream_t s)
+                 cudaStream_t s, const float* depth, float* out_alpha, float* out_depth, uint32_t* out_n)
 {
     const uint32_t gx = (uint32_t)((W + 15) / 16), gy = (uint32_t)((H + 15) / 16);
     if (row1 < 0) row1 = (int)gy;
@@ -676,6 +757,14 @@ int launch_blend(lcgs_b200_ctx* ctx, int W, int H, const float* bg, const uint32
     //                                                          0.451 / 0.432 / 0.420 / 0.439 / 0.463 (10: 48 registers,
     //                                                          spills); two candidates per thread (rounds of 256) at
     //                                                          5 / 6 / 7 / 8: 0.524 / 0.487 / 0.486 / 0.630
+    if (out_alpha || out_depth || out_n) {
+        // the production geometry plus the aux planes: 56 registers at a launch bound of 9 CTAs per SM (at 10 the four
+        // extra accumulators spill)
+        blend2_aux_kernel<9><<<num_tiles, kB2Threads, 0, s>>>(W, H, gx, (uint32_t)row0, bg[0], bg[1], bg[2], rg, ord, point_list,
+                                                                     records, q10, img, rgb8, depth, out_alpha, out_depth, out_n);
+        LCGS_CUDA_CHECK(ctx, cudaGetLastError());
+        return LCGS_B200_OK;
+    }
     auto kern2 = blend2_kernel<10, 1, 2>;
 #ifdef LCGS_TUNING
     {   // A/B selection (tuning library only): LCGS_BLEND2_MODE 0 / 1 / 2, LCGS_BLEND2_CPT 1 / 2 (mode 0), LCGS_BLEND2_OCC

@@ -91,6 +91,8 @@ static int check_frame_lists(lcgs_b200_ctx* ctx, const lcgs_b200_frame* fr)
     LCGS_REQUIRE(ctx, fr->ranges && fr->target_img, "frame: missing ranges / target_img");
     LCGS_REQUIRE(ctx, aligned(fr->point_list_keys_unsorted, 8) && aligned(fr->point_list_keys, 8) && aligned(fr->ranges, 8),
                  "frame: keys / ranges must be 8-byte aligned");
+    LCGS_REQUIRE(ctx, aligned(fr->target_alpha, 4) && aligned(fr->target_depth, 4) && aligned(fr->target_n_contrib, 4),
+                 "frame: target_alpha / target_depth / target_n_contrib must be 4-byte aligned");
     return LCGS_B200_OK;
 }
 
@@ -172,7 +174,8 @@ static int splat_tail(lcgs_b200_ctx* ctx, int P, const lcgs_b200_frame* fr, cons
     // tile schedule (longest list first) + the frame's capacity check, made on the device against the count
     if ((rc = launch_tile_order(ctx, fr->ranges, g.num_tiles, d_n, fr->list_capacity, s))) return rc;
     if ((rc = launch_blend(ctx, g.W, g.H, fr->bg_color, fr->ranges, fr->point_list, (const float4*)ctx->record_ws.ptr, d_n,
-                           fr->target_img, fr->target_rgb8, g.row0, g.row1, s)))
+                           fr->target_img, fr->target_rgb8, g.row0, g.row1, s, fr->depth, fr->target_alpha, fr->target_depth,
+                           fr->target_n_contrib)))
         return rc;
     mark(ctx, s);
     // count, overflow flag and the capacity it was tested against travel back together (in stream order, so

@@ -184,7 +184,8 @@ int launch_ranges(lcgs_b200_ctx* ctx, const uint64_t* keys, size_t n_host, const
                   uint32_t* ranges, int num_tiles, cudaStream_t s, bool cleared = false);
 int launch_blend(lcgs_b200_ctx* ctx, int W, int H, const float* bg, const uint32_t* ranges, const uint32_t* point_list,
                  const float4* records, const uint32_t* d_num_rendered, float* img, uint8_t* rgb8, int row0, int row1,
-                 cudaStream_t s);
+                 cudaStream_t s, const float* depth = nullptr, float* out_alpha = nullptr, float* out_depth = nullptr,
+                 uint32_t* out_n = nullptr);
 int launch_transpose_rgba8(lcgs_b200_ctx* ctx, int W, int H, const float* img, uint8_t* rgba, cudaStream_t s);
 int launch_scene_prepare(lcgs_b200_ctx* ctx, int P, const float* opacity, float* consts, cudaStream_t s);
 int launch_tile_order(lcgs_b200_ctx* ctx, const uint32_t* ranges, int num_tiles, const uint32_t* d_num_rendered,

@@ -210,6 +210,10 @@ class GSSplatForwardOutputProxy:
     width: int
     target_img: torch.Tensor
     radii: torch.Tensor
+    # extension, optional: per-pixel [H*W] planes (see Renderer(aux=True)); None = not rendered
+    target_alpha: Optional[torch.Tensor] = None       # float32, 1 - T
+    target_depth: Optional[torch.Tensor] = None       # float32, sum of w_i * depth_i
+    target_n_contrib: Optional[torch.Tensor] = None   # int32 / uint32, Gaussians blended
 
 
 # --------------------------------------------------------------------------------------------------
@@ -315,6 +319,8 @@ def _frame_struct(accel: GSTileSplatterAccelProxy, inp: GSTileSplatterInputProxy
                           accel.point_list_keys.numel(), accel.point_list.numel())
     f.target_img, f.radii = _ptr(out.target_img), _ptr(out.radii)
     f.tile_row_begin, f.tile_row_end = int(row_begin), int(row_end)
+    f.target_alpha, f.target_depth = _ptr(out.target_alpha), _ptr(out.target_depth)
+    f.target_n_contrib = _ptr(out.target_n_contrib)
     return f
 
 
@@ -419,8 +425,11 @@ class Renderer:
     def __init__(self, device: Device, pos, scale, rotq, sh, opacity, width: int, height: int,
                  list_capacity: int = 20_000_000, sh_deg: int = 3, scale_modifier: float = 1.0,
                  bg_color=(0.0, 0.0, 0.0), tile_rows=(0, -1), keep_intermediates: bool = True,
-                 rgb8: bool = False, prepare_scene: bool = True):
+                 rgb8: bool = False, prepare_scene: bool = True, aux: bool = False):
         """rgb8: the blend kernel also writes the app's uint8 HWC image (main.cpp:322-337) into `self.rgb8`.
+        aux: the blend kernel also writes three per-pixel planes -- accumulated opacity (`alpha()`), the sum of
+        weight * view depth over the blended Gaussians (`depth_map()`, see `expected_depth()`) and the number of
+        Gaussians blended into the pixel (`n_contrib()`).
         prepare_scene: compute the per-scene alpha-test constants once (lcgs_b200_scene_prepare) instead of
         deriving them from the opacity in every frame; call `scene_changed()` after modifying `opacity`."""
         self.device = device
@@ -457,6 +466,10 @@ class Renderer:
         self.radii = z(P, torch.int32)
         self.rgb8 = torch.zeros(3 * self.W * self.H, dtype=torch.uint8, device=dev) if rgb8 else None
         self.alpha_consts = z(2 * P, torch.float32) if prepare_scene else None
+        # per-pixel planes ([H*W]; `self.depth` is the per-Gaussian depth)
+        self.alpha_map = z(self.W * self.H, torch.float32) if aux else None
+        self.depth_plane = z(self.W * self.H, torch.float32) if aux else None
+        self.n_contrib_map = z(self.W * self.H, torch.int32) if aux else None
 
         self.c_scene = _capi.Scene(P, int(sh_deg), _ptr(self.pos), _ptr(self.scale), _ptr(self.rotq), _ptr(self.sh),
                                    _ptr(self.opacity), float(scale_modifier), _ptr(self.alpha_consts))
@@ -472,6 +485,8 @@ class Renderer:
         f.target_img, f.radii = _ptr(self.img), _ptr(self.radii)
         f.tile_row_begin, f.tile_row_end = r0, r1
         f.target_rgb8 = _ptr(self.rgb8)
+        f.target_alpha, f.target_depth = _ptr(self.alpha_map), _ptr(self.depth_plane)
+        f.target_n_contrib = _ptr(self.n_contrib_map)
         device.reserve(P, self.capacity)
         self.scene_changed()
 
@@ -539,6 +554,28 @@ class Renderer:
     def image(self) -> torch.Tensor:
         return self.img.view(3, self.H, self.W)
 
+    def _aux_plane(self, t: Optional[torch.Tensor]) -> torch.Tensor:
+        if t is None:
+            raise LcgsError(_capi.ERR_INVALID, "the per-pixel planes need Renderer(..., aux=True)")
+        return t.view(self.H, self.W)
+
+    def alpha(self) -> torch.Tensor:
+        """[H, W] float32: accumulated opacity 1 - T of the last frame (same row order as `image()`)."""
+        return self._aux_plane(self.alpha_map)
+
+    def depth_map(self) -> torch.Tensor:
+        """[H, W] float32: sum over the blended Gaussians of weight * view depth, in blend order (not normalised)."""
+        return self._aux_plane(self.depth_plane)
+
+    def n_contrib(self) -> torch.Tensor:
+        """[H, W] int32: number of Gaussians blended into each pixel (the saturating entry is not counted)."""
+        return self._aux_plane(self.n_contrib_map)
+
+    def expected_depth(self) -> torch.Tensor:
+        """[H, W] float32: depth_map / alpha where alpha > 0, else 0."""
+        a, d = self.alpha(), self.depth_map()
+        return torch.where(a > 0, d / torch.where(a > 0, a, torch.ones_like(a)), torch.zeros_like(d))
+
     def intermediates(self, n: Optional[int] = None) -> dict:
         """Host copies of every buffer of the last frame, typed like the oracle's Frame."""
         n = self.device.num_rendered() if n is None else n
@@ -549,6 +586,10 @@ class Renderer:
             keys_unsorted=self.keys_unsorted[:n].cpu().numpy().view(np.uint64), vals_unsorted=u32(self.vals_unsorted[:n]),
             keys_sorted=self.keys[:n].cpu().numpy().view(np.uint64), vals_sorted=u32(self.vals[:n]),
             ranges=u32(self.ranges).reshape(-1, 2)[:self.num_tiles], img=self.image().cpu().numpy())
+        if self.alpha_map is not None:
+            out["alpha"] = self.alpha().cpu().numpy()
+            out["depth_map"] = self.depth_map().cpu().numpy()
+            out["n_contrib"] = u32(self.n_contrib_map).reshape(self.H, self.W)
         if self.conic is not None:
             out["means_2d"] = self.means_2d.cpu().numpy().reshape(-1, 2)
             out["conic"] = self.conic.cpu().numpy().reshape(-1, 3)
