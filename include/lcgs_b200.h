@@ -253,6 +253,44 @@ LCGS_B200_API int lcgs_b200_splat_forward(lcgs_b200_ctx* ctx, int num_gaussians,
 LCGS_B200_API int lcgs_b200_render(lcgs_b200_ctx* ctx, const lcgs_b200_scene* scene, const lcgs_b200_view_params* vp,
                                    const lcgs_b200_frame* frame, lcgs_b200_stream stream);
 
+/* ---- backward (no reference counterpart: the reference renders only) ------------------------
+ *
+ * Gradients of a scalar loss L of one whole frame's planar image target_img [3][H][W], rendered by
+ * lcgs_b200_render, with respect to the five scene arrays as the forward uses them (after activation; chaining to
+ * pre-activation parameters is the caller's).  Semantics, restated from the forward as written:
+ *   blend, per pixel, over the entries i = 1..n the forward blended, in list order: w_i = T_i alpha_i,
+ *     T_{i+1} = T_i (1 - alpha_i), C = sum w_i c_i + T_{n+1} bg; with G = dL/dC
+ *       dL/dc_i = w_i G,  dL/dalpha_i = T_i (c_i . G) - (R_i . G) / (1 - alpha_i),  R_i = C - sum_{j<=i} w_j c_j.
+ *     C is read back from target_img, so the backward walks front to back like the forward, with the same culling,
+ *     ex2-based alpha and T (1 - alpha) < 1e-4 stop.  Entries the alpha test rejects and the entry that would saturate
+ *     the pixel get no gradient.
+ *   alpha = min(0.99, o e^power): zero gradient where the cap is active, else dalpha/do = alpha / o and
+ *     dalpha/dpower = alpha; power = -1/2 (A dx^2 + C dy^2) - B dx dy, dx = mean_x - x_p (no half-pixel offset).
+ *   preprocess: the projection, EWA covariance (unnormalised quaternion, scale_modifier), the +0.3 low-pass and
+ *     det + 1e-6 of the conic, and the SH colour are differentiated as written.  The tx/ty clamp to +-1.3 tanfov and
+ *     the [0,1] colour clamp (per channel) pass gradient only where inactive; the view direction of SH degree >= 1
+ *     reaches pos.  radius, the tile rect, depth order and tiles_touched are discrete: a Gaussian with
+ *     tiles_touched == 0 gets exactly zero in every output.  An empty frame gives all-zero gradients.
+ * Gradients are summed with float atomics: the last bits vary from run to run. */
+typedef struct lcgs_b200_grad {
+    const float* dl_dimg; /* [3][H][W], layout of target_img */
+    /* scene gradients, each optional (NULL = not wanted); overwritten, not accumulated; 4-byte aligned */
+    float *grad_pos, *grad_scale, *grad_rotq, *grad_sh, *grad_opacity;
+    /* optional: gradients of the blend's per-Gaussian inputs -- pixel-space mean [P][2] (also the
+       densification statistic trainers accumulate), conic [P][3], post-clamp colour [P][3] */
+    float *grad_means_2d, *grad_conic, *grad_color;
+} lcgs_b200_grad;
+
+/* Backward of one whole frame.  `scene`, `vp` and `frame` are those the frame was rendered with; the call reads only
+ * the frame's point_list, ranges, means_2d, conic, color, tiles_touched and target_img (all required), plus the scene
+ * and the view -- not the context's workspace from the forward, so any number of frames, on this context or another,
+ * may be rendered between a frame and its backward as long as that frame's buffers are intact.  Enqueue only (no
+ * host synchronisation except workspace growth).  LCGS_B200_ERR_INVALID for a NULL required pointer or a misaligned
+ * pointer, LCGS_B200_ERR_UNSUPPORTED for a tile-row band (whole frames only). */
+LCGS_B200_API int lcgs_b200_render_backward(lcgs_b200_ctx* ctx, const lcgs_b200_scene* scene,
+                                            const lcgs_b200_view_params* vp, const lcgs_b200_frame* frame,
+                                            const lcgs_b200_grad* grad, lcgs_b200_stream stream);
+
 /* The value GSTileSplatter::forward returns (impl.cpp:179): synchronises `stream` (the one the
  * last whole-frame call was enqueued on) and stores that frame's num_rendered.  Returns LCGS_B200_ERR_CAPACITY if it exceeded
  * list_capacity (the frame's image is then incomplete).  The comparison is made ON THE DEVICE by the

@@ -56,6 +56,14 @@ class Frame(C.Structure):
                 ("target_n_contrib", C.c_void_p)]
 
 
+class Grad(C.Structure):
+    """lcgs_b200_grad: dL/dimg in, per-Gaussian gradients out (each output optional)."""
+
+    _fields_ = [("dl_dimg", C.c_void_p), ("grad_pos", C.c_void_p), ("grad_scale", C.c_void_p), ("grad_rotq", C.c_void_p),
+                ("grad_sh", C.c_void_p), ("grad_opacity", C.c_void_p), ("grad_means_2d", C.c_void_p),
+                ("grad_conic", C.c_void_p), ("grad_color", C.c_void_p)]
+
+
 PEER_HANDLE_BYTES = 64
 _VP = C.c_void_p
 _I = C.c_int
@@ -89,6 +97,7 @@ _PROTOS = {
     "lcgs_b200_blend": (_I, [_VP, _I, _I, _I, C.POINTER(_F), _VP, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _I, _I, _VP]),
     "lcgs_b200_splat_forward": (_I, [_VP, _I, _VP, C.POINTER(Frame), _VP]),
     "lcgs_b200_render": (_I, [_VP, C.POINTER(Scene), C.POINTER(ViewParams), C.POINTER(Frame), _VP]),
+    "lcgs_b200_render_backward": (_I, [_VP, C.POINTER(Scene), C.POINTER(ViewParams), C.POINTER(Frame), C.POINTER(Grad), _VP]),
     "lcgs_b200_num_rendered": (_I, [_VP, _VP, C.POINTER(_I)]),
     "lcgs_b200_read_num_rendered_async": (_I, [_VP, _VP, _VP]),
     "lcgs_b200_read_image": (_I, [_VP, C.POINTER(Frame), _VP, _VP]),

@@ -271,6 +271,7 @@ int lcgs_b200_ctx_destroy(lcgs_b200_ctx* ctx)
     if (ctx->order_ws.ptr) cudaFree(ctx->order_ws.ptr);
     if (ctx->tile_order_ws.ptr) cudaFree(ctx->tile_order_ws.ptr);
     if (ctx->emit_ws.ptr) cudaFree(ctx->emit_ws.ptr);
+    if (ctx->grad_ws.ptr) cudaFree(ctx->grad_ws.ptr);
     sort_free_plans(ctx);
     for (int i = 0; i < 16; i++)
         if (ctx->ev[i]) cudaEventDestroy(ctx->ev[i]);
@@ -549,6 +550,39 @@ int lcgs_b200_render(lcgs_b200_ctx* ctx, const lcgs_b200_scene* sc, const lcgs_b
     if ((rc = launch_preprocess_fused(ctx, sc, vp, fr, (float4*)ctx->record_ws.ptr, order_ws_views(ctx, P).rects, s))) return rc;
     mark(ctx, s);
     return splat_tail(ctx, P, fr, g, fr->means_2d, true, s);
+}
+
+int lcgs_b200_render_backward(lcgs_b200_ctx* ctx, const lcgs_b200_scene* sc, const lcgs_b200_view_params* vp,
+                              const lcgs_b200_frame* fr, const lcgs_b200_grad* gr, lcgs_b200_stream stream)
+{
+    int rc = enter(ctx);
+    if (rc) return rc;
+    LCGS_REQUIRE(ctx, sc && vp && fr && gr, "render_backward: null argument");
+    FrameGeom g;
+    if ((rc = frame_geom(ctx, fr, &g))) return rc;
+    if (g.row0 != 0 || g.row1 != (int)g.gy) {
+        snprintf(ctx->last_error, sizeof(ctx->last_error), "render_backward: tile-row bands are not supported");
+        return LCGS_B200_ERR_UNSUPPORTED;
+    }
+    const int P = sc->num_gaussians;
+    LCGS_REQUIRE(ctx, P >= 0 && sc->sh_deg >= 0 && sc->sh_deg <= 3, "render_backward: bad scene");
+    LCGS_REQUIRE(ctx, vp->width == fr->width && vp->height == fr->height, "render_backward: view/frame resolution mismatch");
+    LCGS_REQUIRE(ctx, fr->ranges && fr->target_img && gr->dl_dimg, "render_backward: missing ranges / target_img / dl_dimg");
+    LCGS_REQUIRE(ctx, P == 0 || (sc->pos && sc->scale && sc->rotq && sc->sh && sc->opacity), "render_backward: null scene array");
+    LCGS_REQUIRE(ctx, P == 0 || (fr->point_list && fr->means_2d && fr->conic && fr->color && fr->tiles_touched),
+                 "render_backward: point_list / means_2d / conic / color / tiles_touched are required");
+    LCGS_REQUIRE(ctx, aligned(sc->rotq, 16) && aligned(sc->sh, 16) && aligned(sc->alpha_consts, 8),
+                 "render_backward: rotq and sh must be 16-byte, alpha_consts 8-byte aligned");
+    LCGS_REQUIRE(ctx, aligned(fr->ranges, 8) && aligned(fr->means_2d, 8), "render_backward: ranges / means_2d must be 8-byte aligned");
+    LCGS_REQUIRE(ctx, aligned(sc->pos, 4) && aligned(sc->scale, 4) && aligned(sc->opacity, 4) && aligned(fr->conic, 4) &&
+                          aligned(fr->color, 4) && aligned(fr->tiles_touched, 4) && aligned(fr->point_list, 4) &&
+                          aligned(fr->target_img, 4) && aligned(gr->dl_dimg, 4),
+                 "render_backward: float / index buffers must be 4-byte aligned");
+    LCGS_REQUIRE(ctx, aligned(gr->grad_pos, 4) && aligned(gr->grad_scale, 4) && aligned(gr->grad_rotq, 4) && aligned(gr->grad_sh, 4) &&
+                          aligned(gr->grad_opacity, 4) && aligned(gr->grad_means_2d, 4) && aligned(gr->grad_conic, 4) &&
+                          aligned(gr->grad_color, 4),
+                 "render_backward: gradient buffers must be 4-byte aligned");
+    return launch_render_backward(ctx, sc, vp, fr, gr, as_stream(stream));
 }
 
 int lcgs_b200_num_rendered(lcgs_b200_ctx* ctx, lcgs_b200_stream stream, int* num_rendered)

@@ -18,6 +18,17 @@ constexpr int kNumSMs = 148;  // B200; the real count is queried at ctx creation
 //   r2 = (red, green, blue, cull quotient rx)            -- see cull_coef() in lcgs_math.cuh
 constexpr int kRecordFloat4s = 3;
 
+// (thr, l2op) = (alpha_threshold(opacity), log2f(opacity)): the two per-Gaussian constants of the alpha test.
+// Written by the forward's preprocess and rebuilt by the backward from the frame's buffers (backward.cu).
+__device__ __forceinline__ void write_record(float4* rec, const Splat2D& s, float thr, float l2op, const float* rgb)
+{
+    const float    a = -0.5f * s.conic[0], b = -s.conic[1], c = -0.5f * s.conic[2];
+    const CullCoef k = cull_coef(s.px, s.py, a, b, c, thr);
+    rec[0] = make_float4(s.px, s.py, a, b);
+    rec[1] = make_float4(c, thr, l2op, k.ry);  // the blend evaluates alpha as 2^(power*log2e + log2(opacity))
+    rec[2] = make_float4(rgb[0], rgb[1], rgb[2], k.rx);
+}
+
 // Depth keys of the per-Gaussian sort are stored relative to the bit pattern of 0.2f, the smallest
 // depth a Gaussian that touches a tile can have (near cull, gs_projector/shader.cpp:121): for
 // depth < 0.2 * 2^16 they fit in 27 bits = three 9-bit digits, and the fourth pass skips itself.
@@ -54,6 +65,7 @@ struct lcgs_b200_ctx {
     lcgs_b200::Workspace order_ws;    // fused path: packed rects + compacted/sorted (depth, index) pairs + offsets
     lcgs_b200::Workspace tile_order_ws;  // blend: tile ids, longest list first
     lcgs_b200::Workspace emit_ws;        // emission: entries + pieces of the Gaussians expanded by emit_big_kernel
+    lcgs_b200::Workspace grad_ws;        // backward: packed per-Gaussian gradient of the blend's inputs [P][12]
     // per-stage timing
     int          profiling  = 0;
     cudaEvent_t  ev[16];
@@ -190,6 +202,9 @@ int launch_transpose_rgba8(lcgs_b200_ctx* ctx, int W, int H, const float* img, u
 int launch_scene_prepare(lcgs_b200_ctx* ctx, int P, const float* opacity, float* consts, cudaStream_t s);
 int launch_tile_order(lcgs_b200_ctx* ctx, const uint32_t* ranges, int num_tiles, const uint32_t* d_num_rendered,
                       size_t list_capacity, cudaStream_t s);
+// lcgs_b200_render_backward of a whole frame (backward.cu); arguments checked by the caller
+int launch_render_backward(lcgs_b200_ctx* ctx, const lcgs_b200_scene* sc, const lcgs_b200_view_params* vp,
+                           const lcgs_b200_frame* fr, const lcgs_b200_grad* gr, cudaStream_t s);
 int launch_peer_signal(lcgs_b200_ctx* ctx, uint32_t* flag, uint32_t value, cudaStream_t s);
 int launch_peer_wait(lcgs_b200_ctx* ctx, const uint32_t* flag, uint32_t value, uint32_t timeout_ms, cudaStream_t s);
 int launch_checksum_u32(lcgs_b200_ctx* ctx, const void* data, size_t num_words, uint64_t* out, cudaStream_t s);

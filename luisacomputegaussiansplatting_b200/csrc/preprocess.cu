@@ -50,16 +50,6 @@ struct GlobalSh {
     __device__ __forceinline__ float operator()(int k, int c) const { return __ldg(p + k * 3 + c); }
 };
 
-// (thr, l2op) = (alpha_threshold(opacity), log2f(opacity)): the two per-Gaussian constants of the alpha test
-__device__ __forceinline__ void write_record(float4* rec, const Splat2D& s, float thr, float l2op, const float* rgb)
-{
-    const float    a = -0.5f * s.conic[0], b = -s.conic[1], c = -0.5f * s.conic[2];
-    const CullCoef k = cull_coef(s.px, s.py, a, b, c, thr);
-    rec[0] = make_float4(s.px, s.py, a, b);
-    rec[1] = make_float4(c, thr, l2op, k.ry);  // the blend evaluates alpha as 2^(power*log2e + log2(opacity))
-    rec[2] = make_float4(rgb[0], rgb[1], rgb[2], k.rx);
-}
-
 // The alpha-test constants depend on the opacity alone.  Computing the threshold is a binary64 search
 // (alpha_threshold(), ~25 % of the fused kernel's issue slots), so a caller that renders many frames of one
 // scene computes them once (lcgs_b200_scene_prepare) and passes them in lcgs_b200_scene::alpha_consts.

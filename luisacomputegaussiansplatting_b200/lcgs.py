@@ -595,3 +595,133 @@ class Renderer:
             out["conic"] = self.conic.cpu().numpy().reshape(-1, 3)
             out["color"] = self.color.cpu().numpy().reshape(-1, 3)
         return out
+
+
+# --------------------------------------------------------------------------------------------------
+# differentiable rendering (extension: no reference counterpart)
+# --------------------------------------------------------------------------------------------------
+
+def _scene_input(t: torch.Tensor, device: torch.device) -> torch.Tensor:
+    """float32, contiguous, 16-byte aligned copy (or the tensor itself when it already is one), detached."""
+    t = t.detach().to(device=device, dtype=torch.float32).contiguous()
+    return t if t.data_ptr() % 16 == 0 else t.clone()
+
+
+class _RenderFunction(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, dr: "DifferentiableRenderer", vp: ViewParams, pos, scale, rotq, sh, opacity):
+        img, (scene, b) = dr._forward(vp, pos, scale, rotq, sh, opacity)
+        # the image is the output: it goes through save_for_backward (an attribute would make a reference cycle)
+        ctx.save_for_backward(img)
+        ctx.dr, ctx.vp, ctx.saved = dr, vp, (scene, {k: v for k, v in b.items() if k != "img"})
+        ctx.shapes = [t.shape for t in (pos, scale, rotq, sh, opacity)]
+        return img
+
+    @staticmethod
+    def backward(ctx, dl_dimg):
+        want = ctx.needs_input_grad[2:]
+        scene, b = ctx.saved
+        b = dict(b, img=ctx.saved_tensors[0])
+        grads = ctx.dr._backward(ctx.vp, (scene, b), dl_dimg, want)
+        ctx.saved = None  # the frame's buffers are released with the graph
+        out = [g.view(s) if g is not None else None for g, s in zip(grads, ctx.shapes)]
+        return (None, None, *out)
+
+
+class DifferentiableRenderer:
+    """Renders one whole frame as the output of a torch.autograd.Function: `dr(pos, scale, rotq, sh, opacity, cam)`
+    returns the planar [3, H, W] image, and `backward` runs lcgs_b200_render_backward (CUDA kernels, no reference
+    counterpart) to produce gradients shaped like the five inputs.  The inputs are the scene arrays after activation
+    (pos [P,3], scale [P,3], rotq [P,4] = (r,x,y,z), sh [P,(sh_deg+1)^2,3], opacity [P]); chaining to pre-activation
+    parameters is ordinary torch code around the call.  The image is bit-identical to `Renderer.render`'s.
+
+    Each call allocates the buffers its backward reads (instance list, ranges, means_2d, conic, colour,
+    tiles_touched, image) and keeps them on the autograd graph, so several views may be rendered before one
+    `loss.backward()`.  The unsorted / sorted key lists are scratch shared by every call of this renderer.  The
+    alpha-test constants are recomputed every call, because the opacity changes every step.  A frame with more
+    instances than `list_capacity` raises CapacityError in the forward.
+
+    keep_means_2d_grad: keep the last backward's [P, 2] pixel-space mean gradient (the densification statistic) in
+    `means_2d_grad`."""
+
+    def __init__(self, device: Device, width: int, height: int, list_capacity: int = 4_000_000, sh_deg: int = 3,
+                 bg_color=(0.0, 0.0, 0.0), scale_modifier: float = 1.0, keep_means_2d_grad: bool = False):
+        self.device = device
+        self.W, self.H = int(width), int(height)
+        self.gx, self.gy = (self.W + 15) // 16, (self.H + 15) // 16
+        self.capacity = int(list_capacity)
+        self.sh_deg = int(sh_deg)
+        self.bg_color = tuple(float(x) for x in bg_color)
+        self.scale_modifier = float(scale_modifier)
+        self.keep_means_2d_grad = keep_means_2d_grad
+        self.means_2d_grad: Optional[torch.Tensor] = None
+        dev = device.torch_device
+        self.keys_unsorted = torch.zeros(self.capacity, dtype=torch.int64, device=dev)
+        self.vals_unsorted = torch.zeros(self.capacity, dtype=torch.int32, device=dev)
+        self.keys = torch.zeros(self.capacity, dtype=torch.int64, device=dev)
+        self._reserved = -1
+
+    def __call__(self, pos, scale, rotq, sh, opacity, cam: Camera) -> torch.Tensor:
+        return _RenderFunction.apply(self, view_params(cam), pos, scale, rotq, sh, opacity)
+
+    def _scene(self, pos, scale, rotq, sh, opacity, alpha_consts) -> _capi.Scene:
+        P = int(pos.shape[0])
+        return _capi.Scene(P, self.sh_deg, _ptr(pos), _ptr(scale), _ptr(rotq), _ptr(sh), _ptr(opacity),
+                           self.scale_modifier, _ptr(alpha_consts))
+
+    def _frame(self, b: dict) -> _capi.Frame:
+        f = _capi.Frame()
+        f.width, f.height = self.W, self.H
+        f.bg_color[:] = list(self.bg_color)
+        f.means_2d, f.depth, f.conic, f.color = _ptr(b["means_2d"]), _ptr(b["depth"]), _ptr(b["conic"]), _ptr(b["color"])
+        f.tiles_touched, f.point_offsets = _ptr(b["tiles_touched"]), _ptr(b["point_offsets"])
+        f.point_list_keys_unsorted, f.point_list_unsorted = _ptr(self.keys_unsorted), _ptr(self.vals_unsorted)
+        f.point_list_keys, f.point_list = _ptr(self.keys), _ptr(b["point_list"])
+        f.ranges, f.list_capacity = _ptr(b["ranges"]), self.capacity
+        f.target_img, f.radii = _ptr(b["img"]), _ptr(b["radii"])
+        f.tile_row_begin, f.tile_row_end = 0, -1
+        return f
+
+    def _forward(self, vp: ViewParams, pos, scale, rotq, sh, opacity):
+        d = self.device
+        dev = d.torch_device
+        feat = (self.sh_deg + 1) ** 2
+        P = int(pos.shape[0])
+        assert tuple(sh.shape) == (P, feat, 3), "sh must be [P, (sh_deg+1)^2, 3]"
+        assert vp.width == self.W and vp.height == self.H, "camera resolution differs from the renderer's"
+        scene = [_scene_input(t, dev) for t in (pos, scale, rotq, sh, opacity)]
+        if P > self._reserved:
+            d.reserve(P, self.capacity)
+            self._reserved = P
+        z = lambda n, dt: torch.zeros(int(n), dtype=dt, device=dev)  # noqa: E731
+        b = dict(means_2d=z(2 * P, torch.float32), depth=z(P, torch.float32), conic=z(3 * P, torch.float32),
+                 color=z(3 * P, torch.float32), tiles_touched=z(P, torch.int32), point_offsets=z(P, torch.int32),
+                 point_list=torch.empty(self.capacity, dtype=torch.int32, device=dev),
+                 ranges=z(2 * max(self.gx * self.gy, 1), torch.int32), img=z(3 * self.W * self.H, torch.float32),
+                 radii=z(P, torch.int32), alpha_consts=torch.empty(2 * P, dtype=torch.float32, device=dev))
+        stream = _stream_handle(None)
+        d.check(d.lib.lcgs_b200_scene_prepare(d.ctx, P, _ptr(scene[4]), _ptr(b["alpha_consts"]), stream))
+        c_scene = self._scene(*scene, b["alpha_consts"])
+        f = self._frame(b)
+        d.check(d.lib.lcgs_b200_render(d.ctx, C.byref(c_scene), C.byref(vp), C.byref(f), stream))
+        d.num_rendered()  # raises CapacityError on overflow
+        return b["img"].view(3, self.H, self.W), (scene, b)
+
+    def _backward(self, vp: ViewParams, saved, dl_dimg: torch.Tensor, want) -> list:
+        d = self.device
+        scene, b = saved
+        P = int(scene[0].shape[0])
+        dl = dl_dimg.detach().to(dtype=torch.float32).contiguous()
+        grads = [torch.empty_like(t) if w else None for t, w in zip(scene, want)]
+        g = _capi.Grad()
+        g.dl_dimg = _ptr(dl)
+        g.grad_pos, g.grad_scale, g.grad_rotq, g.grad_sh, g.grad_opacity = (_ptr(t) for t in grads)
+        m2 = torch.empty((P, 2), dtype=torch.float32, device=dl.device) if self.keep_means_2d_grad else None
+        g.grad_means_2d = _ptr(m2)
+        c_scene = self._scene(*scene, b["alpha_consts"])
+        f = self._frame(b)
+        d.check(d.lib.lcgs_b200_render_backward(d.ctx, C.byref(c_scene), C.byref(vp), C.byref(f), C.byref(g),
+                                                _stream_handle(None)))
+        if self.keep_means_2d_grad:
+            self.means_2d_grad = m2
+        return grads
