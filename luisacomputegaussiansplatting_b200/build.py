@@ -8,11 +8,14 @@ the repository snapshot.  Flags that matter:
 """
 from __future__ import annotations
 
+import atexit
 import fcntl
 import hashlib
 import os
+import shutil
 import subprocess
 import sys
+import tempfile
 from concurrent.futures import ThreadPoolExecutor
 
 HERE = os.path.dirname(os.path.abspath(__file__))
@@ -20,7 +23,7 @@ CSRC = os.path.join(HERE, "csrc")
 BUILD = os.path.join(CSRC, "build")
 LIB = os.path.join(HERE, "liblcgs_b200.so")
 SOURCES = ["capi.cu", "preprocess.cu", "scan.cu", "binning.cu", "sort.cu", "blend.cu", "backward.cu"]
-HEADERS = ["common.cuh", "lcgs_math.cuh", "lcgs_grad.cuh", "lookback.cuh", os.path.join("..", "..", "include", "lcgs_b200.h")]
+HEADERS = ["common.cuh", "lcgs_math.cuh", "lcgs_grad.cuh", "lookback.cuh", "blend_walk.cuh", os.path.join("..", "..", "include", "lcgs_b200.h")]
 
 NVCC = os.environ.get("LCGS_NVCC", "/usr/local/cuda/bin/nvcc")
 NVCC_FLAGS = [
@@ -153,23 +156,37 @@ FACADE_TEST_SRC = os.path.join(HERE, "..", "tests", "facade", "test_facade.cpp")
 FACADE_TEST_BIN = os.path.join(HERE, "..", "tests", "facade", "test_facade")
 
 
+_facade_tmp = None  # private directory of a facade test built outside a read-only tree
+
+
 def build_facade_test(force: bool = False) -> str:
     """tests/facade/test_facade: the reference's GSTileSplatter::forward call sequence and a 16-byte-float3 camera
-    compiled against the C++ facade (checks that the facade keeps the reference's argument lists)."""
+    compiled against the C++ facade (checks that the facade keeps the reference's argument lists).  In a tree the
+    tests cannot write to, a stale or missing binary is built into a private temporary directory instead, removed when
+    Python exits."""
+    global _facade_tmp
     lib = build_native()
     newest = max([_mtime(f) for f in _app_deps()] + [_mtime(lib), _mtime(FACADE_TEST_SRC)])
-    if not force and _mtime(FACADE_TEST_BIN) >= newest:
-        return FACADE_TEST_BIN
+    out = FACADE_TEST_BIN
+    if not force and _mtime(out) >= newest:
+        return out
+    if not os.access(os.path.dirname(out), os.W_OK) or (os.path.exists(out) and not os.access(out, os.W_OK)):
+        if _facade_tmp is None:
+            _facade_tmp = tempfile.mkdtemp(prefix="lcgs_b200_facade_")
+            atexit.register(shutil.rmtree, _facade_tmp, True)
+        out = os.path.join(_facade_tmp, "test_facade")
+        if not force and _mtime(out) >= newest:
+            return out
     cmd = ["g++", "-O1", "-std=c++20", "-Wall", "-Wextra", "-Wno-missing-field-initializers"]
     for inc in APP_INCLUDES:
         cmd += ["-I", inc]
-    cmd += [FACADE_TEST_SRC, os.path.join(APP_DIR, "gaussians.cpp"), "-o", FACADE_TEST_BIN, "-L", HERE, "-llcgs_b200",
+    cmd += [FACADE_TEST_SRC, os.path.join(APP_DIR, "gaussians.cpp"), "-o", out, "-L", HERE, "-llcgs_b200",
             "-Wl,-rpath," + HERE, "-L/usr/local/cuda/lib64", "-lcudart_static", "-ldl", "-lrt", "-lpthread"]
     r = subprocess.run(cmd, capture_output=True, text=True)
     if r.returncode != 0:
         sys.stderr.write(r.stdout + r.stderr)
         raise RuntimeError("building tests/facade/test_facade failed")
-    return FACADE_TEST_BIN
+    return out
 
 
 if __name__ == "__main__":

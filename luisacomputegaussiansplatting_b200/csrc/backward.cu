@@ -1,62 +1,29 @@
 // backward.cu -- gradients of a rendered whole frame with respect to the scene (lcgs_b200_render_backward).
 // No reference counterpart: the reference renders only.  The derivatives themselves live in lcgs_grad.cuh.
 //
-//  * rebuild_records_kernel : the 48-byte blend records of the frame, rebuilt from the frame's own means_2d, conic
-//    and colour and the scene's opacity (or alpha_consts) with the forward's write_record -- bit-identical to what
-//    the forward's preprocess wrote, so the backward never depends on the context's workspace from the forward and
-//    any number of frames may be rendered between a frame and its backward.
-//  * blend_backward_kernel : one 128-thread CTA per tile in the forward's longest-first order, the forward's
-//    geometry (four warps, 8x8 patch per warp, lane = pixels (x, y) and (x, y + 4)) and its round-based cp.async
-//    staging with one barrier per round.  Each pixel replays the forward's front-to-back walk with the forward's
-//    operations (blend_power, ex2-based alpha, T (1 - alpha) < 1e-4 stop), so it blends exactly the entries the
-//    forward blended; the final colour C is read back from the image, and R_i . G = C . G - sum_{j<=i} w_j c_j . G
-//    needs no reverse walk and no stored per-pixel state.  Per hit, each lane adds its two pixels' contributions to
-//    the Gaussian's 9 values (mean x/y, conic, dL/dpower, colour), the warp reduces them with shuffles and three
-//    lanes add the sums to the Gaussian's packed [12] float entry with one vector reduction each (RED.128): one
-//    global atomic set per (patch, Gaussian) with a contribution.
+//  * the 48-byte blend records of the frame are rebuilt by the forward's build_records_kernel (preprocess.cu) from the
+//    frame's own means_2d, conic and colour and the scene's opacity (or alpha_consts) -- bit-identical to what the
+//    forward's preprocess wrote, so the backward never depends on the context's workspace from the forward and any
+//    number of frames may be rendered between a frame and its backward.
+//  * blend_backward_kernel : the forward's tile walk (walk_tile, blend_walk.cuh) in the forward's longest-first tile
+//    order.  Each pixel replays the forward's front-to-back walk with the forward's operations (blend_power, ex2-based
+//    alpha, T (1 - alpha) < 1e-4 stop), so it blends exactly the entries the forward blended; the final colour C is
+//    read back from the image, and R_i . G = C . G - sum_{j<=i} w_j c_j . G needs no reverse walk and no stored
+//    per-pixel state.  Per hit, each lane adds its two pixels' contributions to the Gaussian's 9 values (mean x/y,
+//    conic, dL/dpower, colour), the warp reduces them with shuffles and three lanes add the sums to the Gaussian's
+//    packed [12] float entry with one vector reduction each (RED.128): one global atomic set per (patch, Gaussian)
+//    with a contribution.
 //  * preprocess_backward_kernel : one thread per Gaussian; Gaussians with tiles_touched == 0 get zeros.  Recomputes
 //    the forward's intermediates from the scene and chains the packed 2D gradient to pos / scale / rotq / sh /
 //    opacity.
 // Float atomics make the summation order, and so the last bits of the gradients, vary from run to run; the forward
 // is untouched and stays bit-reproducible.
-#include "common.cuh"
+#include "blend_walk.cuh"
 #include "lcgs_grad.cuh"
 
 namespace lcgs_b200 {
 
 namespace {
-
-constexpr int kBwdThreads = 128;
-constexpr int kBwdWarps   = kBwdThreads / 32;
-
-__device__ __forceinline__ float4 bwd_lds128(uint32_t addr)
-{
-    float4 v;
-    asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(addr));
-    return v;
-}
-
-__device__ __forceinline__ float bwd_lds32(uint32_t addr)
-{
-    float v;
-    asm volatile("ld.shared.f32 %0, [%1];" : "=f"(v) : "r"(addr));
-    return v;
-}
-
-__device__ __forceinline__ void bwd_cp_async_16(uint32_t smem_addr, const void* gptr)
-{
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 16;" ::"r"(smem_addr), "l"(gptr) : "memory");
-}
-
-__device__ __forceinline__ void bwd_cp_async_wait_all() { asm volatile("cp.async.commit_group;\ncp.async.wait_group 0;" ::: "memory"); }
-
-// the forward's alpha: 2^(power * log2(e) + log2(opacity)) on MUFU.EX2 (blend.cu)
-__device__ __forceinline__ float bwd_ex2_ftz(float x)
-{
-    float y;
-    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
-    return y;
-}
 
 struct GlobalShIn {
     const float* p;
@@ -73,63 +40,26 @@ struct GlobalShOut {
 
 }  // namespace
 
-__global__ void __launch_bounds__(256)
-    rebuild_records_kernel(int P, const float* __restrict__ means_2d, const float* __restrict__ conic,
-                           const float* __restrict__ color, const float* __restrict__ opacity,
-                           const float2* __restrict__ alpha_consts, const uint32_t* __restrict__ tiles_touched,
-                           float4* __restrict__ records)
-{
-    const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= P || __ldg(tiles_touched + i) == 0u) return;
-    Splat2D s;
-    s.px       = __ldg(means_2d + 2 * i);
-    s.py       = __ldg(means_2d + 2 * i + 1);
-    s.conic[0] = __ldg(conic + 3 * i);
-    s.conic[1] = __ldg(conic + 3 * i + 1);
-    s.conic[2] = __ldg(conic + 3 * i + 2);
-    const float rgb[3] = { __ldg(color + 3 * i), __ldg(color + 3 * i + 1), __ldg(color + 3 * i + 2) };
-    float       thr, l2op;
-    if (alpha_consts) {
-        const float2 k = __ldg(alpha_consts + i);
-        thr = k.x; l2op = k.y;
-    } else {
-        const float op = __ldg(opacity + i);
-        thr  = alpha_threshold(op);
-        l2op = log2f(op);
-    }
-    write_record(records + (size_t)i * kRecordFloat4s, s, thr, l2op, rgb);
-}
-
-__global__ void __launch_bounds__(kBwdThreads)
+__global__ void __launch_bounds__(kWalkThreads)
     blend_backward_kernel(int W, int H, uint32_t gx, const uint2* __restrict__ ranges, const uint32_t* __restrict__ order,
                           const uint32_t* __restrict__ point_list, const float4* __restrict__ records,
                           const float* __restrict__ img, const float* __restrict__ dl_dimg, float4* __restrict__ grad2d)
 {
-    __shared__ float4   s_rec[2][3][kBwdThreads];  // [buffer][plane][slot], planes as in the forward's blend
-    __shared__ uint32_t s_id[2][kBwdThreads];     // [buffer][slot]: Gaussian index of the staged record
-    __shared__ uint32_t s_cnt[2][kBwdWarps];
+    __shared__ float4   s_rec[2][3][kWalkThreads];  // [buffer][plane][slot], planes as in the record (common.cuh)
+    __shared__ uint32_t s_cnt[2][kWalkWarps];
+    __shared__ uint32_t s_id[2 * kWalkThreads];  // [buffer * 128 + slot]: Gaussian index of the staged record
 
-    const int      tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const unsigned FULL  = 0xFFFFFFFFu;
-    const uint32_t sbase = (uint32_t)__cvta_generic_to_shared(&s_rec[0][0][0]);
-    constexpr uint32_t kPlane = kBwdThreads * 16u, kBuf = 3u * kPlane;
-
-    const uint32_t tile    = __ldg(order + blockIdx.x);
-    const uint32_t tile_by = tile / gx, tile_bx = tile - tile_by * gx;
-    const int tile_x0 = (int)tile_bx * 16, tile_y0 = (int)tile_by * 16;
-    const int patch_x0 = tile_x0 + (warp & 1) * 8, patch_y0 = tile_y0 + (warp >> 1) * 8;
-    const int px = patch_x0 + (lane & 7);
-    const int pya = patch_y0 + (lane >> 3), pyb = pya + 4;
-    const bool  in_a = px < W && pya < H, in_b = px < W && pyb < H;
-    const float pxf = (float)px, pyaf = (float)pya, pybf = (float)pyb;  // no half-pixel offset (Q2)
-    // the patch: culling is conservative, so any rectangle containing the pixels gives the forward's decisions
-    const float wx0 = (float)patch_x0, wy0 = (float)patch_y0, wx1 = (float)(patch_x0 + 7), wy1 = (float)(patch_y0 + 7);
+    const int        tid  = threadIdx.x;
+    const unsigned   FULL = 0xFFFFFFFFu;
+    const TilePixels p    = tile_pixels(tid & 31, tid >> 5, order, gx, 0u);
+    const bool       in_a = p.px < W && p.pya < H, in_b = p.px < W && p.pyb < H;
+    const float      pxf = (float)p.px, pyaf = (float)p.pya, pybf = (float)p.pyb;  // no half-pixel offset (Q2)
 
     const size_t plane = (size_t)W * (size_t)H;
     PixelGrad    pa, pb;
     {
         float C[3] = { 0.f, 0.f, 0.f }, G[3] = { 0.f, 0.f, 0.f };
-        const size_t ia = (size_t)px + (size_t)W * (size_t)pya, ib = (size_t)px + (size_t)W * (size_t)pyb;
+        const size_t ia = (size_t)p.px + (size_t)W * (size_t)p.pya, ib = (size_t)p.px + (size_t)W * (size_t)p.pyb;
         if (in_a)
             for (int k = 0; k < 3; k++) { C[k] = __ldg(img + ia + k * plane); G[k] = __ldg(dl_dimg + ia + k * plane); }
         pa = pixel_grad_init(in_a, C, G);
@@ -140,97 +70,41 @@ __global__ void __launch_bounds__(kBwdThreads)
         pb = pixel_grad_init(in_b, C, G);
     }
 
-    const uint2    range   = __ldg(ranges + tile);
-    const uint32_t len     = range.y > range.x ? range.y - range.x : 0u;
-    const uint32_t nrounds = (len + kBwdThreads - 1) / kBwdThreads;
-
-    // entry `lane` of the warp's 32 candidates goes to slot 31 - lane of the warp's segment (filled from the top, so
-    // the walk from the highest hit bit meets the list in order), as in the forward
-    auto stage = [&](uint32_t buf, bool valid, uint32_t id) {
-        if (valid) {
-            const uint32_t slot = (uint32_t)(warp * 32 + 31 - lane);
-            const float4*  rec  = records + (size_t)id * kRecordFloat4s;
-            const uint32_t addr = sbase + buf * kBuf + slot * 16u;
-            bwd_cp_async_16(addr, rec);
-            bwd_cp_async_16(addr + kPlane, rec + 1);
-            bwd_cp_async_16(addr + 2u * kPlane, rec + 2);
-            s_id[buf][slot] = id;
-        }
-        const unsigned v = __ballot_sync(FULL, valid);
-        if (lane == 0) s_cnt[buf][warp] = __popc(v);
-    };
-
-    uint32_t next_id = 0;
-    {
-        const bool v0 = (uint32_t)tid < len;
-        stage(0u, v0, v0 ? __ldg(point_list + range.x + tid) : 0u);
-        if (kBwdThreads + (uint32_t)tid < len) next_id = __ldg(point_list + range.x + kBwdThreads + tid);
-        bwd_cp_async_wait_all();
-    }
-    __syncthreads();
-
-    for (uint32_t r = 0; r < nrounds; r++) {
-        const uint32_t buf  = r & 1u;
-        const uint32_t nidx = (r + 1u) * kBwdThreads + tid;
-        if (r + 1u < nrounds) stage(buf ^ 1u, nidx < len, next_id);
-        if (nidx + kBwdThreads < len) next_id = __ldg(point_list + range.x + nidx + kBwdThreads);
-
-        if (!__all_sync(FULL, !(pa.T > 0.0f) && !(pb.T > 0.0f))) {
-            const uint32_t abase = sbase + buf * kBuf;
-#pragma unroll 1
-            for (int seg = 0; seg < kBwdWarps; seg++) {
-                const uint32_t cnt     = s_cnt[buf][seg];
-                const uint32_t segbase = abase + seg * 512u;
-                bool           hit     = false;
-                if ((uint32_t)lane + cnt >= 32u) {
-                    const float4 ga = bwd_lds128(segbase + lane * 16u);
-                    const float4 gb = bwd_lds128(segbase + kPlane + lane * 16u);
-                    const float  rx = bwd_lds32(segbase + 2u * kPlane + lane * 16u + 12u);
-                    hit = !cull_rect_fast(ga.x, ga.y, ga.z, ga.w, gb.x, gb.y, gb.w, rx, wx0, wy0, wx1, wy1);
-                }
-                unsigned hits = __ballot_sync(FULL, hit);
-                while (hits) {
-                    const int      top  = 31 - __clz(hits);
-                    const uint32_t addr = segbase + top * 16u;
-                    hits ^= 1u << top;
-                    const float4 ea = bwd_lds128(addr);
-                    const float4 eb = bwd_lds128(addr + kPlane);
-                    const float4 ec = bwd_lds128(addr + 2u * kPlane);
-                    const float  rgb[3] = { ec.x, ec.y, ec.z };
-                    float        g[kGrad2DValues];
+    // The walk's cull box shrinks to the pixels still accumulating, as in the forward: the cull is conservative and a
+    // finished pixel adds nothing in blend_entry_grad, so every pixel still meets the entries the forward blended.
+    auto stage_id  = [&](uint32_t entry, uint32_t id) { s_id[entry] = id; };
+    auto no_consts = [] { return 0; };  // the scalar evaluation keeps no per-walk constants
+    auto accumulate = [&](int, const float4& ea, const float4& eb, const float4& ec, uint32_t entry) {
+        const float rgb[3] = { ec.x, ec.y, ec.z };
+        float       g[kGrad2DValues];
 #pragma unroll
-                    for (int k = 0; k < kGrad2DValues; k++) g[k] = 0.0f;
-                    // the forward's per-pixel operations (blend2_body's evaluate, scalar form)
-                    const float dx  = ea.x - pxf;
-                    const float dya = ea.y - pyaf, dyb = ea.y - pybf;
-                    const float pwa = blend_power(ea.z, ea.w, eb.x, dx, dya);
-                    const float pwb = blend_power(ea.z, ea.w, eb.x, dx, dyb);
-                    const bool  oka = !(pwa > 0.0f) && !(pwa < eb.y);
-                    const bool  okb = !(pwb > 0.0f) && !(pwb < eb.y);
-                    const float ea_ = bwd_ex2_ftz(__fmaf_rn(pwa, 1.4426950408889634f, eb.z));
-                    const float eb_ = bwd_ex2_ftz(__fmaf_rn(pwb, 1.4426950408889634f, eb.z));
-                    bool contributed = blend_entry_grad(pa, oka, ea_, dx, dya, ea.z, ea.w, eb.x, rgb, g);
-                    contributed |= blend_entry_grad(pb, okb, eb_, dx, dyb, ea.z, ea.w, eb.x, rgb, g);
-                    if (__any_sync(FULL, contributed)) {
+        for (int k = 0; k < kGrad2DValues; k++) g[k] = 0.0f;
+        // the forward's per-pixel operations (blend2_body's evaluate, scalar form)
+        const float dx  = ea.x - pxf;
+        const float dya = ea.y - pyaf, dyb = ea.y - pybf;
+        const float pwa = blend_power(ea.z, ea.w, eb.x, dx, dya);
+        const float pwb = blend_power(ea.z, ea.w, eb.x, dx, dyb);
+        const bool  oka = !(pwa > 0.0f) && !(pwa < eb.y);
+        const bool  okb = !(pwb > 0.0f) && !(pwb < eb.y);
+        const float ea_ = ex2_ftz(__fmaf_rn(pwa, 1.4426950408889634f, eb.z));
+        const float eb_ = ex2_ftz(__fmaf_rn(pwb, 1.4426950408889634f, eb.z));
+        bool contributed = blend_entry_grad(pa, oka, ea_, dx, dya, ea.z, ea.w, eb.x, rgb, g);
+        contributed |= blend_entry_grad(pb, okb, eb_, dx, dyb, ea.z, ea.w, eb.x, rgb, g);
+        if (__any_sync(FULL, contributed)) {
 #pragma unroll
-                        for (int k = 0; k < kGrad2DValues; k++)
+            for (int k = 0; k < kGrad2DValues; k++)
 #pragma unroll
-                            for (int o = 16; o > 0; o >>= 1) g[k] += __shfl_xor_sync(FULL, g[k], o);
-                        if (lane < 3) {
-                            const uint32_t id = s_id[buf][seg * 32 + top];
-                            const float4   v  = lane == 0 ? make_float4(g[0], g[1], g[2], g[3])
-                                                : lane == 1 ? make_float4(g[4], g[5], g[6], g[7])
-                                                            : make_float4(g[8], 0.0f, 0.0f, 0.0f);
-                            atomicAdd(grad2d + (size_t)id * 3 + lane, v);  // RED.E.ADD.F32x4
-                        }
-                    }
-                }
-                if (__all_sync(FULL, !(pa.T > 0.0f) && !(pb.T > 0.0f))) break;
+                for (int o = 16; o > 0; o >>= 1) g[k] += __shfl_xor_sync(FULL, g[k], o);
+            if (p.lane < 3) {
+                const uint32_t id = s_id[entry];
+                const float4   v  = p.lane == 0 ? make_float4(g[0], g[1], g[2], g[3])
+                                    : p.lane == 1 ? make_float4(g[4], g[5], g[6], g[7])
+                                                  : make_float4(g[8], 0.0f, 0.0f, 0.0f);
+                atomicAdd(grad2d + (size_t)id * 3 + p.lane, v);  // RED.E.ADD.F32x4
             }
         }
-        bwd_cp_async_wait_all();
-        if (__syncthreads_and(!(pa.T > 0.0f) && !(pb.T > 0.0f))) break;
-    }
+    };
+    walk_tile(tid, p, ranges, point_list, records, s_rec, s_cnt, pa.T, pb.T, stage_id, no_consts, accumulate);
 }
 
 struct PreprocessGradArgs {
@@ -322,13 +196,12 @@ int launch_render_backward(lcgs_b200_ctx* ctx, const lcgs_b200_scene* sc, const 
     float4* grad2d  = (float4*)ctx->grad_ws.ptr;
     LCGS_CUDA_CHECK(ctx, cudaMemsetAsync(grad2d, 0, (size_t)P * kGrad2DFloats * sizeof(float), s));
 
-    rebuild_records_kernel<<<bwd_div_up(P, 256), 256, 0, s>>>(P, fr->means_2d, fr->conic, fr->color, sc->opacity,
-                                                               reinterpret_cast<const float2*>(sc->alpha_consts),
-                                                               fr->tiles_touched, records);
-    LCGS_CUDA_CHECK(ctx, cudaGetLastError());
+    if ((rc = launch_build_records(ctx, P, fr->means_2d, fr->conic, sc->opacity, sc->alpha_consts, fr->color,
+                                   fr->tiles_touched, records, s)))
+        return rc;
     // the tile schedule only: no count, so the context's device scalars (the last forward's) stay untouched
     if ((rc = launch_tile_order(ctx, fr->ranges, num_tiles, nullptr, 0, s))) return rc;
-    blend_backward_kernel<<<(unsigned)num_tiles, kBwdThreads, 0, s>>>(W, H, gx, reinterpret_cast<const uint2*>(fr->ranges),
+    blend_backward_kernel<<<(unsigned)num_tiles, kWalkThreads, 0, s>>>(W, H, gx, reinterpret_cast<const uint2*>(fr->ranges),
                                                                       (const uint32_t*)ctx->tile_order_ws.ptr, fr->point_list,
                                                                       records, fr->target_img, gr->dl_dimg, grad2d);
     LCGS_CUDA_CHECK(ctx, cudaGetLastError());

@@ -492,7 +492,8 @@ int lcgs_b200_blend(lcgs_b200_ctx* ctx, int P, int width, int height, const floa
     LCGS_REQUIRE(ctx, aligned(ranges, 8), "blend: ranges must be 8-byte aligned");
     if ((rc = ws_reserve(ctx, ctx->record_ws, (size_t)(P > 0 ? P : 1) * kRecordFloat4s * sizeof(float4)))) return rc;
     cudaStream_t s = as_stream(stream);
-    if ((rc = launch_build_records(ctx, P, means_2d, conic, opacity, color, tiles_touched, (float4*)ctx->record_ws.ptr, s)))
+    if ((rc = launch_build_records(ctx, P, means_2d, conic, opacity, nullptr, color, tiles_touched,
+                                   (float4*)ctx->record_ws.ptr, s)))
         return rc;
     const int gx = (width + 15) / 16, gy = (height + 15) / 16;
     if ((rc = launch_tile_order(ctx, ranges, gx * ((row1 < 0 ? gy : row1) - row0), nullptr, 0, s))) return rc;
@@ -520,7 +521,7 @@ int lcgs_b200_splat_forward(lcgs_b200_ctx* ctx, int P, const float* opacity, con
     if ((rc = launch_allocate_tiles(ctx, P, g.W, g.H, fr->depth, fr->means_2d, fr->conic, fr->tiles_touched, fr->radii,
                                     g.row0, g.row1, s)))
         return rc;
-    if ((rc = launch_build_records(ctx, P, fr->means_2d, fr->conic, opacity, fr->color, fr->tiles_touched,
+    if ((rc = launch_build_records(ctx, P, fr->means_2d, fr->conic, opacity, nullptr, fr->color, fr->tiles_touched,
                                    (float4*)ctx->record_ws.ptr, s)))
         return rc;
     mark(ctx, s);

@@ -19,7 +19,8 @@ constexpr int kNumSMs = 148;  // B200; the real count is queried at ctx creation
 constexpr int kRecordFloat4s = 3;
 
 // (thr, l2op) = (alpha_threshold(opacity), log2f(opacity)): the two per-Gaussian constants of the alpha test.
-// Written by the forward's preprocess and rebuilt by the backward from the frame's buffers (backward.cu).
+// Written by the forward's preprocess and by build_records_kernel (preprocess.cu), which also rebuilds them for the
+// backward from the frame's buffers.
 __device__ __forceinline__ void write_record(float4* rec, const Splat2D& s, float thr, float l2op, const float* rgb)
 {
     const float    a = -0.5f * s.conic[0], b = -s.conic[1], c = -0.5f * s.conic[2];
@@ -181,8 +182,10 @@ int launch_project(lcgs_b200_ctx* ctx, int P, const float* pos, const float* sca
                    cudaStream_t s);
 int launch_allocate_tiles(lcgs_b200_ctx* ctx, int P, int W, int H, const float* depth, float* means_2d, float* covs_2d,
                           uint32_t* tiles_touched, int32_t* radii, int row0, int row1, cudaStream_t s);
+// alpha_consts (lcgs_b200_scene_prepare) and tiles_touched may be null
 int launch_build_records(lcgs_b200_ctx* ctx, int P, const float* means_2d, const float* conic, const float* opacity,
-                         const float* color, const uint32_t* tiles_touched, float4* records, cudaStream_t s);
+                         const float* alpha_consts, const float* color, const uint32_t* tiles_touched, float4* records,
+                         cudaStream_t s);
 int launch_scan(lcgs_b200_ctx* ctx, const uint32_t* in, uint32_t* out, size_t n, uint32_t* d_total, cudaStream_t s);
 int launch_duplicate_keys(lcgs_b200_ctx* ctx, int P, int W, int H, const float* means_2d, const uint32_t* offsets,
                           const int32_t* radii, const float* depth, uint64_t* keys, uint32_t* vals, size_t capacity,

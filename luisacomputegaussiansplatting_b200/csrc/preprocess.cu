@@ -5,7 +5,8 @@
 //    Replaces three DSL kernels with HBM round trips in between (sh_preprocessor.cpp:159-166,
 //    gs_projector/shader.cpp:82-139, gs_tile_splatter/shader.cpp:102-163).
 //  * sh_kernel / project_kernel / allocate_tiles_kernel / build_records_kernel : the same
-//    arithmetic behind the reference's separate entry points.
+//    arithmetic behind the reference's separate entry points (build_records_kernel also rebuilds a
+//    frame's records for the backward pass).
 //
 // HBM-bound: algorithmic bytes per Gaussian = 40 (pos, scale, rotq) + 192 (SH, only when the
 // Gaussian touches a tile) + outputs.  SH rows are fetched with block-cooperative, fully coalesced
@@ -245,24 +246,36 @@ __global__ void __launch_bounds__(256)
     tiles_touched[i] = tiles;
 }
 
-// Packs the reference-layout buffers (after allocate_tiles) into blend records.
+// Packs the reference-layout buffers (after allocate_tiles) into blend records: the forward's separate passes, and the
+// backward's rebuild of a frame's records.  alpha_consts (optional): the scene's per-Gaussian (threshold, log2 opacity),
+// used in place of opacity as the fused preprocess does.  tiles_touched (optional): Gaussians that touch no tile are
+// skipped, their records never read.
 __global__ void __launch_bounds__(256)
     build_records_kernel(int P, const float* __restrict__ means_2d, const float* __restrict__ conic,
-                         const float* __restrict__ opacity, const float* __restrict__ color,
-                         const uint32_t* __restrict__ tiles_touched, float4* __restrict__ records)
+                         const float* __restrict__ opacity, const float2* __restrict__ alpha_consts,
+                         const float* __restrict__ color, const uint32_t* __restrict__ tiles_touched,
+                         float4* __restrict__ records)
 {
     const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= P) return;
-    if (tiles_touched && tiles_touched[i] == 0u) return;
+    if (tiles_touched && __ldg(tiles_touched + i) == 0u) return;
     Splat2D s;
-    s.px       = means_2d[2 * i];
-    s.py       = means_2d[2 * i + 1];
-    s.conic[0] = conic[3 * i];
-    s.conic[1] = conic[3 * i + 1];
-    s.conic[2] = conic[3 * i + 2];
-    const float rgb[3] = { color[3 * i], color[3 * i + 1], color[3 * i + 2] };
-    const float op = opacity[i];
-    write_record(records + (size_t)i * kRecordFloat4s, s, alpha_threshold(op), log2f(op), rgb);
+    s.px       = __ldg(means_2d + 2 * i);
+    s.py       = __ldg(means_2d + 2 * i + 1);
+    s.conic[0] = __ldg(conic + 3 * i);
+    s.conic[1] = __ldg(conic + 3 * i + 1);
+    s.conic[2] = __ldg(conic + 3 * i + 2);
+    const float rgb[3] = { __ldg(color + 3 * i), __ldg(color + 3 * i + 1), __ldg(color + 3 * i + 2) };
+    float       thr, l2op;
+    if (alpha_consts) {
+        const float2 k = __ldg(alpha_consts + i);
+        thr = k.x; l2op = k.y;
+    } else {
+        const float op = __ldg(opacity + i);
+        thr  = alpha_threshold(op);
+        l2op = log2f(op);
+    }
+    write_record(records + (size_t)i * kRecordFloat4s, s, thr, l2op, rgb);
 }
 
 // ---- launchers -------------------------------------------------------------------------------
@@ -333,10 +346,13 @@ int launch_allocate_tiles(lcgs_b200_ctx* ctx, int P, int W, int H, const float* 
 }
 
 int launch_build_records(lcgs_b200_ctx* ctx, int P, const float* means_2d, const float* conic, const float* opacity,
-                         const float* color, const uint32_t* tiles_touched, float4* records, cudaStream_t s)
+                         const float* alpha_consts, const float* color, const uint32_t* tiles_touched, float4* records,
+                         cudaStream_t s)
 {
     if (P <= 0) return LCGS_B200_OK;
-    build_records_kernel<<<div_up(P, 256), 256, 0, s>>>(P, means_2d, conic, opacity, color, tiles_touched, records);
+    build_records_kernel<<<div_up(P, 256), 256, 0, s>>>(P, means_2d, conic, opacity,
+                                                        reinterpret_cast<const float2*>(alpha_consts), color,
+                                                        tiles_touched, records);
     LCGS_CUDA_CHECK(ctx, cudaGetLastError());
     return LCGS_B200_OK;
 }

@@ -90,7 +90,7 @@ def main():
             per[e.key] = per.get(e.key, 0.0) + t / 20.0 / 1000.0
     split = {"record_rebuild": 0.0, "blend_backward": 0.0, "preprocess_backward": 0.0, "other": 0.0}
     for k, v in per.items():
-        if "rebuild_records" in k or "tile_order" in k or "Memset" in k or "memset" in k:
+        if "build_records" in k or "tile_order" in k or "Memset" in k or "memset" in k:
             split["record_rebuild"] += v
         elif "blend_backward" in k:
             split["blend_backward"] += v

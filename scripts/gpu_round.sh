@@ -1,4 +1,4 @@
-# usage: [SKIP_TESTS=1] [SKIP_BENCH=1] bash scripts/gpu_round.sh <tag> [ncu] [tune] [blendab] [c5] [ncufull]   -- GPU tests + bench (+ optional ncu launch list, tuning sweep)
+# usage: [SKIP_TESTS=1] [SKIP_BENCH=1] bash scripts/gpu_round.sh <tag> [ncu] [tune] [c5] [ncufull]   -- GPU tests + bench (+ optional ncu launch list, tuning sweep)
 TAG=${1:-x}
 mkdir -p gpurun_out
 nvidia-smi -L | head -2; nproc
@@ -25,13 +25,6 @@ if [ "$a" = "tune" ]; then
 export LCGS_TUNING=1
 for v in 2 3 4 5 6 7 8; do LCGS_SORT_VARIANT=$v timeout 120 python scripts/tune_frame.py C3 2>&1 | tail -1; done
 for b in 32 64 256 1000000; do LCGS_EMIT_BIG=$b timeout 120 python scripts/tune_frame.py C3 2>&1 | tail -1; done
-unset LCGS_TUNING
-fi
-if [ "$a" = "blendab" ]; then
-export LCGS_TUNING=1
-LCGS_BLEND_P2=0 timeout 120 python scripts/tune_frame.py C3 2>&1 | tail -1
-for o in 5 6 7; do LCGS_BLEND2_OCC=$o timeout 120 python scripts/tune_frame.py C3 2>&1 | tail -1; done
-for o in 6 7 8 9 10; do LCGS_BLEND2_CPT=1 LCGS_BLEND2_OCC=$o timeout 120 python scripts/tune_frame.py C3 2>&1 | tail -1; done
 unset LCGS_TUNING
 fi
 if [ "$a" = "c5" ]; then

@@ -61,7 +61,7 @@ def excerpt(title, fname_part, start_pat, end_pat, before=0, after=0):
 
 
 excerpt("blend: the hit-evaluation loop (one (Gaussian, 8x8 patch) pair per iteration, two pixels per lane: FLO / BMSK walk of the ballot, "
-        "three broadcast LDS.128, power on FADD2 / FMUL2 / FFMA2, threshold compares, 2 x MUFU.EX2, blend)", "blend2_kernel<10, 1, 2>", r"FLO\.U32", r"@P\d BRA", before=1, after=0)
+        "three broadcast LDS.128, power on FADD2 / FMUL2 / FFMA2, threshold compares, 2 x MUFU.EX2, blend)", "blend2_kernel<10>", r"FLO\.U32", r"@P\d BRA", before=1, after=0)
 excerpt("onesweep<u64, 256x20, 7-bit digits, HI>: ranking of one item (7 x [LOP3 test, VOTE, SEL, LOP3], ATOMS by the group leader, SHFL)",
         "onesweep_pass_kernel<unsigned long long, 256, 20, 7, 2, false, true>", r"VOTE\.ANY", r"SHFL\.IDX", before=2, after=2)
 excerpt("onesweep<u64, 256x20>: the scatter -- keys by STS.64, values by LDGSTS (global -> shared, no register)",

@@ -2,10 +2,8 @@
 torch.autograd.gradcheck, the CUDA path's derivative header (csrc/lcgs_grad.cuh, built with g++ from
 tests/grad_mirror) against the reference's autograd, the ctypes Grad struct against the C header, and the SASS of
 the backward kernels."""
-import collections
 import ctypes as C
 import os
-import re
 import shutil
 import subprocess
 
@@ -17,6 +15,7 @@ from luisacomputegaussiansplatting_b200 import _capi, build, scenes
 from oracle import oracle as orc
 
 import torch_reference as tr
+from sass_ops import kernel_ops
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 REPO = os.path.dirname(HERE)
@@ -266,24 +265,10 @@ def test_ctypes_grad_matches_the_header(tmp_path):
 
 
 @pytest.mark.skipif(shutil.which("cuobjdump") is None, reason="cuobjdump not available")
-def test_backward_kernels_sass():
-    lib = build.build_native()
-    sass = subprocess.run(["cuobjdump", "-sass", lib], capture_output=True, text=True, check=True).stdout
-    funcs, name, archs = collections.OrderedDict(), None, set()
-    for ln in sass.splitlines():
-        m = re.search(r"arch = (sm_\w+)", ln)
-        if m:
-            archs.add(m.group(1))
-        m = re.search(r"Function : (\S+)", ln)
-        if m:
-            name = subprocess.run(["c++filt", m.group(1)], capture_output=True, text=True).stdout.strip()
-            funcs[name] = collections.Counter()
-        elif name:
-            m = re.match(r"\s+/\*[0-9a-f]{4}\*/\s+(?:@!?U?P\d+\s+)?([A-Z0-9_]+)", ln)
-            if m:
-                funcs[name][m.group(1)] += 1
+def test_backward_and_record_kernels_sass():
+    archs, funcs = kernel_ops(build.build_native())
     assert archs == {"sm_100a"}
-    for part in ("rebuild_records_kernel", "blend_backward_kernel", "preprocess_backward_kernel"):
+    for part in ("build_records_kernel", "blend_backward_kernel", "preprocess_backward_kernel"):
         hits = [v for k, v in funcs.items() if part in k]
         assert len(hits) == 1, part
         ops = hits[0]

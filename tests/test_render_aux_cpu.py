@@ -1,15 +1,14 @@
 """Static checks of the per-pixel aux outputs (no GPU needed): the ctypes frame matches the C header's layout, and the
 shipped library's aux blend kernel is what DESIGN.md says (sm_100a, no spills, depth staged with cp.async, packed FP32)."""
-import collections
 import ctypes
 import os
-import re
 import shutil
 import subprocess
 
 import pytest
 
 from luisacomputegaussiansplatting_b200 import _capi, build
+from sass_ops import kernel_ops
 
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -33,21 +32,7 @@ def test_ctypes_frame_matches_the_header(tmp_path):
 
 @pytest.mark.skipif(shutil.which("cuobjdump") is None, reason="cuobjdump not available")
 def test_aux_blend_kernel_sass():
-    lib = build.build_native()
-    sass = subprocess.run(["cuobjdump", "-sass", lib], capture_output=True, text=True, check=True).stdout
-    funcs, name, archs = collections.OrderedDict(), None, set()
-    for ln in sass.splitlines():
-        m = re.search(r"arch = (sm_\w+)", ln)
-        if m:
-            archs.add(m.group(1))
-        m = re.search(r"Function : (\S+)", ln)
-        if m:
-            name = subprocess.run(["c++filt", m.group(1)], capture_output=True, text=True).stdout.strip()
-            funcs[name] = collections.Counter()
-        elif name:
-            m = re.match(r"\s+/\*[0-9a-f]{4}\*/\s+(?:@!?U?P\d+\s+)?([A-Z0-9_]+)", ln)
-            if m:
-                funcs[name][m.group(1)] += 1
+    archs, funcs = kernel_ops(build.build_native())
     assert archs == {"sm_100a"}
     hits = [v for k, v in funcs.items() if "blend2_aux_kernel<" in k]
     assert len(hits) == 1, [k for k in funcs if "aux" in k]

@@ -1,35 +1,19 @@
 """Static checks on the SASS of the shipped library (cuobjdump; no GPU needed): the hot kernels are what DESIGN.md says
 they are -- sm_100a only, packed FP32 and asynchronous staging in the blend, no local-memory spills in the production
 geometries, no tensor-core or TMA instructions (no stage is a contraction; TMA staging was measured slower)."""
-import collections
-import os
-import re
 import shutil
-import subprocess
 
 import pytest
 
 from luisacomputegaussiansplatting_b200 import build
+from sass_ops import kernel_ops
 
 pytestmark = pytest.mark.skipif(shutil.which("cuobjdump") is None, reason="cuobjdump not available")
 
 
 @pytest.fixture(scope="module")
 def kernels():
-    lib = build.build_native()
-    sass = subprocess.run(["cuobjdump", "-sass", lib], capture_output=True, text=True, check=True).stdout
-    archs = set(re.findall(r"arch = (sm_\w+)", sass))
-    funcs, name = collections.OrderedDict(), None
-    for ln in sass.splitlines():
-        m = re.search(r"Function : (\S+)", ln)
-        if m:
-            name = re.sub(r"\(.*", "", subprocess.run(["c++filt", m.group(1)], capture_output=True, text=True).stdout.strip())
-            funcs[name] = collections.Counter()
-        elif name:
-            m = re.match(r"\s+/\*[0-9a-f]{4}\*/\s+(?:@!?U?P\d+\s+)?([A-Z0-9_]+)", ln)
-            if m:
-                funcs[name][m.group(1)] += 1
-    return archs, funcs
+    return kernel_ops(build.build_native())
 
 
 def find(funcs, part):
@@ -44,8 +28,8 @@ def test_library_is_sm_100a_only(kernels):
     assert len(funcs) >= 20
 
 
-def test_blend_kernel_uses_packed_fp32_and_async_staging(kernels):
-    ops = find(kernels[1], "blend2_kernel<10, 1, 2>")
+def test_production_blend_kernel_uses_packed_fp32_and_async_staging(kernels):
+    ops = find(kernels[1], "blend2_kernel<10>")
     assert ops["FFMA2"] >= 6 and ops["FMUL2"] >= 4 and ops["FADD2"] >= 2  # the pair's arithmetic of the hit loop
     assert ops["LDGSTS"] >= 3                                             # three 16-byte planes per candidate
     assert ops["MUFU"] >= 2 and ops["FLO"] >= 1 and ops["BMSK"] >= 1
