@@ -23,7 +23,7 @@ CSRC = os.path.join(HERE, "csrc")
 BUILD = os.path.join(CSRC, "build")
 LIB = os.path.join(HERE, "liblcgs_b200.so")
 SOURCES = ["capi.cu", "preprocess.cu", "scan.cu", "binning.cu", "sort.cu", "blend.cu", "backward.cu"]
-HEADERS = ["common.cuh", "lcgs_math.cuh", "lcgs_grad.cuh", "lookback.cuh", "blend_walk.cuh", os.path.join("..", "..", "include", "lcgs_b200.h")]
+HEADERS = ["common.cuh", "frame_plan.cuh", "lcgs_math.cuh", "lcgs_grad.cuh", "lookback.cuh", "blend_walk.cuh", os.path.join("..", "..", "include", "lcgs_b200.h")]
 
 NVCC = os.environ.get("LCGS_NVCC", "/usr/local/cuda/bin/nvcc")
 NVCC_FLAGS = [

@@ -93,10 +93,7 @@ __global__ void __launch_bounds__(256)
 // (lookback.cuh) and expand their Gaussians warp-cooperatively as above, 32 Gaussians per warp and step.
 // A ticket is only taken when the CTA is ready to load, count and publish at once: a tile that is held
 // back (e.g. taken ahead of time to prefetch it) stalls the look-back of every tile behind it.
-constexpr int kEmitThreads = 256;
-constexpr int kEmitWarps   = kEmitThreads / 32;
-constexpr int kEmitItems   = 4;  // Gaussians per thread and tile: chunk c of a warp is 32 consecutive ones
-constexpr int kEmitTile    = kEmitThreads * kEmitItems;
+constexpr int kEmitWarps = kEmitThreads / 32;  // kEmitThreads, kEmitTile: frame_plan.cuh
 
 __device__ __forceinline__ void red_shared_add(uint32_t addr, uint32_t v)
 {
@@ -107,17 +104,8 @@ __device__ __forceinline__ void red_shared_add(uint32_t addr, uint32_t v)
 // 10 000-tile rect is the whole kernel's tail: on a sparse band of the 8K frame 1 % of the Gaussians hold a third of the
 // instances, and a single warp was found emitting 52 000 instances while the rest of the GPU idled).  The warp only
 // reserves their output range (offsets are chained over the TRUE counts) and appends (entry, piece) work items;
-// emit_big_kernel then expands all pieces of kBigPiece instances, one CTA per piece, perfectly balanced.
-constexpr uint32_t kBigPiece = 2048;
-struct BigEntry {
-    uint32_t dst, cnt, xy0, w, dbits, idx, pad0, pad1;  // first output slot, tile count, x0 | y0<<16, rect width, depth bits, Gaussian
-};
-struct BigLists {
-    BigEntry* entries;
-    uint2*    pieces;    // (entry, piece index)
-    uint32_t* counters;  // [0] entries, [1] pieces
-    uint32_t  entry_capacity, piece_capacity, threshold;
-};
+// emit_big_kernel then expands all pieces of kBigPiece instances, one CTA per piece, perfectly balanced (BigLists,
+// frame_plan.cuh).
 
 // Tile-bit digit histograms of up to 32 emitted keys (one per lane; every lane of the warp must call).  Consecutive lanes
 // emit consecutive tiles of one Gaussian, so the upper digit is counted once per run of equal digits.
@@ -165,7 +153,7 @@ __device__ __forceinline__ void duplicate_keys_sorted_body(const uint32_t* __res
     // digit histograms of the tile bits of the emitted keys (two passes at most: the tile sort then skips
     // its histogram kernel).  Consecutive lanes emit consecutive tiles of one Gaussian, so the upper digit
     // is aggregated per run of equal digits.
-    __shared__ uint32_t s_hist[2 * 512];
+    __shared__ uint32_t s_hist[kEmitHistPasses * kMaxRadix];
     __shared__ uint32_t s_wsum[kEmitWarps];
     __shared__ uint32_t s_base;
     __shared__ uint32_t s_tk;
@@ -377,7 +365,7 @@ __global__ void __launch_bounds__(kEmitThreads)
     emit_big_kernel(uint32_t gx, uint32_t row0, unsigned long long* __restrict__ keys, uint32_t* __restrict__ vals, size_t capacity,
                     const __grid_constant__ SortDigits digits, bool exact_div, const __grid_constant__ BigLists big)
 {
-    __shared__ uint32_t s_hist[2 * 512];
+    __shared__ uint32_t s_hist[kEmitHistPasses * kMaxRadix];
     const bool     do_hist = digits.hist != nullptr;
     const int      nbins   = do_hist ? (digits.num_passes << digits.radix_bits) : 0;
     const int      tid = threadIdx.x, lane = tid & 31;
@@ -485,34 +473,12 @@ int launch_duplicate_keys(lcgs_b200_ctx* ctx, int P, int W, int H, const float* 
     return LCGS_B200_OK;
 }
 
-static size_t emit_ws_layout(int P, size_t capacity, uint32_t* threshold, uint32_t* entry_capacity, uint32_t* piece_capacity,
-                             size_t* entries_bytes)
-{
-    *threshold         = (uint32_t)LCGS_TUNE_INT("LCGS_EMIT_BIG", 128);
-    const size_t by_p  = (size_t)(P > 0 ? P : 1), by_cap = capacity / ((size_t)*threshold + 1) + 1;
-    *entry_capacity    = (uint32_t)(by_p < by_cap ? by_p : by_cap);
-    *piece_capacity    = (uint32_t)(capacity / kBigPiece + *entry_capacity + 1);
-    *entries_bytes     = (size_t)*entry_capacity * sizeof(BigEntry);
-    return *entries_bytes + (size_t)*piece_capacity * sizeof(uint2);
-}
-
-size_t emit_ws_bytes(int P, size_t capacity)
-{
-    uint32_t t, e, p;
-    size_t   b;
-    return emit_ws_layout(P, capacity, &t, &e, &p, &b);
-}
-
 int launch_duplicate_keys_sorted(lcgs_b200_ctx* ctx, const uint32_t* d_m, int P, int W, int H, int num_rows,
                                  const SortedPairsU32& sorted, const uint2* rects, uint64_t* keys, uint32_t* vals,
-                                 size_t capacity, int row0, const SortDigits* digits, cudaStream_t s, bool cleared)
+                                 size_t capacity, int row0, const FramePlan& fp, cudaStream_t s)
 {
     if (P <= 0) return LCGS_B200_OK;
-    // fused histograms need the digits to live in the tile id (key bits >= 32) and at most two passes
-    SortDigits dg{};
-    if (digits && digits->hist && digits->num_passes >= 1 && digits->num_passes <= 2 && digits->radix_bits <= 9 &&
-        digits->shift[0] >= 32)
-        dg = *digits;
+    SortDigits dg = producer_digits(fp.tile);
     if (dg.num_passes < 2) dg.shift[1] = 32;  // unused, but keep the kernel's shift amounts in range
     const uint32_t gx = (uint32_t)((W + 15) / 16);
     // index inside a rect / rect width as a multiply-high: exact while j * w < 2^32; j < w * h with w <= gx and
@@ -521,29 +487,7 @@ int launch_duplicate_keys_sorted(lcgs_b200_ctx* ctx, const uint32_t* d_m, int P,
     // path (division, owner search by shuffle) is covered by the extreme-aspect test (640000 x 48 pixels).
     const uint32_t gy        = (uint32_t)(num_rows > 0 ? num_rows : (H + 15) / 16);
     const bool     exact_div = (unsigned long long)gx * gx * gy < 0x100000000ull;
-    const uint32_t tiles     = (uint32_t)(((size_t)P + kEmitTile - 1) / kEmitTile);
-    static_assert(kEmitTile == 1024, "scan.cu: emit_status_words");
-    int                 rc;
-    uint32_t*           ticket = ctx->d_scalars + LCGS_SCALAR_DUP_TICKET;
-    unsigned long long* status;
-    if (cleared) {
-        // scan_frame_prepare: the emission's status words follow the scan's (2 per 2048 Gaussians) and are zero already
-        status = (unsigned long long*)ctx->scan_ws.ptr + 2 * (((size_t)P + 2047) / 2048);
-    } else {
-        if ((rc = ws_reserve(ctx, ctx->scan_ws, (size_t)tiles * sizeof(unsigned long long)))) return rc;
-        status = (unsigned long long*)ctx->scan_ws.ptr;
-        LCGS_CUDA_CHECK(ctx, cudaMemsetAsync(status, 0, (size_t)tiles * sizeof(unsigned long long), s));
-        LCGS_CUDA_CHECK(ctx, cudaMemsetAsync(ticket, 0, 3 * sizeof(uint32_t), s));  // ticket + the two big-list counters
-    }
-    // side lists of the big Gaussians: each holds more than `threshold` instances, so a frame within its list capacity
-    // has at most capacity / (threshold + 1) of them (a frame that overflows is reported as such; entries beyond are dropped)
-    BigLists big;
-    size_t   entries_bytes;
-    const size_t emit_bytes = emit_ws_layout(P, capacity, &big.threshold, &big.entry_capacity, &big.piece_capacity, &entries_bytes);
-    if ((rc = ws_reserve(ctx, ctx->emit_ws, emit_bytes))) return rc;
-    big.entries  = (BigEntry*)ctx->emit_ws.ptr;
-    big.pieces   = (uint2*)((char*)ctx->emit_ws.ptr + entries_bytes);
-    big.counters = ticket + 1;
+    const uint32_t tiles     = (uint32_t)emit_tiles(P);
     // persistent CTAs; tiles are handed out by ticket, so CTAs that are not resident yet hold nothing back
     const uint32_t max_blocks = (uint32_t)ctx->num_sms * (uint32_t)LCGS_TUNE_INT("LCGS_EMIT_CTAS", 6);
     const uint32_t blocks     = tiles < max_blocks ? tiles : max_blocks;
@@ -551,16 +495,17 @@ int launch_duplicate_keys_sorted(lcgs_b200_ctx* ctx, const uint32_t* d_m, int P,
     auto* const k64 = reinterpret_cast<unsigned long long*>(keys);
     if (big_path) {
         auto kern = exact_div ? duplicate_keys_sorted_big_kernel<true> : duplicate_keys_sorted_big_kernel<false>;
-        kern<<<blocks, kEmitThreads, 0, s>>>(d_m, (uint32_t)P, gx, (uint32_t)row0, sorted, rects, status, ticket, k64, vals, capacity, dg, big);
+        kern<<<blocks, kEmitThreads, 0, s>>>(d_m, (uint32_t)P, gx, (uint32_t)row0, sorted, rects, fp.emit_status, fp.emit_ticket, k64, vals,
+                                             capacity, dg, fp.big);
     } else {
         auto kern = exact_div ? duplicate_keys_sorted_kernel<true> : duplicate_keys_sorted_kernel<false>;
         if (exact_div && dg.hist && dg.num_passes == 2 && LCGS_TUNE_INT("LCGS_EMIT_HIST2", 1)) kern = duplicate_keys_sorted_kernel<true, true>;
-        kern<<<blocks, kEmitThreads, 0, s>>>(d_m, (uint32_t)P, gx, (uint32_t)row0, sorted, rects, status, ticket, k64, vals, capacity, dg);
+        kern<<<blocks, kEmitThreads, 0, s>>>(d_m, (uint32_t)P, gx, (uint32_t)row0, sorted, rects, fp.emit_status, fp.emit_ticket, k64, vals,
+                                             capacity, dg);
     }
     LCGS_CUDA_CHECK(ctx, cudaGetLastError());
     if (big_path) {
-        emit_big_kernel<<<max_blocks, kEmitThreads, 0, s>>>(gx, (uint32_t)row0, reinterpret_cast<unsigned long long*>(keys), vals,
-                                                            capacity, dg, exact_div, big);
+        emit_big_kernel<<<max_blocks, kEmitThreads, 0, s>>>(gx, (uint32_t)row0, k64, vals, capacity, dg, exact_div, fp.big);
         LCGS_CUDA_CHECK(ctx, cudaGetLastError());
     }
     return LCGS_B200_OK;
@@ -654,7 +599,7 @@ int launch_checksum_u32(lcgs_b200_ctx* ctx, const void* data, size_t num_words, 
     return LCGS_B200_OK;
 }
 
-// ---- one clear for everything a fused frame needs zeroed (ClearList, common.cuh) ---------------------------------
+// ---- one clear for everything a fused frame needs zeroed (ClearList, frame_plan.cuh) -----------------------------
 __global__ void __launch_bounds__(256) frame_clear_kernel(const __grid_constant__ ClearList cl)
 {
     const uint32_t gtid = blockIdx.x * blockDim.x + threadIdx.x, gsize = gridDim.x * blockDim.x;

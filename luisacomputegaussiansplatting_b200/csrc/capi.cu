@@ -114,6 +114,21 @@ static OrderWs order_ws_views(lcgs_b200_ctx* ctx, int P)
     return o;
 }
 
+static uint32_t big_threshold() { return (uint32_t)LCGS_TUNE_INT("LCGS_EMIT_BIG", (int)kBigThreshold); }
+
+// The fused frame's plan (frame_plan.cuh): both sorts' geometry, then every scratch region, ticket and histogram placed in
+// the workspaces reserve_all reserved, before the first kernel.
+static int plan_frame(lcgs_b200_ctx* ctx, int P, const lcgs_b200_frame* fr, const FrameGeom& g, FramePlan* fp)
+{
+    int rc;
+    if ((rc = sort_plan_geometry(ctx, (size_t)P, 0, 32, &fp->depth))) return rc;
+    if ((rc = sort_plan_geometry(ctx, fr->list_capacity, 32, g.end_bit, &fp->tile))) return rc;
+    const char* err = place_frame(fp, P, fr->list_capacity, big_threshold(), ctx->scan_ws, ctx->sort_ws, ctx->emit_ws,
+                                  ctx->d_scalars, fr->ranges, (size_t)g.num_tiles);
+    LCGS_REQUIRE(ctx, !err, err);
+    return LCGS_B200_OK;
+}
+
 // scan -> [depth sort of the Gaussians] -> duplicate -> sort -> ranges -> blend, all on device-resident counts.
 // depth_ordered = false: the reference's data flow (emit in index order, sort all key bits).
 // depth_ordered = true : sort the Gaussians by depth, emit in that order, stable-sort by tile bits only;
@@ -126,33 +141,24 @@ static int splat_tail(lcgs_b200_ctx* ctx, int P, const lcgs_b200_frame* fr, cons
     uint32_t* d_m = ctx->d_scalars + LCGS_SCALAR_NUM_TOUCHING;
     if (depth_ordered) {
         const OrderWs o = order_ws_views(ctx, P);
-        SortDigits    dg32, dg64;
-        // Plan first: both sorts' geometry and workspace, the scan's and the emission's status words, tickets and the
-        // ranges buffer are known before the first kernel, so ONE kernel zeroes all of it.
         // Depth keys are stored relative to bits(0.2f) (kDepthKeyBase): 27 bits for any depth below 13107, so the
         // fourth 9-bit pass normally skips itself.  The compaction kernel also fills the depth sort's digit
         // histograms, the emission kernel those of the tile sort.
-        ClearList cl;
-        if ((rc = sort_prepare_frame(ctx, (size_t)P, fr->list_capacity, g.end_bit, &dg32, &dg64, &cl))) return rc;
-        if ((rc = scan_frame_prepare(ctx, P, &cl))) return rc;
-        cl.add(ctx->d_scalars + LCGS_SCALAR_SCAN_TICKET, 10 * sizeof(uint32_t));  // scan ticket, 8 sort tickets, spare
-        cl.add(ctx->d_scalars + LCGS_SCALAR_DUP_TICKET, 3 * sizeof(uint32_t));    // emission ticket + big-list counters
-        cl.add(fr->ranges, (size_t)g.num_tiles * 2 * sizeof(uint32_t));
-        if ((rc = launch_clear(ctx, cl, s))) return rc;
-        if ((rc = launch_scan_compact(ctx, fr->tiles_touched, fr->depth, P, fr->point_offsets, o.ckeys, o.cvals, d_n, d_m, &dg32, s, true)))
+        FramePlan fp;
+        if ((rc = plan_frame(ctx, P, fr, g, &fp))) return rc;
+        if ((rc = launch_clear(ctx, fp.clear, s))) return rc;
+        if ((rc = launch_scan_compact(ctx, fr->tiles_touched, fr->depth, P, fr->point_offsets, o.ckeys, o.cvals, d_n, d_m, fp, s)))
             return rc;
         mark(ctx, s);
-        const bool hist32 = dg32.hist && dg32.num_passes <= 4;
         SortedPairsU32 sorted;
-        if ((rc = sort_run_u32(ctx, o.ckeys, o.skeys, o.cvals, o.svals, d_m, (size_t)P, hist32, &sorted, s))) return rc;
+        if ((rc = sort_run_u32(ctx, fp.depth, o.ckeys, o.skeys, o.cvals, o.svals, d_m, (size_t)P, &sorted, s))) return rc;
         mark(ctx, s);
-        const bool hist64 = dg64.hist && dg64.num_passes >= 1 && dg64.num_passes <= 2;
         if ((rc = launch_duplicate_keys_sorted(ctx, d_m, P, g.W, g.H, g.row1 - g.row0, sorted, o.rects, fr->point_list_keys_unsorted,
-                                               fr->point_list_unsorted, fr->list_capacity, g.row0, hist64 ? &dg64 : nullptr, s, true)))
+                                               fr->point_list_unsorted, fr->list_capacity, g.row0, fp, s)))
             return rc;
         mark(ctx, s);
-        if ((rc = sort_run_u64(ctx, fr->point_list_keys_unsorted, fr->point_list_keys, fr->point_list_unsorted,
-                               fr->point_list, d_n, fr->list_capacity, hist64, s)))
+        if ((rc = sort_run_u64(ctx, fp.tile, fr->point_list_keys_unsorted, fr->point_list_keys, fr->point_list_unsorted,
+                               fr->point_list, d_n, fr->list_capacity, s)))
             return rc;
         mark(ctx, s);
     } else {
@@ -197,15 +203,15 @@ static int reserve_all(lcgs_b200_ctx* ctx, int P, size_t max_instances)
 {
     int rc;
     if (P > 0) {
+        const FrameWsBytes b = frame_ws_bytes(P, max_instances, big_threshold());
         if ((rc = ws_reserve(ctx, ctx->record_ws, (size_t)P * kRecordFloat4s * sizeof(float4)))) return rc;
-        // look-back status: 2 chains x P/2048 tiles (scan + compaction), P/256 tiles (instance emission)
-        if ((rc = ws_reserve(ctx, ctx->scan_ws, (((size_t)P + 255) / 256) * sizeof(unsigned long long)))) return rc;
+        if ((rc = ws_reserve(ctx, ctx->scan_ws, b.scan))) return rc;
         if ((rc = ws_reserve(ctx, ctx->order_ws, (size_t)P * 24))) return rc;
-        if ((rc = ws_reserve(ctx, ctx->emit_ws, emit_ws_bytes(P, max_instances)))) return rc;
+        if ((rc = ws_reserve(ctx, ctx->emit_ws, b.emit))) return rc;
+        if ((rc = ws_reserve(ctx, ctx->sort_ws, b.sort))) return rc;
+    } else if (max_instances > 0) {
+        if ((rc = ws_reserve(ctx, ctx->sort_ws, sort_temp_bytes(max_instances)))) return rc;
     }
-    const size_t sort_items = max_instances > (size_t)(P > 0 ? P : 0) ? max_instances : (size_t)(P > 0 ? P : 0);
-    if (sort_items > 0)
-        if ((rc = ws_reserve(ctx, ctx->sort_ws, sort_temp_bytes(sort_items)))) return rc;
     return LCGS_B200_OK;
 }
 
@@ -272,7 +278,6 @@ int lcgs_b200_ctx_destroy(lcgs_b200_ctx* ctx)
     if (ctx->tile_order_ws.ptr) cudaFree(ctx->tile_order_ws.ptr);
     if (ctx->emit_ws.ptr) cudaFree(ctx->emit_ws.ptr);
     if (ctx->grad_ws.ptr) cudaFree(ctx->grad_ws.ptr);
-    sort_free_plans(ctx);
     for (int i = 0; i < 16; i++)
         if (ctx->ev[i]) cudaEventDestroy(ctx->ev[i]);
     for (int i = 0; i < 3; i++)

@@ -6,6 +6,7 @@
 #include <stdio.h>
 
 #include "../../include/lcgs_b200.h"
+#include "frame_plan.cuh"
 #include "lcgs_math.cuh"
 
 namespace lcgs_b200 {
@@ -35,19 +36,6 @@ __device__ __forceinline__ void write_record(float4* rec, const Splat2D& s, floa
 // depth < 0.2 * 2^16 they fit in 27 bits = three 9-bit digits, and the fourth pass skips itself.
 constexpr uint32_t kDepthKeyBase = 0x3E4CCCCDu;
 
-// Radix sort (onesweep, sort.cu): at most 8 passes (64 key bits in 9-bit digits).
-constexpr int kMaxSortPasses  = 8;
-
-// Scan geometry (decoupled look-back).
-constexpr int kScanThreads = 256;
-constexpr int kScanItems   = 16;
-constexpr int kScanTile    = kScanThreads * kScanItems;
-
-struct Workspace {
-    void*  ptr   = nullptr;
-    size_t bytes = 0;
-};
-
 }  // namespace lcgs_b200
 
 // The opaque context of the C ABI.
@@ -55,8 +43,7 @@ struct lcgs_b200_ctx {
     int          device     = 0;
     int          num_sms    = lcgs_b200::kNumSMs;
     char         last_error[256];
-    // device scalars: [0] num_rendered (instances), [1] Gaussians touching a tile, [2..] tickets, [13] overflow flag
-    uint32_t*    d_scalars  = nullptr;
+    uint32_t*    d_scalars  = nullptr;  // LCGS_SCALAR_* (frame_plan.cuh)
     uint32_t*    h_scalars  = nullptr;  // pinned mirror
     // workspaces, grown geometrically and never shrunk (like ensure_*_temp_buffer,
     // lcgs/src/gs_tile_splatter/impl.cpp:31-61)
@@ -73,22 +60,10 @@ struct lcgs_b200_ctx {
     int          ev_count   = 0;
     int          ev_valid   = 0;
     bool         sweep_attr_set[2][32] = {};  // onesweep variants whose shared-memory opt-in has been done
-    void*        plan32 = nullptr;   // prepared sorts of the fused path (sort.cu)
-    void*        plan64 = nullptr;
     cudaEvent_t  ev_sort[3] = { nullptr, nullptr, nullptr };  // before histogram, before passes, after passes
     int          sort_passes = 0;
     int          ev_sort_valid = 0;
 };
-
-#define LCGS_SCALAR_NUM_RENDERED 0
-#define LCGS_SCALAR_NUM_TOUCHING 1   /* Gaussians with tiles_touched > 0 (fused path) */
-#define LCGS_SCALAR_SCAN_TICKET  2
-#define LCGS_SCALAR_SORT_TICKET  3   /* .. 3 + kMaxSortPasses - 1 */
-#define LCGS_SCALAR_DUP_TICKET   16  /* + 17, 18: entry / piece counters of the emission's big-Gaussian lists */
-#define LCGS_SCALAR_OVERFLOW     13  /* 1 iff the last frame's num_rendered exceeded its list_capacity (device-side test) */
-#define LCGS_SCALAR_CAPACITY     14  /* that frame's list_capacity (clamped to 2^32-1), written in-stream; = OVERFLOW + 1 */
-#define LCGS_SCALAR_PEER_TIMEOUTS 15  /* sticky: peer waits that gave up (lcgs_b200_peer_error) */
-#define LCGS_NUM_SCALARS         24
 
 #define LCGS_CUDA_CHECK(ctx, expr)                                                                   \
     do {                                                                                             \
@@ -122,59 +97,33 @@ int tuning_env_int(const char* name, int fallback);
 #define LCGS_TUNE_INT(name, fallback) (fallback)
 #endif
 
-// Everything a fused frame needs zeroed before its first kernel -- digit histograms, look-back status words of the two
-// sorts, of the scan and of the emission, tickets, the ranges buffer -- collected while the frame is planned and cleared
-// by ONE kernel (nine cudaMemsetAsync nodes per frame cost ~25 us of a 1.5 ms frame).
-struct ClearList {
-    static constexpr int kMax = 8;
-    void*    ptr[kMax];
-    uint32_t words[kMax];  // 32-bit words; ptr 4-byte aligned
-    int      n = 0;
-    void add(void* p, size_t bytes)
-    {
-        if (bytes == 0 || n >= kMax) return;
-        ptr[n]   = p;
-        words[n] = (uint32_t)((bytes + 3) / 4);
-        n++;
-    }
-};
 int launch_clear(lcgs_b200_ctx* ctx, const ClearList& cl, cudaStream_t s);
 
 // stage launchers (one group per .cu); all enqueue on `s` and return an lcgs_b200_status
 int launch_preprocess_fused(lcgs_b200_ctx* ctx, const lcgs_b200_scene* sc, const lcgs_b200_view_params* vp,
                             const lcgs_b200_frame* fr, float4* records, uint2* rects, cudaStream_t s);
-struct SortDigits;
-// `cleared`: the status words (scan_ws) and the ticket have been zeroed by the frame's clear kernel (scan_frame_prepare)
+// the fused frame's stages take their scratch, tickets and histograms from its plan (frame_plan.cuh)
 int launch_scan_compact(lcgs_b200_ctx* ctx, const uint32_t* tiles_touched, const float* depth, int P, uint32_t* offsets,
-                        uint32_t* ckeys, uint32_t* cvals, uint32_t* d_total, uint32_t* d_count, const SortDigits* digits,
-                        cudaStream_t s, bool cleared = false);
-// reserves the look-back status words of the scan+compaction and of the emission (disjoint) and lists them for clearing
-int scan_frame_prepare(lcgs_b200_ctx* ctx, int P, ClearList* cl);
-struct SortedPairsU32;
-int launch_duplicate_keys_sorted(lcgs_b200_ctx* ctx, const uint32_t* d_m, int P, int W, int H, int num_rows,
-                                 const SortedPairsU32& sorted, const uint2* rects, uint64_t* keys, uint32_t* vals,
-                                 size_t capacity, int row0, const SortDigits* digits, cudaStream_t s, bool cleared = false);
-// digit layout of a prepared sort, for kernels that accumulate its histograms while producing the keys
-struct SortDigits {
-    uint32_t* hist;  // [num_passes][1 << radix_bits], zeroed
-    int       num_passes, radix_bits;
-    int       shift[kMaxSortPasses];
-    uint32_t  mask[kMaxSortPasses];
-};
-void sort_free_plans(lcgs_b200_ctx* ctx);
-// both sorts of the fused frame planned at once (depth sort of <= P Gaussians over 32 bits, tile sort of <= L instances over
-// key bits [32, end_bit)): one workspace reservation, disjoint status words and tickets, everything to zero listed in `cl`
-int sort_prepare_frame(lcgs_b200_ctx* ctx, size_t P, size_t L, int end_bit, SortDigits* dg32, SortDigits* dg64, ClearList* cl);
+                        uint32_t* ckeys, uint32_t* cvals, uint32_t* d_total, uint32_t* d_count, const FramePlan& fp,
+                        cudaStream_t s);
 // Where a u32 sort left its result: (keys, vals), or (alt_keys, alt_vals) when the last pass found all
 // its keys in digit 0 and skipped itself -- the case iff last_hist && *last_hist == n (device-side test).
 struct SortedPairsU32 {
     const uint32_t *keys, *vals, *alt_keys, *alt_vals, *last_hist;
 };
 __device__ __forceinline__ bool sorted_in_alt(const SortedPairsU32& r, uint32_t n) { return r.last_hist && __ldg(r.last_hist) == n; }
-int sort_run_u32(lcgs_b200_ctx* ctx, uint32_t* keys_a, uint32_t* keys_b, uint32_t* vals_a, uint32_t* vals_b,
-                 const uint32_t* d_n, size_t capacity, bool hist_ready, SortedPairsU32* res, cudaStream_t s);
-int sort_run_u64(lcgs_b200_ctx* ctx, const uint64_t* keys_in, uint64_t* keys_out, const uint32_t* vals_in, uint32_t* vals_out,
-                 const uint32_t* d_n, size_t capacity, bool hist_ready, cudaStream_t s);
+int launch_duplicate_keys_sorted(lcgs_b200_ctx* ctx, const uint32_t* d_m, int P, int W, int H, int num_rows,
+                                 const SortedPairsU32& sorted, const uint2* rects, uint64_t* keys, uint32_t* vals,
+                                 size_t capacity, int row0, const FramePlan& fp, cudaStream_t s);
+// digit cut, kernel geometry and tile count of a sort over `bound` pairs; no memory, no ticket
+template <typename KeyT>
+int sort_plan_geometry(lcgs_b200_ctx* ctx, size_t bound, int begin_bit, int end_bit, SortPlan<KeyT>* plan);
+// Sorts (keys_a, vals_a) using (keys_b, vals_b) as the ping-pong partner; both pairs are scratch.  The
+// result is in res->keys/vals, or in res->alt_* when the last pass skipped itself (SortedPairsU32).
+int sort_run_u32(lcgs_b200_ctx* ctx, const SortPlan<uint32_t>& plan, uint32_t* keys_a, uint32_t* keys_b, uint32_t* vals_a,
+                 uint32_t* vals_b, const uint32_t* d_n, size_t capacity, SortedPairsU32* res, cudaStream_t s);
+int sort_run_u64(lcgs_b200_ctx* ctx, const SortPlan<unsigned long long>& plan, const uint64_t* keys_in, uint64_t* keys_out,
+                 const uint32_t* vals_in, uint32_t* vals_out, const uint32_t* d_n, size_t capacity, cudaStream_t s);
 int launch_sh(lcgs_b200_ctx* ctx, int P, int deg, const float* cam_pos, const float* pos, const float* sh, float* color,
               cudaStream_t s);
 int launch_project(lcgs_b200_ctx* ctx, int P, const float* pos, const float* scale, const float* rotq,
@@ -190,8 +139,6 @@ int launch_scan(lcgs_b200_ctx* ctx, const uint32_t* in, uint32_t* out, size_t n,
 int launch_duplicate_keys(lcgs_b200_ctx* ctx, int P, int W, int H, const float* means_2d, const uint32_t* offsets,
                           const int32_t* radii, const float* depth, uint64_t* keys, uint32_t* vals, size_t capacity,
                           int row0, int row1, cudaStream_t s);
-size_t sort_temp_bytes(size_t n);
-size_t emit_ws_bytes(int P, size_t capacity);
 int launch_sort(lcgs_b200_ctx* ctx, const uint64_t* keys_in, uint64_t* keys_out, const uint32_t* vals_in,
                 uint32_t* vals_out, size_t n_host, const uint32_t* d_n, size_t capacity, int begin_bit, int end_bit,
                 cudaStream_t s);

@@ -129,9 +129,6 @@ __device__ __forceinline__ ScanPair block_scan_pair(ScanPair v, ScanPair* s_warp
     return ScanPair{ pre.a + xa - v.a, pre.b + xb - v.b };
 }
 
-constexpr int kCompactItems = 8;                          // per thread
-constexpr int kCompactTile  = kScanThreads * kCompactItems;  // 2048 Gaussians per CTA
-
 __global__ void __launch_bounds__(kScanThreads)
     scan_compact_kernel(const uint32_t* __restrict__ tiles_touched, const float* __restrict__ depth, uint32_t n,
                         uint32_t num_tiles, uint32_t* __restrict__ offsets, uint32_t* __restrict__ ckeys,
@@ -139,7 +136,7 @@ __global__ void __launch_bounds__(kScanThreads)
                         uint32_t* ticket, uint32_t* d_total, uint32_t* d_count, const __grid_constant__ SortDigits digits, int vec_ok)
 {
     // digit histograms of the depth keys this CTA compacts (the depth sort then skips its histogram kernel)
-    __shared__ uint32_t s_hist[4 * 512];
+    __shared__ uint32_t s_hist[kCompactHistPasses * kMaxRadix];
     // the CTA's compacted (key, index) pairs, staged so that they leave as two coalesced runs
     __shared__ uint32_t s_key[kCompactTile], s_idx[kCompactTile];
     const bool          do_hist = digits.hist != nullptr;
@@ -222,7 +219,7 @@ __global__ void __launch_bounds__(kScanThreads)
         cvals[base_cnt + i] = s_idx[i];
         if (do_hist) {
 #pragma unroll
-            for (int p = 0; p < 4; p++)
+            for (int p = 0; p < kCompactHistPasses; p++)
                 if (p < digits.num_passes) atomicAdd(&s_hist[(p << digits.radix_bits) + ((key >> digits.shift[p]) & digits.mask[p])], 1u);
         }
     }
@@ -236,25 +233,10 @@ __global__ void __launch_bounds__(kScanThreads)
     }
 }
 
-// scan_ws of a fused frame: [2 x scan tiles][emission tiles] 64-bit status words
-static inline size_t scan_status_words(int P) { return 2 * (((size_t)(P > 0 ? P : 1) + kCompactTile - 1) / kCompactTile); }
-static inline size_t emit_status_words(int P) { return ((size_t)(P > 0 ? P : 1) + 1023) / 1024; }  // kEmitTile (binning.cu)
-
-int scan_frame_prepare(lcgs_b200_ctx* ctx, int P, ClearList* cl)
-{
-    const size_t bytes = (scan_status_words(P) + emit_status_words(P)) * sizeof(unsigned long long);
-    int          rc    = ws_reserve(ctx, ctx->scan_ws, bytes);
-    if (rc) return rc;
-    cl->add(ctx->scan_ws.ptr, bytes);
-    return LCGS_B200_OK;
-}
-
 int launch_scan_compact(lcgs_b200_ctx* ctx, const uint32_t* tiles_touched, const float* depth, int P, uint32_t* offsets,
-                        uint32_t* ckeys, uint32_t* cvals, uint32_t* d_total, uint32_t* d_count, const SortDigits* digits,
-                        cudaStream_t s, bool cleared)
+                        uint32_t* ckeys, uint32_t* cvals, uint32_t* d_total, uint32_t* d_count, const FramePlan& fp,
+                        cudaStream_t s)
 {
-    SortDigits dg{};
-    if (digits && digits->hist && digits->num_passes <= 4 && digits->radix_bits <= 9) dg = *digits;
     if (P <= 0) {
         LCGS_CUDA_CHECK(ctx, cudaMemsetAsync(d_total, 0, sizeof(uint32_t), s));
         LCGS_CUDA_CHECK(ctx, cudaMemsetAsync(d_count, 0, sizeof(uint32_t), s));
@@ -262,18 +244,11 @@ int launch_scan_compact(lcgs_b200_ctx* ctx, const uint32_t* tiles_touched, const
     }
     // 16-byte aligned buffers (any cudaMalloc'ed array) take the vector path, sub-allocated ones the scalar one
     const int vec_ok = ((((uintptr_t)tiles_touched) | ((uintptr_t)offsets) | ((uintptr_t)depth)) & 15) == 0;
-    const uint32_t tiles = (uint32_t)(((size_t)P + kCompactTile - 1) / kCompactTile);
-    uint32_t* ticket = ctx->d_scalars + LCGS_SCALAR_SCAN_TICKET;
-    if (!cleared) {
-        int rc = ws_reserve(ctx, ctx->scan_ws, (size_t)tiles * 2 * sizeof(unsigned long long));
-        if (rc) return rc;
-        LCGS_CUDA_CHECK(ctx, cudaMemsetAsync(ctx->scan_ws.ptr, 0, (size_t)tiles * 2 * sizeof(unsigned long long), s));
-        LCGS_CUDA_CHECK(ctx, cudaMemsetAsync(ticket, 0, sizeof(uint32_t), s));
-    }
-    auto* st = (unsigned long long*)ctx->scan_ws.ptr;
+    const uint32_t tiles = (uint32_t)compact_tiles(P);
     const uint32_t max_blocks = (uint32_t)ctx->num_sms * (uint32_t)LCGS_TUNE_INT("LCGS_SCAN_CTAS", 6);  // persistent: 6 x 256 threads per SM
-    scan_compact_kernel<<<tiles < max_blocks ? tiles : max_blocks, kScanThreads, 0, s>>>(tiles_touched, depth, (uint32_t)P, tiles, offsets, ckeys, cvals, st,
-                                                       st + tiles, ticket, d_total, d_count, dg, vec_ok);
+    scan_compact_kernel<<<tiles < max_blocks ? tiles : max_blocks, kScanThreads, 0, s>>>(tiles_touched, depth, (uint32_t)P, tiles, offsets, ckeys, cvals,
+                                                       fp.scan_sum, fp.scan_count, fp.scan_ticket, d_total, d_count,
+                                                       producer_digits(fp.depth), vec_ok);
     LCGS_CUDA_CHECK(ctx, cudaGetLastError());
     return LCGS_B200_OK;
 }

@@ -23,8 +23,6 @@
 
 namespace lcgs_b200 {
 
-constexpr int      kMaxRadixBits    = 9;
-constexpr int      kMaxRadix        = 1 << kMaxRadixBits;
 constexpr uint32_t kStatusAggregate = 1u << 30;
 constexpr uint32_t kStatusInclusive = 2u << 30;
 constexpr uint32_t kStatusValueMask = (1u << 30) - 1u;
@@ -79,13 +77,6 @@ __device__ __forceinline__ uint32_t key_digit(uint32_t key, int shift, uint32_t 
 __device__ __forceinline__ uint32_t key_digit_hi(uint32_t key, int, uint32_t) { return key; }  // unreachable (shift < 32)
 __device__ __forceinline__ unsigned long long key_ones(unsigned long long) { return ~0ull; }
 __device__ __forceinline__ uint32_t           key_ones(uint32_t) { return ~0u; }
-
-struct SortPassInfo {
-    int      num_passes;
-    int      radix_bits;
-    int      shift[kMaxSortPasses];
-    uint32_t mask[kMaxSortPasses];
-};
 
 // ---- upfront histogram of every pass's digit ---------------------------------------------------
 template <typename KeyT>
@@ -448,9 +439,6 @@ static const SweepVariant<uint32_t> kSweep32[] = {
     LCGS_SWEEP32(512, 8, 9, 2, true),    // 2: MATCH.ANY ranking (the earlier default)
 #endif
 };
-constexpr int kMinSweepTile = 2048;
-constexpr size_t kHistSlotBytes = (size_t)kMaxSortPasses * kMaxRadix * sizeof(uint32_t);  // 16 KB, 256-byte multiple
-
 template <typename KeyT>
 struct SweepTable;
 template <>
@@ -480,45 +468,8 @@ static int sweep_variant_index(int bits)
     return 0;                                            // depth keys: 9-bit digits, one 8192-pair tile per SM
 }
 
-// workspace layout: [hist slot 0][hist slot 1][status: passes*tiles*RADIX u32][tmp keys][tmp vals], a
-// hist slot being [kMaxSortPasses][512] u32.  The depth sort of the fused frame uses slot 0, every other
-// sort slot 1: the consumers of the depth-sorted list still read the depth sort's last histogram (to
-// learn whether its last pass skipped itself) after the tile sort has been prepared.
-static size_t sort_ws_layout(size_t n, size_t key_bytes, size_t* off_status, size_t* off_keys, size_t* off_vals)
-{
-    const size_t tiles = (n + kMinSweepTile - 1) / kMinSweepTile;
-    size_t       off   = 0;
-    off += 2 * kHistSlotBytes;
-    if (off_status) *off_status = off;
-    off += (size_t)kMaxSortPasses * tiles * kMaxRadix * sizeof(uint32_t);
-    off = (off + 255) & ~(size_t)255;
-    if (off_keys) *off_keys = off;
-    off += n * key_bytes;
-    off = (off + 255) & ~(size_t)255;
-    if (off_vals) *off_vals = off;
-    off += n * sizeof(uint32_t);
-    off = (off + 255) & ~(size_t)255;
-    return off;
-}
-
-size_t sort_temp_bytes(size_t n) { return sort_ws_layout(n, sizeof(uint64_t), nullptr, nullptr, nullptr); }
-
-// Everything launch_sort_t needs to know about one sort; filled by sort_prepare_t.
 template <typename KeyT>
-struct SortPlan {
-    SortPassInfo info;
-    int          variant;
-    size_t       bound, tiles;
-    uint32_t *   hist, *status, *tmp_vals, *ticket;
-    KeyT*        tmp_keys;
-};
-
-// Pass geometry + workspace + zeroed histograms / look-back status / tickets.  After this call another
-// kernel may accumulate the digit histograms itself (plan.hist, layout [pass][1 << radix_bits]) and
-// launch_sort_t can be told to skip its own histogram kernel.
-// digit cut, kernel geometry and tile count of a sort over `bound` pairs; no workspace yet
-template <typename KeyT>
-static int sort_plan_geometry(lcgs_b200_ctx* ctx, size_t bound, int begin_bit, int end_bit, SortPlan<KeyT>* plan)
+int sort_plan_geometry(lcgs_b200_ctx* ctx, size_t bound, int begin_bit, int end_bit, SortPlan<KeyT>* plan)
 {
     constexpr int kKeyBits = (int)sizeof(KeyT) * 8;
     LCGS_REQUIRE(ctx, begin_bit >= 0 && end_bit <= kKeyBits && begin_bit <= end_bit, "sort: bad bit range");
@@ -537,60 +488,24 @@ static int sort_plan_geometry(lcgs_b200_ctx* ctx, size_t bound, int begin_bit, i
         info.shift[p] = lo < kKeyBits ? lo : 0;
         info.mask[p]  = w > 0 ? ((1u << w) - 1u) : 0u;
     }
-    plan->variant = vi;
-    plan->bound   = bound;
-    plan->tiles   = (bound + var.tile - 1) / var.tile;
-    plan->hist    = nullptr;
-    plan->ticket  = ctx->d_scalars + LCGS_SCALAR_SORT_TICKET;
+    plan->variant    = vi;
+    plan->bound      = bound;
+    plan->tiles      = (bound + var.tile - 1) / var.tile;
+    plan->hist_ready = false;
     return LCGS_B200_OK;
 }
+template int sort_plan_geometry<uint32_t>(lcgs_b200_ctx*, size_t, int, int, SortPlan<uint32_t>*);
+template int sort_plan_geometry<unsigned long long>(lcgs_b200_ctx*, size_t, int, int, SortPlan<unsigned long long>*);
 
-template <typename KeyT>
-static size_t sort_status_bytes(const SortPlan<KeyT>& plan)
-{
-    if (plan.info.num_passes == 0 || plan.bound == 0) return 0;
-    const size_t b = (size_t)plan.info.num_passes * plan.tiles * ((size_t)1 << plan.info.radix_bits) * sizeof(uint32_t);
-    return (b + 255) & ~(size_t)255;
-}
-
-// Pass geometry + workspace + zeroed histograms / look-back status / tickets.  After this call another
-// kernel may accumulate the digit histograms itself (plan.hist, layout [pass][1 << radix_bits]) and
-// launch_sort_t can be told to skip its own histogram kernel.
-template <typename KeyT>
-static int sort_prepare_t(lcgs_b200_ctx* ctx, size_t bound, int begin_bit, int end_bit, uint32_t* ticket, SortPlan<KeyT>* plan,
-                          cudaStream_t s, int hist_slot = 1)
-{
-    int rc = sort_plan_geometry<KeyT>(ctx, bound, begin_bit, end_bit, plan);
-    if (rc) return rc;
-    plan->ticket = ticket;
-    const SortPassInfo& info = plan->info;
-    if (info.num_passes == 0 || bound == 0) return LCGS_B200_OK;
-
-    size_t       off_status, off_keys, off_vals;
-    const size_t bytes = sort_ws_layout(bound, sizeof(KeyT), &off_status, &off_keys, &off_vals);
-    rc                 = ws_reserve(ctx, ctx->sort_ws, bytes);
-    if (rc) return rc;
-    char* ws       = (char*)ctx->sort_ws.ptr;
-    plan->hist     = (uint32_t*)(ws + (size_t)hist_slot * kHistSlotBytes);
-    plan->status   = (uint32_t*)(ws + off_status);
-    plan->tmp_keys = (KeyT*)(ws + off_keys);
-    plan->tmp_vals = (uint32_t*)(ws + off_vals);
-    // zero this sort's histograms + the look-back status (contiguous) and the tickets
-    char* const zero_from = (char*)plan->hist;
-    LCGS_CUDA_CHECK(ctx, cudaMemsetAsync(zero_from, 0, (size_t)(ws + off_status - zero_from) +
-                                                           (size_t)info.num_passes * plan->tiles * ((size_t)1 << info.radix_bits) * sizeof(uint32_t), s));
-    LCGS_CUDA_CHECK(ctx, cudaMemsetAsync(ticket, 0, kMaxSortPasses * sizeof(uint32_t), s));
-    return LCGS_B200_OK;
-}
-
-// skip_trivial_last: the last pass returns at once when all its keys have digit 0 (it would be the
-// identity permutation); `alt`, if given, receives that pass's input buffers and its histogram, so that
-// the consumer can make the same test (hist[0] == n) and read the right pair of buffers.
+// in_place: (kin, vals_in) and (kout, vals_out) are both scratch and the passes alternate between them instead of going
+// through the workspace (the result is in the output buffers for an odd number of passes, else in the input buffers);
+// the last pass returns at once when all its keys have digit 0 (it would be the identity permutation), and *in_place
+// receives that pass's input buffers and its histogram, so that the consumer can make the same test (hist[0] == n) and
+// read the right pair of buffers.  The other sorts record the profiling events of lcgs_b200_sort_breakdown.
 template <typename KeyT>
 static int launch_sort_t(lcgs_b200_ctx* ctx, const SortPlan<KeyT>& plan, const KeyT* kin, KeyT* kout, const uint32_t* vals_in,
-                         uint32_t* vals_out, size_t n_host, const uint32_t* d_n, size_t capacity, uint32_t* ticket,
-                         bool hist_ready, bool record_events, cudaStream_t s, bool skip_trivial_last = false,
-                         SortedPairsU32* alt = nullptr, bool pingpong_with_input = false)
+                         uint32_t* vals_out, size_t n_host, const uint32_t* d_n, size_t capacity, cudaStream_t s,
+                         SortedPairsU32* in_place = nullptr)
 {
     const size_t bound = plan.bound;
     if (bound == 0) return LCGS_B200_OK;
@@ -607,9 +522,9 @@ static int launch_sort_t(lcgs_b200_ctx* ctx, const SortPlan<KeyT>& plan, const K
     const int    radix = 1 << info.radix_bits;
     const size_t tiles = plan.tiles;
 
-    const bool prof = record_events && ctx->profiling && ctx->ev_sort[0];
+    const bool prof = !in_place && ctx->profiling && ctx->ev_sort[0];
     if (prof) cudaEventRecord(ctx->ev_sort[0], s);
-    if (!hist_ready) {
+    if (!plan.hist_ready) {
         radix_histogram_kernel<KeyT><<<grid_stride_blocks, 256, 0, s>>>(kin, n_host, d_n, capacity, plan.hist, info);
         LCGS_CUDA_CHECK(ctx, cudaGetLastError());
     }
@@ -627,24 +542,23 @@ static int launch_sort_t(lcgs_b200_ctx* ctx, const SortPlan<KeyT>& plan, const K
     const KeyT*     src_k = kin;
     const uint32_t* src_v = vals_in;
     for (int p = 0; p < info.num_passes; p++) {
-        // default: ping-pong with the workspace so that the last pass lands in (kout, vals_out) and the
-        // input survives; pingpong_with_input: alternate between the output and the (scratch) input
-        // buffers, result in the output buffers for an odd number of passes, else in the input buffers
-        const bool to_out = pingpong_with_input ? (p % 2) == 0 : ((info.num_passes - 1 - p) % 2) == 0;
-        KeyT*      dst_k  = to_out ? kout : (pingpong_with_input ? const_cast<KeyT*>(kin) : plan.tmp_keys);
-        uint32_t*  dst_v  = to_out ? vals_out : (pingpong_with_input ? const_cast<uint32_t*>(vals_in) : plan.tmp_vals);
+        // ping-pong with the workspace so that the last pass lands in (kout, vals_out) and the input survives,
+        // or in place (above)
+        const bool to_out = in_place ? (p % 2) == 0 : ((info.num_passes - 1 - p) % 2) == 0;
+        KeyT*      dst_k  = to_out ? kout : (in_place ? const_cast<KeyT*>(kin) : plan.tmp_keys);
+        uint32_t*  dst_v  = to_out ? vals_out : (in_place ? const_cast<uint32_t*>(vals_in) : plan.tmp_vals);
         const bool last = p == info.num_passes - 1;
-        if (last && skip_trivial_last && alt) {
-            alt->alt_keys  = reinterpret_cast<const uint32_t*>(src_k);
-            alt->alt_vals  = src_v;
-            alt->last_hist = plan.hist + (size_t)p * radix;
+        if (last && in_place) {
+            in_place->alt_keys  = reinterpret_cast<const uint32_t*>(src_k);
+            in_place->alt_vals  = src_v;
+            in_place->last_hist = plan.hist + (size_t)p * radix;
         }
         const int hi = (sizeof(KeyT) == 8 && info.shift[p] >= 32) ? 1 : 0;
         var.kernel[hi]<<<sweep_blocks, var.threads, var.smem, s>>>(src_k, dst_k, src_v, dst_v, n_host, d_n, capacity,
                                                               plan.hist + (size_t)p * radix,
-                                                              plan.status + (size_t)p * tiles * radix, ticket + p,
+                                                              plan.status + (size_t)p * tiles * radix, plan.ticket + p,
                                                               info.shift[p], info.mask[p],
-                                                              (last && skip_trivial_last) ? kSweepSkipIfTrivial : 0);
+                                                              (last && in_place) ? kSweepSkipIfTrivial : 0);
         LCGS_CUDA_CHECK(ctx, cudaGetLastError());
         src_k = dst_k;
         src_v = dst_v;
@@ -664,91 +578,45 @@ int launch_sort(lcgs_b200_ctx* ctx, const uint64_t* keys_in, uint64_t* keys_out,
     const size_t bound = d_n ? capacity : n_host;
     if (bound == 0) return LCGS_B200_OK;
     if (!d_n) capacity = n_host;
-    uint32_t*                    ticket = ctx->d_scalars + LCGS_SCALAR_SORT_TICKET;
     SortPlan<unsigned long long> plan;
-    int rc = sort_prepare_t<unsigned long long>(ctx, bound, begin_bit, end_bit, ticket, &plan, s);
+    int rc = sort_plan_geometry<unsigned long long>(ctx, bound, begin_bit, end_bit, &plan);
     if (rc) return rc;
+    plan.ticket = ctx->d_scalars + LCGS_SCALAR_SORT_TICKET;
+    const SortPassInfo& info = plan.info;
+    if (info.num_passes > 0) {
+        const SortWsLayout l = sort_ws_layout(bound, sort_status_bound(bound));
+        if ((rc = ws_reserve(ctx, ctx->sort_ws, l.bytes))) return rc;
+        char* ws      = (char*)ctx->sort_ws.ptr;
+        plan.hist     = (uint32_t*)(ws + kHistSlotBytes);
+        plan.status   = (uint32_t*)(ws + l.status);
+        plan.tmp_keys = (unsigned long long*)(ws + l.keys);
+        plan.tmp_vals = (uint32_t*)(ws + l.vals);
+        // zero this sort's histograms + the look-back status (contiguous) and the tickets
+        LCGS_CUDA_CHECK(ctx, cudaMemsetAsync(plan.hist, 0, (size_t)((char*)plan.status - (char*)plan.hist) + sort_status_bytes(plan), s));
+        LCGS_CUDA_CHECK(ctx, cudaMemsetAsync(plan.ticket, 0, kMaxSortPasses * sizeof(uint32_t), s));
+    }
     return launch_sort_t<unsigned long long>(ctx, plan, reinterpret_cast<const unsigned long long*>(keys_in),
                                              reinterpret_cast<unsigned long long*>(keys_out), vals_in, vals_out, n_host, d_n,
-                                             capacity, ticket, false, true, s);
+                                             capacity, s);
 }
 
-// ---- fused path: the kernel that PRODUCES the keys also accumulates the digit histograms ------------
-// sort_prepare_frame plans both sorts of a frame and returns where the histograms live and how digits are cut;
-// sort_run_* then launches only the onesweep passes.
-// Sorts (keys_a, vals_a) using (keys_b, vals_b) as the ping-pong partner; both pairs are scratch.  The
-// result is in res->keys/vals, or in res->alt_* when the last pass skipped itself (SortedPairsU32).
-int sort_run_u32(lcgs_b200_ctx* ctx, uint32_t* keys_a, uint32_t* keys_b, uint32_t* vals_a, uint32_t* vals_b,
-                 const uint32_t* d_n, size_t capacity, bool hist_ready, SortedPairsU32* res, cudaStream_t s)
+// ---- fused frame: the kernel that PRODUCES the keys also accumulates the digit histograms (FramePlan) -------------
+int sort_run_u32(lcgs_b200_ctx* ctx, const SortPlan<uint32_t>& plan, uint32_t* keys_a, uint32_t* keys_b, uint32_t* vals_a,
+                 uint32_t* vals_b, const uint32_t* d_n, size_t capacity, SortedPairsU32* res, cudaStream_t s)
 {
-    const auto& plan   = *static_cast<const SortPlan<uint32_t>*>(ctx->plan32);
-    const bool  in_b   = (plan.info.num_passes % 2) == 1;  // pass p writes b for even p, a for odd p
+    const bool in_b = (plan.info.num_passes % 2) == 1;  // pass p writes b for even p, a for odd p
     res->keys = res->alt_keys = in_b ? keys_b : keys_a;
     res->vals = res->alt_vals = in_b ? vals_b : vals_a;
     res->last_hist = nullptr;
     if (plan.info.num_passes == 0) return LCGS_B200_OK;  // nothing to sort by: the input is the result
-    return launch_sort_t<uint32_t>(ctx, plan, keys_a, keys_b, vals_a, vals_b, 0, d_n, capacity, plan.ticket, hist_ready, false, s, true,
-                                   res, true);
+    return launch_sort_t<uint32_t>(ctx, plan, keys_a, keys_b, vals_a, vals_b, 0, d_n, capacity, s, res);
 }
 
-int sort_run_u64(lcgs_b200_ctx* ctx, const uint64_t* keys_in, uint64_t* keys_out, const uint32_t* vals_in, uint32_t* vals_out,
-                 const uint32_t* d_n, size_t capacity, bool hist_ready, cudaStream_t s)
+int sort_run_u64(lcgs_b200_ctx* ctx, const SortPlan<unsigned long long>& plan, const uint64_t* keys_in, uint64_t* keys_out,
+                 const uint32_t* vals_in, uint32_t* vals_out, const uint32_t* d_n, size_t capacity, cudaStream_t s)
 {
-    const auto& plan = *static_cast<const SortPlan<unsigned long long>*>(ctx->plan64);
     return launch_sort_t<unsigned long long>(ctx, plan, reinterpret_cast<const unsigned long long*>(keys_in),
-                                             reinterpret_cast<unsigned long long*>(keys_out), vals_in, vals_out, 0, d_n, capacity,
-                                             plan.ticket, hist_ready, true, s);
-}
-
-static void export_digits(const SortPassInfo& info, uint32_t* hist, SortDigits* digits)
-{
-    digits->hist = hist; digits->num_passes = info.num_passes; digits->radix_bits = info.radix_bits;
-    for (int p = 0; p < kMaxSortPasses; p++) { digits->shift[p] = info.shift[p]; digits->mask[p] = info.mask[p]; }
-}
-
-// layout: [hist slot 0][hist slot 1][status of the depth sort][status of the tile sort][tmp keys][tmp vals]; the part up to
-// the tmp buffers is one contiguous region to clear.  Tickets: depth sort SORT_TICKET + 0..3, tile sort SORT_TICKET + 4..7.
-int sort_prepare_frame(lcgs_b200_ctx* ctx, size_t P, size_t L, int end_bit, SortDigits* dg32, SortDigits* dg64, ClearList* cl)
-{
-    if (!ctx->plan32) ctx->plan32 = new SortPlan<uint32_t>();
-    if (!ctx->plan64) ctx->plan64 = new SortPlan<unsigned long long>();
-    auto& p32 = *static_cast<SortPlan<uint32_t>*>(ctx->plan32);
-    auto& p64 = *static_cast<SortPlan<unsigned long long>*>(ctx->plan64);
-    int   rc;
-    if ((rc = sort_plan_geometry<uint32_t>(ctx, P, 0, 32, &p32))) return rc;
-    if ((rc = sort_plan_geometry<unsigned long long>(ctx, L, 32, end_bit, &p64))) return rc;
-    LCGS_REQUIRE(ctx, p32.info.num_passes <= 4 && p64.info.num_passes <= 4, "sort: a fused frame's sorts have at most four passes each");
-    const size_t s32 = sort_status_bytes(p32), s64 = sort_status_bytes(p64);
-    const size_t off_status = 2 * kHistSlotBytes;
-    const size_t off_keys   = (off_status + s32 + s64 + 255) & ~(size_t)255;
-    const size_t off_vals   = (off_keys + L * sizeof(unsigned long long) + 255) & ~(size_t)255;
-    const size_t total      = (off_vals + L * sizeof(uint32_t) + 255) & ~(size_t)255;
-    if ((rc = ws_reserve(ctx, ctx->sort_ws, total))) return rc;
-    char* ws = (char*)ctx->sort_ws.ptr;
-    if (s32) {
-        p32.hist = (uint32_t*)ws;
-        p32.status = (uint32_t*)(ws + off_status);
-        p32.tmp_keys = nullptr; p32.tmp_vals = nullptr;  // the depth sort ping-pongs between its two caller-provided buffers
-    }
-    p32.ticket = ctx->d_scalars + LCGS_SCALAR_SORT_TICKET;
-    if (s64) {
-        p64.hist = (uint32_t*)(ws + kHistSlotBytes);
-        p64.status = (uint32_t*)(ws + off_status + s32);
-        p64.tmp_keys = (unsigned long long*)(ws + off_keys);
-        p64.tmp_vals = (uint32_t*)(ws + off_vals);
-    }
-    p64.ticket = ctx->d_scalars + LCGS_SCALAR_SORT_TICKET + 4;
-    export_digits(p32.info, p32.hist, dg32);
-    export_digits(p64.info, p64.hist, dg64);
-    cl->add(ws, off_status + s32 + s64);
-    return LCGS_B200_OK;
-}
-
-void sort_free_plans(lcgs_b200_ctx* ctx)
-{
-    delete static_cast<SortPlan<uint32_t>*>(ctx->plan32);
-    delete static_cast<SortPlan<unsigned long long>*>(ctx->plan64);
-    ctx->plan32 = ctx->plan64 = nullptr;
+                                             reinterpret_cast<unsigned long long*>(keys_out), vals_in, vals_out, 0, d_n, capacity, s);
 }
 
 }  // namespace lcgs_b200
