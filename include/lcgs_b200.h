@@ -271,6 +271,12 @@ LCGS_B200_API int lcgs_b200_render(lcgs_b200_ctx* ctx, const lcgs_b200_scene* sc
  *     the [0,1] colour clamp (per channel) pass gradient only where inactive; the view direction of SH degree >= 1
  *     reaches pos.  radius, the tile rect, depth order and tiles_touched are discrete: a Gaussian with
  *     tiles_touched == 0 gets exactly zero in every output.  An empty frame gives all-zero gradients.
+ *   aux planes (optional): with dl_dalpha = dL/dA and/or dl_ddepth = dL/dD for the frame's target_alpha
+ *     A = 1 - T_{n+1} and target_depth D = sum w_i z_i (z_i = depth[i], the view depth), each plane is one more channel
+ *     of the blend with colour 1 (alpha) or z_i (depth) and a background of 0: c_i . G above becomes
+ *     c_i . G + z_i dL/dD + dL/dA, C . G becomes C . G + D dL/dD + A dL/dA, and dL/dz_i = sum over pixels w_i dL/dD,
+ *     which reaches pos through the view transform.  A and D are read back from the frame, like C.  n_contrib is
+ *     discrete and has no gradient.
  * Gradients are summed with float atomics: the last bits vary from run to run. */
 typedef struct lcgs_b200_grad {
     const float* dl_dimg; /* [3][H][W], layout of target_img */
@@ -279,14 +285,23 @@ typedef struct lcgs_b200_grad {
     /* optional: gradients of the blend's per-Gaussian inputs -- pixel-space mean [P][2] (also the
        densification statistic trainers accumulate), conic [P][3], post-clamp colour [P][3] */
     float *grad_means_2d, *grad_conic, *grad_color;
+    /* optional gradients of the aux planes, [H][W] in the layout of target_alpha / target_depth, 4-byte aligned
+       (NULL = the plane is not in the loss).  dl_dalpha needs frame->target_alpha, dl_ddepth needs frame->target_depth
+       and frame->depth, all as rendered with the frame. */
+    const float* dl_dalpha;
+    const float* dl_ddepth;
+    /* optional [P]: dL/d(view depth) of each Gaussian, the blend's part (like grad_means_2d); all zeros without
+       dl_ddepth */
+    float* grad_depth;
 } lcgs_b200_grad;
 
 /* Backward of one whole frame.  `scene`, `vp` and `frame` are those the frame was rendered with; the call reads only
  * the frame's point_list, ranges, means_2d, conic, color, tiles_touched and target_img (all required), plus the scene
  * and the view -- not the context's workspace from the forward, so any number of frames, on this context or another,
  * may be rendered between a frame and its backward as long as that frame's buffers are intact.  Enqueue only (no
- * host synchronisation except workspace growth).  LCGS_B200_ERR_INVALID for a NULL required pointer or a misaligned
- * pointer, LCGS_B200_ERR_UNSUPPORTED for a tile-row band (whole frames only). */
+ * host synchronisation except workspace growth).  With dl_dalpha or dl_ddepth it also reads target_alpha /
+ * target_depth and depth.  LCGS_B200_ERR_INVALID for a NULL required pointer (a plane gradient without its plane
+ * included) or a misaligned pointer, LCGS_B200_ERR_UNSUPPORTED for a tile-row band (whole frames only). */
 LCGS_B200_API int lcgs_b200_render_backward(lcgs_b200_ctx* ctx, const lcgs_b200_scene* scene,
                                             const lcgs_b200_view_params* vp, const lcgs_b200_frame* frame,
                                             const lcgs_b200_grad* grad, lcgs_b200_stream stream);

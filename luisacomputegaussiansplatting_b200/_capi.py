@@ -57,11 +57,13 @@ class Frame(C.Structure):
 
 
 class Grad(C.Structure):
-    """lcgs_b200_grad: dL/dimg in, per-Gaussian gradients out (each output optional)."""
+    """lcgs_b200_grad: dL/dimg (and optionally dL/d of the alpha and depth planes) in, per-Gaussian gradients out
+    (each output optional)."""
 
     _fields_ = [("dl_dimg", C.c_void_p), ("grad_pos", C.c_void_p), ("grad_scale", C.c_void_p), ("grad_rotq", C.c_void_p),
                 ("grad_sh", C.c_void_p), ("grad_opacity", C.c_void_p), ("grad_means_2d", C.c_void_p),
-                ("grad_conic", C.c_void_p), ("grad_color", C.c_void_p)]
+                ("grad_conic", C.c_void_p), ("grad_color", C.c_void_p), ("dl_dalpha", C.c_void_p),
+                ("dl_ddepth", C.c_void_p), ("grad_depth", C.c_void_p)]
 
 
 PEER_HANDLE_BYTES = 64

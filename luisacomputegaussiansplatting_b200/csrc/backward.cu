@@ -13,9 +13,12 @@
 //    conic, dL/dpower, colour), the warp reduces them with shuffles and three lanes add the sums to the Gaussian's
 //    packed [12] float entry with one vector reduction each (RED.128): one global atomic set per (patch, Gaussian)
 //    with a contribution.
+//  * blend_backward_aux_kernel : the same walk (blend_backward_body<true>) when dL/d(alpha plane) or dL/d(depth plane)
+//    is given: the planes are two more channels of the pixel's dot products, the candidate's view depth is staged with
+//    its record by a fourth cp.async, and the warp reduces 10 values, the 10th (dL/dz) going to slot kG2Depth.
 //  * preprocess_backward_kernel : one thread per Gaussian; Gaussians with tiles_touched == 0 get zeros.  Recomputes
 //    the forward's intermediates from the scene and chains the packed 2D gradient to pos / scale / rotq / sh /
-//    opacity.
+//    opacity (dL/dz through the view z).
 // Float atomics make the summation order, and so the last bits of the gradients, vary from run to run; the forward
 // is untouched and stays bit-reproducible.
 #include "blend_walk.cuh"
@@ -40,45 +43,78 @@ struct GlobalShOut {
 
 }  // namespace
 
-__global__ void __launch_bounds__(kWalkThreads)
-    blend_backward_kernel(int W, int H, uint32_t gx, const uint2* __restrict__ ranges, const uint32_t* __restrict__ order,
-                          const uint32_t* __restrict__ point_list, const float4* __restrict__ records,
-                          const float* __restrict__ img, const float* __restrict__ dl_dimg, float4* __restrict__ grad2d)
+// AUX (blend_backward_aux_kernel): the gradients of the frame's alpha and depth planes as well (lcgs_grad.cuh,
+// PixelGradAux).  Each pixel also reads A, D and their gradients (a NULL gradient counts as 0); the candidate's view
+// depth z = depth[id] is staged with its record by a fourth, 4-byte cp.async into s_z, as in blend2_aux_kernel
+// (depth == NULL: no depth gradient, z = 0), and the warp reduces 10 values per hit, the 10th being dL/dz.
+template <bool AUX>
+__device__ __forceinline__ void blend_backward_body(const int tid, int W, int H, uint32_t gx, const uint2* __restrict__ ranges,
+                                                    const uint32_t* __restrict__ order, const uint32_t* __restrict__ point_list,
+                                                    const float4* __restrict__ records, const float* __restrict__ img,
+                                                    const float* __restrict__ dl_dimg, const float* __restrict__ alpha,
+                                                    const float* __restrict__ dplane, const float* __restrict__ dl_dalpha,
+                                                    const float* __restrict__ dl_ddepth, const float* __restrict__ depth,
+                                                    float4* __restrict__ grad2d)
 {
     __shared__ float4   s_rec[2][3][kWalkThreads];  // [buffer][plane][slot], planes as in the record (common.cuh)
     __shared__ uint32_t s_cnt[2][kWalkWarps];
-    __shared__ uint32_t s_id[2 * kWalkThreads];  // [buffer * 128 + slot]: Gaussian index of the staged record
+    __shared__ uint32_t s_id[2 * kWalkThreads];            // [buffer * 128 + slot]: Gaussian index of the staged record
+    __shared__ float    s_z[AUX ? 2 * kWalkThreads : 1];  // [buffer * 128 + slot]: its view depth (AUX only)
+    const uint32_t      zbase = AUX ? (uint32_t)__cvta_generic_to_shared(&s_z[0]) : 0u;
+    constexpr int       NV    = AUX ? kGrad2DAuxValues : kGrad2DValues;
 
-    const int        tid  = threadIdx.x;
     const unsigned   FULL = 0xFFFFFFFFu;
     const TilePixels p    = tile_pixels(tid & 31, tid >> 5, order, gx, 0u);
     const bool       in_a = p.px < W && p.pya < H, in_b = p.px < W && p.pyb < H;
     const float      pxf = (float)p.px, pyaf = (float)p.pya, pybf = (float)p.pyb;  // no half-pixel offset (Q2)
 
     const size_t plane = (size_t)W * (size_t)H;
-    PixelGrad    pa, pb;
+    PixelGradAux pa, pb;  // without AUX only .p is used
     {
         float C[3] = { 0.f, 0.f, 0.f }, G[3] = { 0.f, 0.f, 0.f };
         const size_t ia = (size_t)p.px + (size_t)W * (size_t)p.pya, ib = (size_t)p.px + (size_t)W * (size_t)p.pyb;
+        // A, D, dL/dA, dL/dD of a pixel (AUX): a plane whose gradient is NULL does not enter
+        auto planes = [&](bool in, size_t i, float* v) {
+            v[0] = in && dl_dalpha ? __ldg(alpha + i) : 0.0f;
+            v[1] = in && dl_ddepth ? __ldg(dplane + i) : 0.0f;
+            v[2] = in && dl_dalpha ? __ldg(dl_dalpha + i) : 0.0f;
+            v[3] = in && dl_ddepth ? __ldg(dl_ddepth + i) : 0.0f;
+        };
         if (in_a)
             for (int k = 0; k < 3; k++) { C[k] = __ldg(img + ia + k * plane); G[k] = __ldg(dl_dimg + ia + k * plane); }
-        pa = pixel_grad_init(in_a, C, G);
+        if constexpr (AUX) {
+            float v[4];
+            planes(in_a, ia, v);
+            pa = pixel_grad_aux_init(in_a, C, G, v[0], v[1], v[2], v[3]);
+        } else {
+            pa.p = pixel_grad_init(in_a, C, G);
+        }
         if (in_b)
             for (int k = 0; k < 3; k++) { C[k] = __ldg(img + ib + k * plane); G[k] = __ldg(dl_dimg + ib + k * plane); }
         else
             for (int k = 0; k < 3; k++) { C[k] = 0.f; G[k] = 0.f; }
-        pb = pixel_grad_init(in_b, C, G);
+        if constexpr (AUX) {
+            float v[4];
+            planes(in_b, ib, v);
+            pb = pixel_grad_aux_init(in_b, C, G, v[0], v[1], v[2], v[3]);
+        } else {
+            pb.p = pixel_grad_init(in_b, C, G);
+        }
     }
 
     // The walk's cull box shrinks to the pixels still accumulating, as in the forward: the cull is conservative and a
     // finished pixel adds nothing in blend_entry_grad, so every pixel still meets the entries the forward blended.
-    auto stage_id  = [&](uint32_t entry, uint32_t id) { s_id[entry] = id; };
+    auto stage_id = [&](uint32_t entry, uint32_t id) {
+        s_id[entry] = id;
+        if constexpr (AUX)
+            if (depth) cp_async_4(zbase + entry * 4u, depth + id);
+    };
     auto no_consts = [] { return 0; };  // the scalar evaluation keeps no per-walk constants
     auto accumulate = [&](int, const float4& ea, const float4& eb, const float4& ec, uint32_t entry) {
         const float rgb[3] = { ec.x, ec.y, ec.z };
-        float       g[kGrad2DValues];
+        float       g[NV];
 #pragma unroll
-        for (int k = 0; k < kGrad2DValues; k++) g[k] = 0.0f;
+        for (int k = 0; k < NV; k++) g[k] = 0.0f;
         // the forward's per-pixel operations (blend2_body's evaluate, scalar form)
         const float dx  = ea.x - pxf;
         const float dya = ea.y - pyaf, dyb = ea.y - pybf;
@@ -88,23 +124,54 @@ __global__ void __launch_bounds__(kWalkThreads)
         const bool  okb = !(pwb > 0.0f) && !(pwb < eb.y);
         const float ea_ = ex2_ftz(__fmaf_rn(pwa, 1.4426950408889634f, eb.z));
         const float eb_ = ex2_ftz(__fmaf_rn(pwb, 1.4426950408889634f, eb.z));
-        bool contributed = blend_entry_grad(pa, oka, ea_, dx, dya, ea.z, ea.w, eb.x, rgb, g);
-        contributed |= blend_entry_grad(pb, okb, eb_, dx, dyb, ea.z, ea.w, eb.x, rgb, g);
+        bool contributed;
+        if constexpr (AUX) {
+            const float z = depth ? lds32(zbase + entry * 4u) : 0.0f;
+            contributed = blend_entry_grad_aux(pa, oka, ea_, dx, dya, ea.z, ea.w, eb.x, rgb, z, g);
+            contributed |= blend_entry_grad_aux(pb, okb, eb_, dx, dyb, ea.z, ea.w, eb.x, rgb, z, g);
+        } else {
+            contributed = blend_entry_grad(pa.p, oka, ea_, dx, dya, ea.z, ea.w, eb.x, rgb, g);
+            contributed |= blend_entry_grad(pb.p, okb, eb_, dx, dyb, ea.z, ea.w, eb.x, rgb, g);
+        }
         if (__any_sync(FULL, contributed)) {
 #pragma unroll
-            for (int k = 0; k < kGrad2DValues; k++)
+            for (int k = 0; k < NV; k++)
 #pragma unroll
                 for (int o = 16; o > 0; o >>= 1) g[k] += __shfl_xor_sync(FULL, g[k], o);
             if (p.lane < 3) {
                 const uint32_t id = s_id[entry];
                 const float4   v  = p.lane == 0 ? make_float4(g[0], g[1], g[2], g[3])
                                     : p.lane == 1 ? make_float4(g[4], g[5], g[6], g[7])
-                                                  : make_float4(g[8], 0.0f, 0.0f, 0.0f);
+                                                  : make_float4(g[8], AUX ? g[NV - 1] : 0.0f, 0.0f, 0.0f);
                 atomicAdd(grad2d + (size_t)id * 3 + p.lane, v);  // RED.E.ADD.F32x4
             }
         }
     };
-    walk_tile(tid, p, ranges, point_list, records, s_rec, s_cnt, pa.T, pb.T, stage_id, no_consts, accumulate);
+    walk_tile(tid, p, ranges, point_list, records, s_rec, s_cnt, pa.p.T, pb.p.T, stage_id, no_consts, accumulate);
+}
+
+__global__ void __launch_bounds__(kWalkThreads)
+    blend_backward_kernel(int W, int H, uint32_t gx, const uint2* __restrict__ ranges, const uint32_t* __restrict__ order,
+                          const uint32_t* __restrict__ point_list, const float4* __restrict__ records,
+                          const float* __restrict__ img, const float* __restrict__ dl_dimg, float4* __restrict__ grad2d)
+{
+    blend_backward_body<false>((int)threadIdx.x, W, H, gx, ranges, order, point_list, records, img, dl_dimg, nullptr,
+                               nullptr, nullptr, nullptr, nullptr, grad2d);
+}
+
+// blend_backward_kernel plus the gradients of the alpha and depth planes (see blend_backward_body).  alpha / dplane:
+// the frame's target_alpha / target_depth, read where dl_dalpha / dl_ddepth are non-NULL; depth: the frame's
+// per-Gaussian view depth [P], non-NULL iff dl_ddepth is.
+__global__ void __launch_bounds__(kWalkThreads)
+    blend_backward_aux_kernel(int W, int H, uint32_t gx, const uint2* __restrict__ ranges, const uint32_t* __restrict__ order,
+                              const uint32_t* __restrict__ point_list, const float4* __restrict__ records,
+                              const float* __restrict__ img, const float* __restrict__ dl_dimg,
+                              const float* __restrict__ alpha, const float* __restrict__ dplane,
+                              const float* __restrict__ dl_dalpha, const float* __restrict__ dl_ddepth,
+                              const float* __restrict__ depth, float4* __restrict__ grad2d)
+{
+    blend_backward_body<true>((int)threadIdx.x, W, H, gx, ranges, order, point_list, records, img, dl_dimg, alpha, dplane,
+                              dl_dalpha, dl_ddepth, depth, grad2d);
 }
 
 struct PreprocessGradArgs {
@@ -119,10 +186,12 @@ struct PreprocessGradArgs {
     const uint32_t* tiles;
     const float4*   grad2d;
     float *         grad_pos, *grad_scale, *grad_rotq, *grad_sh, *grad_opacity;
-    float *         grad_means_2d, *grad_conic, *grad_color;
+    float *         grad_means_2d, *grad_conic, *grad_color, *grad_depth;
 };
 
-__global__ void __launch_bounds__(128) preprocess_backward_kernel(const __grid_constant__ PreprocessGradArgs a)
+// 6 CTAs per SM: 80 registers, no spills.  Unbounded, the depth plane's dL/dz add in project_backward makes ptxas take
+// 96 registers (5 CTAs per SM).
+__global__ void __launch_bounds__(128, 6) preprocess_backward_kernel(const __grid_constant__ PreprocessGradArgs a)
 {
     const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= a.P) return;
@@ -140,6 +209,7 @@ __global__ void __launch_bounds__(128) preprocess_backward_kernel(const __grid_c
             for (int k = 0; k < 4; k++) a.grad_rotq[4 * i + k] = 0.0f;
         if (a.grad_opacity) a.grad_opacity[i] = 0.0f;
         if (a.grad_means_2d) { a.grad_means_2d[2 * i] = 0.0f; a.grad_means_2d[2 * i + 1] = 0.0f; }
+        if (a.grad_depth) a.grad_depth[i] = 0.0f;
         if (gsh)
             for (int k = 0; k < feat * 3; k++) gsh[k] = 0.0f;
         return;
@@ -152,6 +222,7 @@ __global__ void __launch_bounds__(128) preprocess_backward_kernel(const __grid_c
         g2[8] = v2.x; g2[9] = v2.y; g2[10] = v2.z; g2[11] = v2.w;
     }
     if (a.grad_means_2d) { a.grad_means_2d[2 * i] = g2[kG2MeanX]; a.grad_means_2d[2 * i + 1] = g2[kG2MeanY]; }
+    if (a.grad_depth) a.grad_depth[i] = g2[kG2Depth];
     for (int k = 0; k < 3; k++) {
         if (a.grad_conic) a.grad_conic[3 * i + k] = g2[kG2Conic0 + k];
         if (a.grad_color) a.grad_color[3 * i + k] = g2[kG2Red + k];
@@ -201,9 +272,15 @@ int launch_render_backward(lcgs_b200_ctx* ctx, const lcgs_b200_scene* sc, const 
         return rc;
     // the tile schedule only: no count, so the context's device scalars (the last forward's) stay untouched
     if ((rc = launch_tile_order(ctx, fr->ranges, num_tiles, nullptr, 0, s))) return rc;
-    blend_backward_kernel<<<(unsigned)num_tiles, kWalkThreads, 0, s>>>(W, H, gx, reinterpret_cast<const uint2*>(fr->ranges),
-                                                                      (const uint32_t*)ctx->tile_order_ws.ptr, fr->point_list,
-                                                                      records, fr->target_img, gr->dl_dimg, grad2d);
+    if (gr->dl_dalpha || gr->dl_ddepth)
+        blend_backward_aux_kernel<<<(unsigned)num_tiles, kWalkThreads, 0, s>>>(
+            W, H, gx, reinterpret_cast<const uint2*>(fr->ranges), (const uint32_t*)ctx->tile_order_ws.ptr, fr->point_list,
+            records, fr->target_img, gr->dl_dimg, fr->target_alpha, fr->target_depth, gr->dl_dalpha, gr->dl_ddepth,
+            gr->dl_ddepth ? fr->depth : nullptr, grad2d);
+    else
+        blend_backward_kernel<<<(unsigned)num_tiles, kWalkThreads, 0, s>>>(W, H, gx, reinterpret_cast<const uint2*>(fr->ranges),
+                                                                          (const uint32_t*)ctx->tile_order_ws.ptr, fr->point_list,
+                                                                          records, fr->target_img, gr->dl_dimg, grad2d);
     LCGS_CUDA_CHECK(ctx, cudaGetLastError());
 
     PreprocessGradArgs a;
@@ -216,6 +293,7 @@ int launch_render_backward(lcgs_b200_ctx* ctx, const lcgs_b200_scene* sc, const 
     a.grad_pos = gr->grad_pos; a.grad_scale = gr->grad_scale; a.grad_rotq = gr->grad_rotq; a.grad_sh = gr->grad_sh;
     a.grad_opacity = gr->grad_opacity;
     a.grad_means_2d = gr->grad_means_2d; a.grad_conic = gr->grad_conic; a.grad_color = gr->grad_color;
+    a.grad_depth = gr->grad_depth;
     preprocess_backward_kernel<<<bwd_div_up(P, 128), 128, 0, s>>>(a);
     LCGS_CUDA_CHECK(ctx, cudaGetLastError());
     return LCGS_B200_OK;

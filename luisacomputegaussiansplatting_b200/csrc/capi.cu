@@ -588,6 +588,13 @@ int lcgs_b200_render_backward(lcgs_b200_ctx* ctx, const lcgs_b200_scene* sc, con
                           aligned(gr->grad_opacity, 4) && aligned(gr->grad_means_2d, 4) && aligned(gr->grad_conic, 4) &&
                           aligned(gr->grad_color, 4),
                  "render_backward: gradient buffers must be 4-byte aligned");
+    LCGS_REQUIRE(ctx, !gr->dl_dalpha || fr->target_alpha, "render_backward: dl_dalpha needs the frame's target_alpha");
+    LCGS_REQUIRE(ctx, !gr->dl_ddepth || (fr->target_depth && fr->depth),
+                 "render_backward: dl_ddepth needs the frame's target_depth and depth");
+    LCGS_REQUIRE(ctx, aligned(gr->dl_dalpha, 4) && aligned(gr->dl_ddepth, 4) && aligned(gr->grad_depth, 4) &&
+                          (!gr->dl_dalpha || aligned(fr->target_alpha, 4)) &&
+                          (!gr->dl_ddepth || (aligned(fr->target_depth, 4) && aligned(fr->depth, 4))),
+                 "render_backward: aux plane buffers must be 4-byte aligned");
     return launch_render_backward(ctx, sc, vp, fr, gr, as_stream(stream));
 }
 

@@ -21,6 +21,9 @@
 //   sh_color (the view direction of degree >= 1 reaches pos; the [0,1] colour clamp passes gradient per channel only
 //   where it is inactive) are differentiated exactly as written.  radius, the tile rect, depth order and
 //   tiles_touched are discrete.
+//   aux planes (the blend's optional alpha and depth planes, A = 1 - T_{n+1} and D = sum w_i z_i): two more channels
+//   with colours 1 and z_i and a background of 0 (see PixelGradAux); depth z = view z, so dL/dz joins dL/dvz in
+//   project_backward.
 #pragma once
 
 #include "lcgs_math.cuh"
@@ -29,9 +32,11 @@ namespace lcgs_b200 {
 
 // Packed per-Gaussian gradient of the blend's inputs: 12 floats = three float4, so the blend backward can accumulate
 // it with vector reductions.  kG2LogOp holds dL/dpower summed over the Gaussian's pairs (= dL/dlog(opacity)).
+// kG2Depth holds dL/d(view depth) from the depth plane; only the aux blend backward writes it (kGrad2DAuxValues), the
+// image-only one leaves it at 0.
 enum {
-    kG2MeanX = 0, kG2MeanY, kG2Conic0, kG2Conic1, kG2Conic2, kG2LogOp, kG2Red, kG2Green, kG2Blue,
-    kGrad2DValues = 9, kGrad2DFloats = 12
+    kG2MeanX = 0, kG2MeanY, kG2Conic0, kG2Conic1, kG2Conic2, kG2LogOp, kG2Red, kG2Green, kG2Blue, kG2Depth,
+    kGrad2DValues = 9, kGrad2DAuxValues = 10, kGrad2DFloats = 12
 };
 
 // Per-pixel state of the backward walk.  T < 0 marks a finished pixel (saturated or outside the image), as in the
@@ -51,13 +56,29 @@ LCGS_HD PixelGrad pixel_grad_init(bool inside, const float* C, const float* G)
     return p;
 }
 
-// One entry of the pixel's front-to-back walk.  ok = the entry passed the alpha test (power <= 0 and power >= the
-// Gaussian's threshold); alpha_raw = o e^power as the forward evaluated it, before the 0.99 cap.  (a, b, c) are the
-// record's pre-scaled conic (-0.5 conic.x, -conic.y, -0.5 conic.z), (dx, dy) = mean - pixel.  Adds the pair's
-// contribution to g[kGrad2DValues] and returns true iff the forward blended the entry.  T is updated with the
-// forward's own operations, so the walk stops exactly where the forward's did.
-LCGS_HD bool blend_entry_grad(PixelGrad& px, bool ok, float alpha_raw, float dx, float dy, float a, float b, float c,
-                              const float* rgb, float* g)
+// The aux planes are two more channels of the same blend with a background of 0: the alpha plane A = 1 - T has colour
+// 1 for every entry, the depth plane D = sum w_i z_i has colour z_i = depth[id].  With GA = dL/dA and GD = dL/dD the
+// per-entry colour dot product becomes c_i . G + z_i GD + GA and the final one C . G + D GD + A GA, so the aux walk is
+// the colour walk with that 5-channel dot product, plus dL/dz_i = w_i GD.
+struct PixelGradAux {
+    PixelGrad p;  // p.CG includes the planes' terms
+    float     GA, GD;
+};
+
+LCGS_HD PixelGradAux pixel_grad_aux_init(bool inside, const float* C, const float* G, float A, float D, float GA, float GD)
+{
+    PixelGradAux q;
+    q.p    = pixel_grad_init(inside, C, G);
+    q.p.CG = (q.p.CG + D * GD) + A * GA;
+    q.GA   = GA;
+    q.GD   = GD;
+    return q;
+}
+
+// One entry of the pixel's front-to-back walk (AUX: with the aux channels, z = the entry's view depth).
+template <bool AUX>
+LCGS_HD bool blend_entry_grad_t(PixelGrad& px, bool ok, float alpha_raw, float dx, float dy, float a, float b, float c,
+                                const float* rgb, float z, float GA, float GD, float* g)
 {
     if (!ok || !(px.T > 0.0f)) return false;
     const float T      = px.T;
@@ -68,8 +89,9 @@ LCGS_HD bool blend_entry_grad(PixelGrad& px, bool ok, float alpha_raw, float dx,
         return false;
     }
     const float w  = T * alpha;
-    const float cG = (rgb[0] * px.G[0] + rgb[1] * px.G[1]) + rgb[2] * px.G[2];
-    px.SG          = px.SG + w * cG;
+    float       cG = (rgb[0] * px.G[0] + rgb[1] * px.G[1]) + rgb[2] * px.G[2];
+    if constexpr (AUX) cG = (cG + z * GD) + GA;
+    px.SG              = px.SG + w * cG;
     const float dalpha = T * cG - (px.CG - px.SG) / (1.0f - alpha);
     const float gp     = alpha_raw < 0.99f ? dalpha * alpha : 0.0f;  // dL/dpower; zero under the cap
     g[kG2MeanX]  += gp * ((2.0f * a) * dx + b * dy);
@@ -81,8 +103,27 @@ LCGS_HD bool blend_entry_grad(PixelGrad& px, bool ok, float alpha_raw, float dx,
     g[kG2Red]    += w * px.G[0];
     g[kG2Green]  += w * px.G[1];
     g[kG2Blue]   += w * px.G[2];
+    if constexpr (AUX) g[kG2Depth] += w * GD;
     px.T = test_T;
     return true;
+}
+
+// One entry of the pixel's front-to-back walk.  ok = the entry passed the alpha test (power <= 0 and power >= the
+// Gaussian's threshold); alpha_raw = o e^power as the forward evaluated it, before the 0.99 cap.  (a, b, c) are the
+// record's pre-scaled conic (-0.5 conic.x, -conic.y, -0.5 conic.z), (dx, dy) = mean - pixel.  Adds the pair's
+// contribution to g[kGrad2DValues] and returns true iff the forward blended the entry.  T is updated with the
+// forward's own operations, so the walk stops exactly where the forward's did.
+LCGS_HD bool blend_entry_grad(PixelGrad& px, bool ok, float alpha_raw, float dx, float dy, float a, float b, float c,
+                              const float* rgb, float* g)
+{
+    return blend_entry_grad_t<false>(px, ok, alpha_raw, dx, dy, a, b, c, rgb, 0.0f, 0.0f, 0.0f, g);
+}
+
+// The same step on the aux channels: adds to g[kGrad2DAuxValues] (kG2Depth += w GD).
+LCGS_HD bool blend_entry_grad_aux(PixelGradAux& px, bool ok, float alpha_raw, float dx, float dy, float a, float b,
+                                  float c, const float* rgb, float z, float* g)
+{
+    return blend_entry_grad_t<true>(px.p, ok, alpha_raw, dx, dy, a, b, c, rgb, z, px.GA, px.GD, g);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -336,6 +377,8 @@ LCGS_HD void project_backward(const ViewParams& vp, float scale_modifier, float 
         dvy += dq / pv.z;
         dvz += -dq * pv.y / (pv.z * pv.z);
     }
+    // ---- the depth plane's part: depth = view z
+    dvz += g2[kG2Depth];
     // ---- pixel mean: px = ((ndc + 1) W - 1) / 2, ndc = (v * proj) / (z + 1e-6)
     const float dndx = g2[kG2MeanX] * (0.5f * (float)(uint32_t)vp.width);
     const float dndy = g2[kG2MeanY] * (0.5f * (float)(uint32_t)vp.height);

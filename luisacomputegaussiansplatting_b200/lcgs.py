@@ -628,6 +628,36 @@ class _RenderFunction(torch.autograd.Function):
         return (None, None, *out)
 
 
+class _RenderAuxFunction(torch.autograd.Function):
+    """_RenderFunction with the alpha and depth planes as two more outputs.  Gradients are not materialised: a plane
+    the loss does not use reaches the C call as NULL (the image-only blend backward then runs), and an unused image
+    as a zero gradient."""
+
+    @staticmethod
+    def forward(ctx, dr: "DifferentiableRenderer", vp: ViewParams, pos, scale, rotq, sh, opacity):
+        img, (scene, b) = dr._forward(vp, pos, scale, rotq, sh, opacity)
+        alpha, depth = b["alpha_plane"].view(dr.H, dr.W), b["depth_plane"].view(dr.H, dr.W)
+        ctx.set_materialize_grads(False)
+        ctx.save_for_backward(img, alpha, depth)
+        ctx.dr, ctx.vp = dr, vp
+        ctx.saved = (scene, {k: v for k, v in b.items() if k not in ("img", "alpha_plane", "depth_plane")})
+        ctx.shapes = [t.shape for t in (pos, scale, rotq, sh, opacity)]
+        return img, alpha, depth
+
+    @staticmethod
+    def backward(ctx, dl_dimg, dl_dalpha, dl_ddepth):
+        want = ctx.needs_input_grad[2:]
+        scene, b = ctx.saved
+        img, alpha, depth = ctx.saved_tensors
+        b = dict(b, img=img, alpha_plane=alpha, depth_plane=depth)
+        if dl_dimg is None:
+            dl_dimg = torch.zeros_like(img)
+        grads = ctx.dr._backward(ctx.vp, (scene, b), dl_dimg, want, dl_dalpha, dl_ddepth)
+        ctx.saved = None
+        out = [g.view(s) if g is not None else None for g, s in zip(grads, ctx.shapes)]
+        return (None, None, *out)
+
+
 class DifferentiableRenderer:
     """Renders one whole frame as the output of a torch.autograd.Function: `dr(pos, scale, rotq, sh, opacity, cam)`
     returns the planar [3, H, W] image, and `backward` runs lcgs_b200_render_backward (CUDA kernels, no reference
@@ -642,10 +672,16 @@ class DifferentiableRenderer:
     instances than `list_capacity` raises CapacityError in the forward.
 
     keep_means_2d_grad: keep the last backward's [P, 2] pixel-space mean gradient (the densification statistic) in
-    `means_2d_grad`."""
+    `means_2d_grad`.
+
+    aux: the call returns `(img [3, H, W], alpha [H, W], depth [H, W])`, the planes of `Renderer(aux=True)`:
+    accumulated opacity 1 - T and the sum of weight * view depth over the blended Gaussians (not normalised; the
+    expected depth is `depth / alpha` where alpha > 0, ordinary torch code).  All three are differentiable, so mask,
+    depth and opacity losses train the scene; the image is bit-identical to the one without aux."""
 
     def __init__(self, device: Device, width: int, height: int, list_capacity: int = 4_000_000, sh_deg: int = 3,
-                 bg_color=(0.0, 0.0, 0.0), scale_modifier: float = 1.0, keep_means_2d_grad: bool = False):
+                 bg_color=(0.0, 0.0, 0.0), scale_modifier: float = 1.0, keep_means_2d_grad: bool = False,
+                 aux: bool = False):
         self.device = device
         self.W, self.H = int(width), int(height)
         self.gx, self.gy = (self.W + 15) // 16, (self.H + 15) // 16
@@ -655,14 +691,16 @@ class DifferentiableRenderer:
         self.scale_modifier = float(scale_modifier)
         self.keep_means_2d_grad = keep_means_2d_grad
         self.means_2d_grad: Optional[torch.Tensor] = None
+        self.aux = bool(aux)
         dev = device.torch_device
         self.keys_unsorted = torch.zeros(self.capacity, dtype=torch.int64, device=dev)
         self.vals_unsorted = torch.zeros(self.capacity, dtype=torch.int32, device=dev)
         self.keys = torch.zeros(self.capacity, dtype=torch.int64, device=dev)
         self._reserved = -1
 
-    def __call__(self, pos, scale, rotq, sh, opacity, cam: Camera) -> torch.Tensor:
-        return _RenderFunction.apply(self, view_params(cam), pos, scale, rotq, sh, opacity)
+    def __call__(self, pos, scale, rotq, sh, opacity, cam: Camera):
+        fn = _RenderAuxFunction if self.aux else _RenderFunction
+        return fn.apply(self, view_params(cam), pos, scale, rotq, sh, opacity)
 
     def _scene(self, pos, scale, rotq, sh, opacity, alpha_consts) -> _capi.Scene:
         P = int(pos.shape[0])
@@ -680,6 +718,7 @@ class DifferentiableRenderer:
         f.ranges, f.list_capacity = _ptr(b["ranges"]), self.capacity
         f.target_img, f.radii = _ptr(b["img"]), _ptr(b["radii"])
         f.tile_row_begin, f.tile_row_end = 0, -1
+        f.target_alpha, f.target_depth = _ptr(b.get("alpha_plane")), _ptr(b.get("depth_plane"))
         return f
 
     def _forward(self, vp: ViewParams, pos, scale, rotq, sh, opacity):
@@ -699,6 +738,8 @@ class DifferentiableRenderer:
                  point_list=torch.empty(self.capacity, dtype=torch.int32, device=dev),
                  ranges=z(2 * max(self.gx * self.gy, 1), torch.int32), img=z(3 * self.W * self.H, torch.float32),
                  radii=z(P, torch.int32), alpha_consts=torch.empty(2 * P, dtype=torch.float32, device=dev))
+        if self.aux:
+            b.update(alpha_plane=z(self.W * self.H, torch.float32), depth_plane=z(self.W * self.H, torch.float32))
         stream = _stream_handle(None)
         d.check(d.lib.lcgs_b200_scene_prepare(d.ctx, P, _ptr(scene[4]), _ptr(b["alpha_consts"]), stream))
         c_scene = self._scene(*scene, b["alpha_consts"])
@@ -707,14 +748,16 @@ class DifferentiableRenderer:
         d.num_rendered()  # raises CapacityError on overflow
         return b["img"].view(3, self.H, self.W), (scene, b)
 
-    def _backward(self, vp: ViewParams, saved, dl_dimg: torch.Tensor, want) -> list:
+    def _backward(self, vp: ViewParams, saved, dl_dimg: torch.Tensor, want, dl_dalpha=None, dl_ddepth=None) -> list:
         d = self.device
         scene, b = saved
         P = int(scene[0].shape[0])
         dl = dl_dimg.detach().to(dtype=torch.float32).contiguous()
+        planes = [None if t is None else t.detach().to(dtype=torch.float32).contiguous() for t in (dl_dalpha, dl_ddepth)]
         grads = [torch.empty_like(t) if w else None for t, w in zip(scene, want)]
         g = _capi.Grad()
         g.dl_dimg = _ptr(dl)
+        g.dl_dalpha, g.dl_ddepth = _ptr(planes[0]), _ptr(planes[1])
         g.grad_pos, g.grad_scale, g.grad_rotq, g.grad_sh, g.grad_opacity = (_ptr(t) for t in grads)
         m2 = torch.empty((P, 2), dtype=torch.float32, device=dl.device) if self.keep_means_2d_grad else None
         g.grad_means_2d = _ptr(m2)
