@@ -66,13 +66,20 @@ def scene_arrays(key, P, deg=3, dense=False):
     return [np.ascontiguousarray(a, np.float32) for a in (sc.pos, scale, sc.rotq, sh, opacity)], pose
 
 
-def gpu_backward(lcgs, dev, arrays, pose, W, H, deg, bg, R, list_capacity=2_000_000):
+def gpu_backward(lcgs, dev, arrays, pose, W, H, deg, bg, R, list_capacity=2_000_000, scale_modifier=1.0,
+                 prepare_scene=True):
     """Render with Renderer, then lcgs_b200_render_backward with every output requested; returns (renderer, grads)."""
-    r = lcgs.Renderer(dev, *arrays, W, H, list_capacity=list_capacity, sh_deg=deg, bg_color=bg)
+    r = lcgs.Renderer(dev, *arrays, W, H, list_capacity=list_capacity, sh_deg=deg, bg_color=bg,
+                      scale_modifier=scale_modifier, prepare_scene=prepare_scene)
     cam = lcgs.make_camera(*pose, W, H)
     vp = lcgs.view_params(cam)
     r.render_async(vp)
     dev.num_rendered()
+    return r, run_backward(lcgs, dev, r, vp, R)
+
+
+def run_backward(lcgs, dev, r, vp, R):
+    """lcgs_b200_render_backward of the frame `r` last rendered (with view `vp`), every output requested."""
     P = r.P
     out = {n: torch.zeros_like(t) for n, t in zip(NAMES, (r.pos, r.scale, r.rotq, r.sh, r.opacity))}
     out["means_2d"] = torch.zeros(P, 2, device="cuda")
@@ -85,14 +92,15 @@ def gpu_backward(lcgs, dev, arrays, pose, W, H, deg, bg, R, list_capacity=2_000_
         setattr(g, "grad_" + n, out[n].data_ptr())
     dev.check(dev.lib.lcgs_b200_render_backward(dev.ctx, C.byref(r.c_scene), C.byref(vp), C.byref(r.c_frame), C.byref(g), None))
     torch.cuda.synchronize()
-    return r, {k: v.cpu().numpy() for k, v in out.items()}
+    return {k: v.cpu().numpy() for k, v in out.items()}
 
 
-def reference(arrays, pose, W, H, deg, bg, R):
+def reference(arrays, pose, W, H, deg, bg, R, scale_modifier=1.0):
     vp = orc.view_params(orc.make_camera(*pose, W, H))
-    fr = orc.forward(arrays[0], arrays[1], arrays[2], arrays[3], arrays[4], vp, bg=bg, sh_deg=deg)
+    fr = orc.forward(arrays[0], arrays[1], arrays[2], arrays[3], arrays[4], vp, bg=bg, sh_deg=deg,
+                     scale_modifier=scale_modifier)
     L = [tr.leaf(a) for a in arrays]
-    img, (means, conic, color) = tr.forward(*L, vp, fr, deg=deg, bg=bg, keep_2d=True)
+    img, (means, conic, color) = tr.forward(*L, vp, fr, deg=deg, bg=bg, scale_modifier=scale_modifier, keep_2d=True)
     (img * torch.from_numpy(np.asarray(R, np.float64))).sum().backward()
     want = {n: x.grad.numpy() for n, x in zip(NAMES, L)}
     want.update(means_2d=means.grad.numpy(), conic=conic.grad.numpy(), color=color.grad.numpy())

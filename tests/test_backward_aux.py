@@ -37,8 +37,10 @@ def cuda32(a):
     return None if a is None else torch.from_numpy(np.ascontiguousarray(a, np.float32)).cuda()
 
 
-def render_aux_frame(lcgs, dev, arrays, pose, W, H, deg, bg, list_capacity=2_000_000):
-    r = lcgs.Renderer(dev, *arrays, W, H, list_capacity=list_capacity, sh_deg=deg, bg_color=bg, aux=True)
+def render_aux_frame(lcgs, dev, arrays, pose, W, H, deg, bg, list_capacity=2_000_000, scale_modifier=1.0,
+                     prepare_scene=True):
+    r = lcgs.Renderer(dev, *arrays, W, H, list_capacity=list_capacity, sh_deg=deg, bg_color=bg, aux=True,
+                      scale_modifier=scale_modifier, prepare_scene=prepare_scene)
     vp = lcgs.view_params(lcgs.make_camera(*pose, W, H))
     r.render_async(vp)
     dev.num_rendered()
@@ -56,9 +58,10 @@ def grad_struct(lcgs, P, dl, da, dd, fill=0.0):
     return g, out
 
 
-def gpu_backward_aux(lcgs, dev, arrays, pose, W, H, deg, bg, R, Ra, Rd, list_capacity=2_000_000):
+def gpu_backward_aux(lcgs, dev, arrays, pose, W, H, deg, bg, R, Ra, Rd, list_capacity=2_000_000, scale_modifier=1.0,
+                     prepare_scene=True):
     """Render with Renderer(aux=True), then lcgs_b200_render_backward with every output; Ra / Rd None = NULL."""
-    r, vp = render_aux_frame(lcgs, dev, arrays, pose, W, H, deg, bg, list_capacity)
+    r, vp = render_aux_frame(lcgs, dev, arrays, pose, W, H, deg, bg, list_capacity, scale_modifier, prepare_scene)
     dl, da, dd = cuda32(R), cuda32(Ra), cuda32(Rd)
     g, out = grad_struct(lcgs, r.P, dl, da, dd)
     out["sh"] = torch.zeros_like(r.sh)
@@ -70,11 +73,13 @@ def gpu_backward_aux(lcgs, dev, arrays, pose, W, H, deg, bg, R, Ra, Rd, list_cap
     return r, got
 
 
-def reference_aux(arrays, pose, W, H, deg, bg, R, Ra, Rd):
+def reference_aux(arrays, pose, W, H, deg, bg, R, Ra, Rd, scale_modifier=1.0):
     vp = orc.view_params(orc.make_camera(*pose, W, H))
-    fr = orc.forward(arrays[0], arrays[1], arrays[2], arrays[3], arrays[4], vp, bg=bg, sh_deg=deg)
+    fr = orc.forward(arrays[0], arrays[1], arrays[2], arrays[3], arrays[4], vp, bg=bg, sh_deg=deg,
+                     scale_modifier=scale_modifier)
     L = [tr.leaf(a) for a in arrays]
-    img, alpha, dmap, (means, conic, color, depth) = tra.forward_aux(*L, vp, fr, deg=deg, bg=bg)
+    img, alpha, dmap, (means, conic, color, depth) = tra.forward_aux(*L, vp, fr, deg=deg, bg=bg,
+                                                                     scale_modifier=scale_modifier)
     t = lambda a: torch.from_numpy(np.asarray(a, np.float64))  # noqa: E731
     loss = (img * t(R)).sum()
     if Ra is not None:

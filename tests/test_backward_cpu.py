@@ -278,3 +278,34 @@ def test_backward_and_record_kernels_sass():
     blend = [v for k, v in funcs.items() if "blend_backward_kernel" in k][0]
     assert blend["LDGSTS"] >= 3  # the three record planes, staged as in the forward
     assert blend["RED"] + blend["REDG"] + blend["ATOMG"] >= 1
+
+
+@pytest.mark.parametrize("key,P,W,H,where", [("C3", 4000, 320, 180, "longest"), ("C2", 5000, 309, 205, "corner")])
+def test_windowed_reference_equals_the_whole_frame(key, P, W, H, where):
+    """test_backward_edges.py differentiates 3x3-tile windows of full-size frames with the float64 reference restricted
+    to the window's tiles and to the Gaussians they list.  On a frame small enough for the whole reference, with dL/dimg
+    zero outside the window, that gives the whole frame's gradients, and every other Gaussian's are zero."""
+    from test_backward import reference, scene_arrays
+    from test_backward_edges import window, window_reference
+
+    arrays, pose = scene_arrays(key, P)
+    fr = orc.forward(*arrays, orc.view_params(orc.make_camera(*pose, W, H)))
+    tx0, ty0 = window(fr, W, H, where)
+    gx, _ = orc.grids(W, H)
+    x0, y0 = 16 * tx0, 16 * ty0
+    x1, y1 = min(x0 + 48, W), min(y0 + 48, H)
+    if where == "corner":
+        assert x1 - x0 < 48 and y1 - y0 < 48  # ragged in both directions
+    Rw = np.random.default_rng(18).uniform(-1.0, 1.0, (3, y1 - y0, x1 - x0)).astype(np.float32)
+    R = np.zeros((3, H, W))
+    R[:, y0:y1, x0:x1] = Rw
+    _, whole, _ = reference(arrays, pose, W, H, 3, (0.0, 0.0, 0.0), R)
+    dec = tr.decisions(fr, arrays[4], W, H, [ty * gx + tx for ty in range(ty0, ty0 + 3) for tx in range(tx0, tx0 + 3)])
+    ids = np.unique(np.concatenate([d[2] for d in dec]))
+    assert ids.size > 20
+    want = window_reference(arrays, pose, W, H, 1.0, dec, ids, x0, y0, Rw)
+    rest = np.ones(P, bool)
+    rest[ids] = False
+    for n in want:
+        assert not np.any(whole[n][rest]), n
+        assert rel_l2(want[n], whole[n][ids]) <= 1e-12, n

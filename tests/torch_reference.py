@@ -96,14 +96,15 @@ def _f32_power(mx, my, conic, pxs, pys):
     return (bdx.astype(np.float64) * dy.astype(np.float64) + inner2.astype(np.float64)).astype(f)
 
 
-def decisions(fr, opacity, W, H):
+def decisions(fr, opacity, W, H, tiles=None):
     """Per tile: (pixel x, pixel y, Gaussian ids, blended mask [pixels, entries]) from the oracle's frame, with the
-    oracle's alpha test (power <= 0 and power >= alpha_threshold(opacity)) and its float32 saturation stop."""
+    oracle's alpha test (power <= 0 and power >= alpha_threshold(opacity)) and its float32 saturation stop.
+    tiles: only these tile indices (default: every tile of the frame)."""
     gx, gy = orc.grids(W, H)
     opacity = np.ascontiguousarray(opacity, np.float32)
     thr = {}
     out = []
-    for t in range(gx * gy):
+    for t in (range(gx * gy) if tiles is None else tiles):
         s, e = int(fr.ranges[t, 0]), int(fr.ranges[t, 1])
         bx, by = t % gx, t // gx
         ys, xs = np.meshgrid(np.arange(by * 16, by * 16 + 16), np.arange(bx * 16, bx * 16 + 16), indexing="ij")
@@ -134,6 +135,17 @@ def decisions(fr, opacity, W, H):
 def render(means, conic, color, opacity, dec, W, H, bg=(0.0, 0.0, 0.0)):
     """Planar [3, H, W] float64 image from per-Gaussian tensors and the frozen decisions."""
     bgt = torch.tensor(bg, dtype=F64)
+    pixs, cols = blend_pixels(means, conic, color, opacity, dec, W, bg)
+    img = bgt[:, None].expand(3, H * W)
+    if pixs:
+        img = img.index_put((torch.arange(3)[:, None], torch.cat(pixs)[None]), torch.cat(cols).T)
+    return img.reshape(3, H, W)
+
+
+def blend_pixels(means, conic, color, opacity, dec, W, bg=(0.0, 0.0, 0.0)):
+    """The blend of the pixels of the decisions' tiles that blend anything: (flat pixel indices y * W + x, float64
+    colours [n, 3]) per tile.  The ids in `dec` index the per-Gaussian tensors, which may hold just the Gaussians the tiles list."""
+    bgt = torch.tensor(bg, dtype=F64)
     pixs, cols = [], []
     for xs, ys, ids, blended in dec:
         if ids.size == 0 or not blended.any():
@@ -155,10 +167,7 @@ def render(means, conic, color, opacity, dec, W, H, bg=(0.0, 0.0, 0.0)):
         Cpix = wgt @ color[idt] + T_fin[:, None] * bgt[None]
         pixs.append(torch.from_numpy(xs + W * ys))
         cols.append(Cpix)
-    img = bgt[:, None].expand(3, H * W)
-    if pixs:
-        img = img.index_put((torch.arange(3)[:, None], torch.cat(pixs)[None]), torch.cat(cols).T)
-    return img.reshape(3, H, W)
+    return pixs, cols
 
 
 def forward(pos, scale, rotq, sh, opacity, vp, fr, deg=3, bg=(0.0, 0.0, 0.0), scale_modifier=1.0, dec=None,
