@@ -277,6 +277,18 @@ LCGS_B200_API int lcgs_b200_render(lcgs_b200_ctx* ctx, const lcgs_b200_scene* sc
  *     c_i . G + z_i dL/dD + dL/dA, C . G becomes C . G + D dL/dD + A dL/dA, and dL/dz_i = sum over pixels w_i dL/dD,
  *     which reaches pos through the view transform.  A and D are read back from the frame, like C.  n_contrib is
  *     discrete and has no gradient.
+ *   camera pose (optional grad_view / grad_cam_pos): with V = vp->view (column-major, p_view[k] =
+ *     sum_c V[c*4+k] p[c] + V[12+k]) and dv = dL/dp_view of each Gaussian with tiles_touched > 0 (the depth plane's
+ *     dL/dz included), summed over those Gaussians:
+ *       dL/dV[c*4+k] = sum dv[k] p[c] (c < 3),  dL/dV[12+k] = sum dv[k],
+ *       plus, through the EWA Jacobian's rows T0 = J00 V_col0 + J02 V_col2 and T1 = J11 V_col1 + J12 V_col2 of each
+ *       Gaussian, dL/dV[r*4+0] += J00 dL/dT0[r], dL/dV[r*4+1] += J11 dL/dT1[r], dL/dV[r*4+2] += J02 dL/dT0[r] +
+ *       J12 dL/dT1[r].  V[3], V[7], V[11] and V[15] never enter the forward and get 0.
+ *     dL/dcam_pos = -(sum of the SH view-direction terms of dL/dpos): zero at SH degree 0 and for Gaussians whose
+ *     three colour channels are all clamped.  proj, tanfov and focal are held fixed.  The alpha and depth planes reach
+ *     the pose like the image does (with dl_ddepth the pose gradient includes the depth loss).  An empty frame gives
+ *     zeros.  The per-Gaussian terms are summed per CTA and then, in double and a fixed order, over the CTAs.  The
+ *     scene gradients are the same with or without the pose outputs.
  * Gradients are summed with float atomics: the last bits vary from run to run. */
 typedef struct lcgs_b200_grad {
     const float* dl_dimg; /* [3][H][W], layout of target_img */
@@ -293,6 +305,10 @@ typedef struct lcgs_b200_grad {
     /* optional [P]: dL/d(view depth) of each Gaussian, the blend's part (like grad_means_2d); all zeros without
        dl_ddepth */
     float* grad_depth;
+    /* optional, device memory, 4-byte aligned, overwritten: dL/d(vp->view) [16] (column-major like vp->view;
+       entries 3, 7, 11, 15 are 0) and dL/d(vp->cam_pos) [3] (through the SH view direction only). */
+    float* grad_view;
+    float* grad_cam_pos;
 } lcgs_b200_grad;
 
 /* Backward of one whole frame.  `scene`, `vp` and `frame` are those the frame was rendered with; the call reads only

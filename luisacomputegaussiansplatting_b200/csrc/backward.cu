@@ -19,6 +19,12 @@
 //  * preprocess_backward_kernel : one thread per Gaussian; Gaussians with tiles_touched == 0 get zeros.  Recomputes
 //    the forward's intermediates from the scene and chains the packed 2D gradient to pos / scale / rotq / sh /
 //    opacity (dL/dz through the view z).
+//  * preprocess_pose_grad_kernel : the same body (preprocess_backward_body<true>), run instead when dL/d(view) or
+//    dL/d(cam_pos) is requested.  Each thread also keeps its Gaussian's 15 pose terms (12 of the view, 3 of the camera
+//    position; zero past P and for tiles_touched == 0), the warp sums them with shuffles, the CTA's four warps in
+//    shared memory, and one double partial per CTA goes to the context's pose_ws ([15][CTAs]).
+//  * pose_grad_reduce_kernel : one CTA per pose term sums that term's partials in a fixed order, in double, so the
+//    pose gradient is the same from run to run given the same per-Gaussian 2D gradients.
 // Float atomics make the summation order, and so the last bits of the gradients, vary from run to run; the forward
 // is untouched and stays bit-reproducible.
 #include "blend_walk.cuh"
@@ -189,9 +195,12 @@ struct PreprocessGradArgs {
     float *         grad_means_2d, *grad_conic, *grad_color, *grad_depth;
 };
 
-// 6 CTAs per SM: 80 registers, no spills.  Unbounded, the depth plane's dL/dz add in project_backward makes ptxas take
-// 96 registers (5 CTAs per SM).
-__global__ void __launch_bounds__(128, 6) preprocess_backward_kernel(const __grid_constant__ PreprocessGradArgs a)
+// One Gaussian per thread.  POSE: pose[15] (zeroed by the caller) receives the Gaussian's terms of dL/d(view) (pose[j]
+// for view[pose_view_index(j)], j < 12) and dL/d(cam_pos) (pose[12..14]), and project_backward / sh_color_backward run
+// even when no scene gradient is requested (tracking against a frozen scene).  The early returns leave the pose terms
+// at 0 and only end the body: the caller's reduction still runs on every thread.
+template <bool POSE>
+__device__ __forceinline__ void preprocess_backward_body(const PreprocessGradArgs& a, float* pose)
 {
     const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= a.P) return;
@@ -229,14 +238,29 @@ __global__ void __launch_bounds__(128, 6) preprocess_backward_kernel(const __gri
     }
     const float px = __ldg(a.pos + 3 * i), py = __ldg(a.pos + 3 * i + 1), pz = __ldg(a.pos + 3 * i + 2);
     float       dpos[3] = { 0.f, 0.f, 0.f }, dscale[3], drot[4];
-    if (a.grad_pos || a.grad_scale || a.grad_rotq) {
+    if (POSE || a.grad_pos || a.grad_scale || a.grad_rotq) {
         const float4 q = __ldg(reinterpret_cast<const float4*>(a.rotq) + i);
-        project_backward(a.vp, a.scale_modifier, px, py, pz, __ldg(a.scale + 3 * i), __ldg(a.scale + 3 * i + 1),
-                         __ldg(a.scale + 3 * i + 2), q.x, q.y, q.z, q.w, g2, dpos, dscale, drot);
+        if constexpr (POSE)
+            project_backward_pose(a.vp, a.scale_modifier, px, py, pz, __ldg(a.scale + 3 * i), __ldg(a.scale + 3 * i + 1),
+                                  __ldg(a.scale + 3 * i + 2), q.x, q.y, q.z, q.w, g2, dpos, dscale, drot, pose);
+        else
+            project_backward(a.vp, a.scale_modifier, px, py, pz, __ldg(a.scale + 3 * i), __ldg(a.scale + 3 * i + 1),
+                             __ldg(a.scale + 3 * i + 2), q.x, q.y, q.z, q.w, g2, dpos, dscale, drot);
     }
-    if (a.grad_pos || gsh)
+    if constexpr (POSE) {
+        // the view-direction term on its own: it is dL/dpos's and, negated, dL/dcam_pos's (dpos gets the same sum
+        // as when sh_color_backward adds it in place)
+        float ddir[3] = { 0.f, 0.f, 0.f };
+        sh_color_backward(a.sh_deg, a.vp.cam_pos, px, py, pz, GlobalShIn{ a.sh + (size_t)i * feat * 3 }, g2 + kG2Red,
+                          GlobalShOut{ gsh }, ddir);
+        for (int k = 0; k < 3; k++) {
+            dpos[k] += ddir[k];
+            pose[12 + k] = -ddir[k];
+        }
+    } else if (a.grad_pos || gsh) {
         sh_color_backward(a.sh_deg, a.vp.cam_pos, px, py, pz, GlobalShIn{ a.sh + (size_t)i * feat * 3 }, g2 + kG2Red,
                           GlobalShOut{ gsh }, dpos);
+    }
     if (a.grad_pos)
         for (int k = 0; k < 3; k++) a.grad_pos[3 * i + k] = dpos[k];
     if (a.grad_scale)
@@ -250,13 +274,88 @@ __global__ void __launch_bounds__(128, 6) preprocess_backward_kernel(const __gri
     }
 }
 
+// 6 CTAs per SM: 80 registers, no spills.  Unbounded, the depth plane's dL/dz add in project_backward makes ptxas take
+// 96 registers (5 CTAs per SM).
+__global__ void __launch_bounds__(128, 6) preprocess_backward_kernel(const __grid_constant__ PreprocessGradArgs a)
+{
+    preprocess_backward_body<false>(a, nullptr);
+}
+
+constexpr int kPoseTerms = 15;  // 12 of the view (pose_view_index), 3 of the camera position
+
+struct PoseGradArgs {
+    PreprocessGradArgs a;
+    double*            partials;  // [kPoseTerms][gridDim.x]
+};
+
+// 96 registers (5 CTAs per SM), no spills; bounded to 6 CTAs per SM (80 registers) ptxas spills 32 bytes.
+__global__ void __launch_bounds__(128) preprocess_pose_grad_kernel(const __grid_constant__ PoseGradArgs pa)
+{
+    __shared__ float s_warp[kPoseTerms][4];
+    float            pose[kPoseTerms];
+#pragma unroll
+    for (int k = 0; k < kPoseTerms; k++) pose[k] = 0.0f;
+    preprocess_backward_body<true>(pa.a, pose);
+    const unsigned FULL = 0xFFFFFFFFu;
+    const int      lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+    for (int k = 0; k < kPoseTerms; k++) {
+        float v = pose[k];
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(FULL, v, o);
+        if (lane == 0) s_warp[k][warp] = v;
+    }
+    __syncthreads();
+    if (threadIdx.x < kPoseTerms) {
+        const int k = threadIdx.x;
+        pa.partials[(size_t)k * gridDim.x + blockIdx.x] =
+            (((double)s_warp[k][0] + (double)s_warp[k][1]) + (double)s_warp[k][2]) + (double)s_warp[k][3];
+    }
+}
+
+// Block k < kPoseTerms sums term k's n partials in a fixed order (strided per thread, then a fixed tree) and writes
+// it; block kPoseTerms writes the four view entries (3, 7, 11, 15) the forward never reads.
+constexpr int kPoseReduceThreads = 512;
+
+__global__ void __launch_bounds__(kPoseReduceThreads)
+    pose_grad_reduce_kernel(const double* __restrict__ partials, uint32_t n, float* __restrict__ grad_view,
+                            float* __restrict__ grad_cam_pos)
+{
+    __shared__ double s[kPoseReduceThreads];
+    const int         k = blockIdx.x;
+    if (k == kPoseTerms) {
+        if (threadIdx.x < 4 && grad_view) grad_view[threadIdx.x * 4 + 3] = 0.0f;
+        return;
+    }
+    const double* p   = partials + (size_t)k * n;
+    double        acc = 0.0;
+    for (uint32_t j = threadIdx.x; j < n; j += kPoseReduceThreads) acc += p[j];
+    s[threadIdx.x] = acc;
+    __syncthreads();
+    for (int w = kPoseReduceThreads / 2; w > 0; w >>= 1) {
+        if ((int)threadIdx.x < w) s[threadIdx.x] += s[threadIdx.x + w];
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) {
+        if (k < 12) {
+            if (grad_view) grad_view[pose_view_index(k)] = (float)s[0];
+        } else if (grad_cam_pos) {
+            grad_cam_pos[k - 12] = (float)s[0];
+        }
+    }
+}
+
 static inline uint32_t bwd_div_up(long a, long b) { return (uint32_t)((a + b - 1) / b); }
 
 int launch_render_backward(lcgs_b200_ctx* ctx, const lcgs_b200_scene* sc, const lcgs_b200_view_params* vp,
                            const lcgs_b200_frame* fr, const lcgs_b200_grad* gr, cudaStream_t s)
 {
     const int P = sc->num_gaussians;
-    if (P <= 0) return LCGS_B200_OK;
+    if (P <= 0) {  // no Gaussian: the pose gradient is zero
+        if (gr->grad_view) LCGS_CUDA_CHECK(ctx, cudaMemsetAsync(gr->grad_view, 0, 16 * sizeof(float), s));
+        if (gr->grad_cam_pos) LCGS_CUDA_CHECK(ctx, cudaMemsetAsync(gr->grad_cam_pos, 0, 3 * sizeof(float), s));
+        return LCGS_B200_OK;
+    }
     const int      W = fr->width, H = fr->height;
     const uint32_t gx = (uint32_t)((W + 15) / 16), gy = (uint32_t)((H + 15) / 16);
     const int      num_tiles = (int)(gx * gy);  // whole frames only
@@ -294,7 +393,19 @@ int launch_render_backward(lcgs_b200_ctx* ctx, const lcgs_b200_scene* sc, const 
     a.grad_opacity = gr->grad_opacity;
     a.grad_means_2d = gr->grad_means_2d; a.grad_conic = gr->grad_conic; a.grad_color = gr->grad_color;
     a.grad_depth = gr->grad_depth;
-    preprocess_backward_kernel<<<bwd_div_up(P, 128), 128, 0, s>>>(a);
+    if (!gr->grad_view && !gr->grad_cam_pos) {
+        preprocess_backward_kernel<<<bwd_div_up(P, 128), 128, 0, s>>>(a);
+        LCGS_CUDA_CHECK(ctx, cudaGetLastError());
+        return LCGS_B200_OK;
+    }
+    const uint32_t ctas = bwd_div_up(P, 128);
+    if ((rc = ws_reserve(ctx, ctx->pose_ws, (size_t)kPoseTerms * ctas * sizeof(double)))) return rc;
+    PoseGradArgs pa;
+    pa.a        = a;
+    pa.partials = (double*)ctx->pose_ws.ptr;
+    preprocess_pose_grad_kernel<<<ctas, 128, 0, s>>>(pa);
+    LCGS_CUDA_CHECK(ctx, cudaGetLastError());
+    pose_grad_reduce_kernel<<<kPoseTerms + 1, kPoseReduceThreads, 0, s>>>(pa.partials, ctas, gr->grad_view, gr->grad_cam_pos);
     LCGS_CUDA_CHECK(ctx, cudaGetLastError());
     return LCGS_B200_OK;
 }

@@ -278,6 +278,7 @@ int lcgs_b200_ctx_destroy(lcgs_b200_ctx* ctx)
     if (ctx->tile_order_ws.ptr) cudaFree(ctx->tile_order_ws.ptr);
     if (ctx->emit_ws.ptr) cudaFree(ctx->emit_ws.ptr);
     if (ctx->grad_ws.ptr) cudaFree(ctx->grad_ws.ptr);
+    if (ctx->pose_ws.ptr) cudaFree(ctx->pose_ws.ptr);
     for (int i = 0; i < 16; i++)
         if (ctx->ev[i]) cudaEventDestroy(ctx->ev[i]);
     for (int i = 0; i < 3; i++)
@@ -595,6 +596,8 @@ int lcgs_b200_render_backward(lcgs_b200_ctx* ctx, const lcgs_b200_scene* sc, con
                           (!gr->dl_dalpha || aligned(fr->target_alpha, 4)) &&
                           (!gr->dl_ddepth || (aligned(fr->target_depth, 4) && aligned(fr->depth, 4))),
                  "render_backward: aux plane buffers must be 4-byte aligned");
+    LCGS_REQUIRE(ctx, aligned(gr->grad_view, 4) && aligned(gr->grad_cam_pos, 4),
+                 "render_backward: grad_view / grad_cam_pos must be 4-byte aligned");
     return launch_render_backward(ctx, sc, vp, fr, gr, as_stream(stream));
 }
 

@@ -54,6 +54,7 @@ struct lcgs_b200_ctx {
     lcgs_b200::Workspace tile_order_ws;  // blend: tile ids, longest list first
     lcgs_b200::Workspace emit_ws;        // emission: entries + pieces of the Gaussians expanded by emit_big_kernel
     lcgs_b200::Workspace grad_ws;        // backward: packed per-Gaussian gradient of the blend's inputs [P][12]
+    lcgs_b200::Workspace pose_ws;        // backward: per-CTA partial sums of the pose gradient [15][CTAs] (double)
     // per-stage timing
     int          profiling  = 0;
     cudaEvent_t  ev[16];

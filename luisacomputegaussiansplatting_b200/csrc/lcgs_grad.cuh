@@ -24,6 +24,13 @@
 //   aux planes (the blend's optional alpha and depth planes, A = 1 - T_{n+1} and D = sum w_i z_i): two more channels
 //   with colours 1 and z_i and a background of 0 (see PixelGradAux); depth z = view z, so dL/dz joins dL/dvz in
 //   project_backward.
+//   camera pose (project_backward_pose, preprocess_pose_grad_kernel): V = vp.view, column-major, p_view[k] =
+//   sum_c V[c*4+k] p[c] + V[12+k].  With dv = dL/dp_view (dL/dz of the depth plane included) and the EWA Jacobian's
+//   T0 = J00 V_col0 + J02 V_col2, T1 = J11 V_col1 + J12 V_col2 (rows r of mat3(view)):
+//     dL/dV[c*4+k] = dv[k] p[c] (c < 3),  dL/dV[12+k] = dv[k],
+//     dL/dV[r*4+0] += J00 dT0[r],  dL/dV[r*4+1] += J11 dT1[r],  dL/dV[r*4+2] += J02 dT0[r] + J12 dT1[r];
+//   V[3], V[7], V[11], V[15] never enter the forward.  dL/dcam_pos = -(sh_color's view-direction term of dL/dpos),
+//   zero for degree 0 and where every colour channel is clamped.  proj, focal and tanfov are held fixed.
 #pragma once
 
 #include "lcgs_math.cuh"
@@ -242,11 +249,12 @@ LCGS_HD void sh_color_backward(int deg, const float* cam_pos, float px, float py
 // ---------------------------------------------------------------------------------------------
 // Projection backward: from the packed 2D gradient g2 (pixel mean, conic) of one visible Gaussian to dL/dpos,
 // dL/dscale and dL/drotq (stored order r, x, y, z).  dpos is accumulated into (the SH term adds to it too), dscale
-// and drot are written.
+// and drot are written.  POSE: dL/d(view) is accumulated into dview[12], dview[c*3+k] for V[c*4+k] (k < 3).
 // ---------------------------------------------------------------------------------------------
-LCGS_HD void project_backward(const ViewParams& vp, float scale_modifier, float px, float py, float pz, float s0, float s1,
-                              float s2, float qr, float qx, float qy, float qz, const float* g2, float* dpos, float* dscale,
-                              float* drot)
+template <bool POSE>
+LCGS_HD void project_backward_t(const ViewParams& vp, float scale_modifier, float px, float py, float pz, float s0,
+                                float s1, float s2, float qr, float qx, float qy, float qz, const float* g2, float* dpos,
+                                float* dscale, float* drot, float* dview)
 {
     const ViewPoint pv = view_transform(vp, px, py, pz);
     // ---- forward intermediates, as ewa_cov2d computes them
@@ -390,6 +398,41 @@ LCGS_HD void project_backward(const ViewParams& vp, float scale_modifier, float 
     dpos[0] += (dvx * V[0] + dvy * V[1]) + dvz * V[2];
     dpos[1] += (dvx * V[4] + dvy * V[5]) + dvz * V[6];
     dpos[2] += (dvx * V[8] + dvy * V[9]) + dvz * V[10];
+    if constexpr (POSE) {
+        // the affine map p_view = mat3(view) p + view[12..14]
+        const float dv[3] = { dvx, dvy, dvz }, p[3] = { px, py, pz };
+#pragma unroll
+        for (int k = 0; k < 3; k++) {
+#pragma unroll
+            for (int c = 0; c < 3; c++) dview[c * 3 + k] += dv[k] * p[c];
+            dview[9 + k] += dv[k];
+        }
+        // the rows of mat3(view) in T0 and T1
+#pragma unroll
+        for (int r = 0; r < 3; r++) {
+            dview[r * 3 + 0] += J00 * dT0[r];
+            dview[r * 3 + 1] += J11 * dT1[r];
+            dview[r * 3 + 2] += J02 * dT0[r] + J12 * dT1[r];
+        }
+    }
 }
+
+LCGS_HD void project_backward(const ViewParams& vp, float scale_modifier, float px, float py, float pz, float s0, float s1,
+                              float s2, float qr, float qx, float qy, float qz, const float* g2, float* dpos, float* dscale,
+                              float* drot)
+{
+    project_backward_t<false>(vp, scale_modifier, px, py, pz, s0, s1, s2, qr, qx, qy, qz, g2, dpos, dscale, drot, nullptr);
+}
+
+// project_backward that also accumulates dL/d(view) into dview[12] (dview[c*3+k] for vp.view[c*4+k], k < 3).
+LCGS_HD void project_backward_pose(const ViewParams& vp, float scale_modifier, float px, float py, float pz, float s0,
+                                   float s1, float s2, float qr, float qx, float qy, float qz, const float* g2, float* dpos,
+                                   float* dscale, float* drot, float* dview)
+{
+    project_backward_t<true>(vp, scale_modifier, px, py, pz, s0, s1, s2, qr, qx, qy, qz, g2, dpos, dscale, drot, dview);
+}
+
+// The index into vp.view [16] of pose term j < 12 (dview[j] of project_backward_pose).
+LCGS_HD int pose_view_index(int j) { return (j / 3) * 4 + j % 3; }
 
 }  // namespace lcgs_b200

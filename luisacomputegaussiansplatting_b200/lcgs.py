@@ -67,6 +67,12 @@ def world_to_local_matrix(cam: Camera) -> np.ndarray:
     return _mat(_capi.load().lcgs_b200_world_to_local_matrix, C.byref(cam))
 
 
+def world_to_camera(cam: Camera) -> np.ndarray:
+    """[4, 4] float32, row-major: p_cam = M[:3, :3] @ p + M[:3, 3], the transpose of world_to_local_matrix's
+    column-major array.  The pose input of DifferentiableRenderer."""
+    return np.ascontiguousarray(world_to_local_matrix(cam).reshape(4, 4).T)
+
+
 def projection_matrix(tanfovx: float, tanfovy: float, znear: float = 0.1, zfar: float = 100.0) -> np.ndarray:
     return _mat(_capi.load().lcgs_b200_projection_matrix, tanfovx, tanfovy, znear, zfar)
 
@@ -607,25 +613,42 @@ def _scene_input(t: torch.Tensor, device: torch.device) -> torch.Tensor:
     return t if t.data_ptr() % 16 == 0 else t.clone()
 
 
+def _pose_like(*ts):
+    """(device, dtype) of the pose inputs given to the Function (empty when it was called without them)."""
+    return [] if all(t is None for t in ts) else [None if t is None else (t.device, t.dtype) for t in ts]
+
+
+def _pose_want(ctx) -> tuple:
+    return tuple(ctx.needs_input_grad[7:9]) + (False, False)[len(ctx.needs_input_grad[7:9]):]
+
+
+def _pose_grads(ctx, pose) -> list:
+    """The pose gradients on their inputs' device and dtype, one per pose input the Function was given."""
+    return [None if g is None or like is None else g.to(*like) for g, like in zip(pose, ctx.pose_like)]
+
+
 class _RenderFunction(torch.autograd.Function):
+    # view: the [4, 4] world-to-camera tensor vp.view was taken from, cam_pos: the [3] tensor vp.cam_pos was taken
+    # from (None: the camera's own); their gradients come from grad_view and grad_cam_pos
     @staticmethod
-    def forward(ctx, dr: "DifferentiableRenderer", vp: ViewParams, pos, scale, rotq, sh, opacity):
+    def forward(ctx, dr: "DifferentiableRenderer", vp: ViewParams, pos, scale, rotq, sh, opacity, view=None, cam_pos=None):
         img, (scene, b) = dr._forward(vp, pos, scale, rotq, sh, opacity)
         # the image is the output: it goes through save_for_backward (an attribute would make a reference cycle)
         ctx.save_for_backward(img)
         ctx.dr, ctx.vp, ctx.saved = dr, vp, (scene, {k: v for k, v in b.items() if k != "img"})
         ctx.shapes = [t.shape for t in (pos, scale, rotq, sh, opacity)]
+        ctx.pose_like = _pose_like(view, cam_pos)
         return img
 
     @staticmethod
     def backward(ctx, dl_dimg):
-        want = ctx.needs_input_grad[2:]
+        want = ctx.needs_input_grad[2:7]
         scene, b = ctx.saved
         b = dict(b, img=ctx.saved_tensors[0])
-        grads = ctx.dr._backward(ctx.vp, (scene, b), dl_dimg, want)
+        grads, pose = ctx.dr._backward(ctx.vp, (scene, b), dl_dimg, want, pose_want=_pose_want(ctx))
         ctx.saved = None  # the frame's buffers are released with the graph
         out = [g.view(s) if g is not None else None for g, s in zip(grads, ctx.shapes)]
-        return (None, None, *out)
+        return (None, None, *out, *_pose_grads(ctx, pose))
 
 
 class _RenderAuxFunction(torch.autograd.Function):
@@ -634,7 +657,7 @@ class _RenderAuxFunction(torch.autograd.Function):
     as a zero gradient."""
 
     @staticmethod
-    def forward(ctx, dr: "DifferentiableRenderer", vp: ViewParams, pos, scale, rotq, sh, opacity):
+    def forward(ctx, dr: "DifferentiableRenderer", vp: ViewParams, pos, scale, rotq, sh, opacity, view=None, cam_pos=None):
         img, (scene, b) = dr._forward(vp, pos, scale, rotq, sh, opacity)
         alpha, depth = b["alpha_plane"].view(dr.H, dr.W), b["depth_plane"].view(dr.H, dr.W)
         ctx.set_materialize_grads(False)
@@ -642,20 +665,22 @@ class _RenderAuxFunction(torch.autograd.Function):
         ctx.dr, ctx.vp = dr, vp
         ctx.saved = (scene, {k: v for k, v in b.items() if k not in ("img", "alpha_plane", "depth_plane")})
         ctx.shapes = [t.shape for t in (pos, scale, rotq, sh, opacity)]
+        ctx.pose_like = _pose_like(view, cam_pos)
         return img, alpha, depth
 
     @staticmethod
     def backward(ctx, dl_dimg, dl_dalpha, dl_ddepth):
-        want = ctx.needs_input_grad[2:]
+        want = ctx.needs_input_grad[2:7]
         scene, b = ctx.saved
         img, alpha, depth = ctx.saved_tensors
         b = dict(b, img=img, alpha_plane=alpha, depth_plane=depth)
         if dl_dimg is None:
             dl_dimg = torch.zeros_like(img)
-        grads = ctx.dr._backward(ctx.vp, (scene, b), dl_dimg, want, dl_dalpha, dl_ddepth)
+        grads, pose = ctx.dr._backward(ctx.vp, (scene, b), dl_dimg, want, dl_dalpha, dl_ddepth,
+                                       pose_want=_pose_want(ctx))
         ctx.saved = None
         out = [g.view(s) if g is not None else None for g, s in zip(grads, ctx.shapes)]
-        return (None, None, *out)
+        return (None, None, *out, *_pose_grads(ctx, pose))
 
 
 class DifferentiableRenderer:
@@ -677,7 +702,16 @@ class DifferentiableRenderer:
     aux: the call returns `(img [3, H, W], alpha [H, W], depth [H, W])`, the planes of `Renderer(aux=True)`:
     accumulated opacity 1 - T and the sum of weight * view depth over the blended Gaussians (not normalised; the
     expected depth is `depth / alpha` where alpha > 0, ordinary torch code).  All three are differentiable, so mask,
-    depth and opacity losses train the scene; the image is bit-identical to the one without aux."""
+    depth and opacity losses train the scene; the image is bit-identical to the one without aux.
+
+    Camera pose: `dr(..., cam, world_to_camera=M)` renders with the [4, 4] tensor M (p_cam = M[:3, :3] @ p + M[:3, 3];
+    row 3 is ignored) in place of the camera's view matrix, `cam` still giving the resolution and the field of view,
+    and M receives dL/dM (the gradient of the EWA Jacobian's rows and of the projected means; the fov and focal
+    lengths are held fixed).  `camera_position` (a [3] tensor) is the point the SH view directions start from; it
+    defaults to the camera centre of M, -M[:3, :3]^-1 M[:3, 3], computed in torch so that its gradient reaches M too.
+    `world_to_camera(cam)` gives the camera's own M.  Without either argument the call is exactly the plain one.
+    The scene tensors may all be frozen (camera tracking against a fixed scene): the backward then computes the pose
+    gradient only."""
 
     def __init__(self, device: Device, width: int, height: int, list_capacity: int = 4_000_000, sh_deg: int = 3,
                  bg_color=(0.0, 0.0, 0.0), scale_modifier: float = 1.0, keep_means_2d_grad: bool = False,
@@ -698,9 +732,25 @@ class DifferentiableRenderer:
         self.keys = torch.zeros(self.capacity, dtype=torch.int64, device=dev)
         self._reserved = -1
 
-    def __call__(self, pos, scale, rotq, sh, opacity, cam: Camera):
+    def __call__(self, pos, scale, rotq, sh, opacity, cam: Camera, world_to_camera: Optional[torch.Tensor] = None,
+                 camera_position: Optional[torch.Tensor] = None):
         fn = _RenderAuxFunction if self.aux else _RenderFunction
-        return fn.apply(self, view_params(cam), pos, scale, rotq, sh, opacity)
+        vp = view_params(cam)
+        if world_to_camera is None and camera_position is None:
+            return fn.apply(self, vp, pos, scale, rotq, sh, opacity)
+        if world_to_camera is not None:
+            assert tuple(world_to_camera.shape) == (4, 4), "world_to_camera must be [4, 4]"
+            M = world_to_camera
+            if camera_position is None:
+                camera_position = -torch.linalg.solve(M[:3, :3], M[:3, 3])
+            m = M.detach().to(device="cpu", dtype=torch.float32)
+            for c in range(4):  # vp.view is column-major; its row 3 stays the camera's
+                for r in range(3):
+                    vp.view[c * 4 + r] = float(m[r, c])
+        if camera_position is not None:
+            assert tuple(camera_position.shape) == (3,), "camera_position must be [3]"
+            vp.cam_pos[:] = [float(x) for x in camera_position.detach().to(device="cpu", dtype=torch.float32)]
+        return fn.apply(self, vp, pos, scale, rotq, sh, opacity, world_to_camera, camera_position)
 
     def _scene(self, pos, scale, rotq, sh, opacity, alpha_consts) -> _capi.Scene:
         P = int(pos.shape[0])
@@ -748,7 +798,9 @@ class DifferentiableRenderer:
         d.num_rendered()  # raises CapacityError on overflow
         return b["img"].view(3, self.H, self.W), (scene, b)
 
-    def _backward(self, vp: ViewParams, saved, dl_dimg: torch.Tensor, want, dl_dalpha=None, dl_ddepth=None) -> list:
+    def _backward(self, vp: ViewParams, saved, dl_dimg: torch.Tensor, want, dl_dalpha=None, dl_ddepth=None,
+                  pose_want=(False, False)):
+        """(the five scene gradients or None, (dL/d world_to_camera [4, 4] or None, dL/d camera_position [3] or None))"""
         d = self.device
         scene, b = saved
         P = int(scene[0].shape[0])
@@ -761,10 +813,13 @@ class DifferentiableRenderer:
         g.grad_pos, g.grad_scale, g.grad_rotq, g.grad_sh, g.grad_opacity = (_ptr(t) for t in grads)
         m2 = torch.empty((P, 2), dtype=torch.float32, device=dl.device) if self.keep_means_2d_grad else None
         g.grad_means_2d = _ptr(m2)
+        gv = torch.empty(16, dtype=torch.float32, device=dl.device) if pose_want[0] else None
+        gc = torch.empty(3, dtype=torch.float32, device=dl.device) if pose_want[1] else None
+        g.grad_view, g.grad_cam_pos = _ptr(gv), _ptr(gc)
         c_scene = self._scene(*scene, b["alpha_consts"])
         f = self._frame(b)
         d.check(d.lib.lcgs_b200_render_backward(d.ctx, C.byref(c_scene), C.byref(vp), C.byref(f), C.byref(g),
                                                 _stream_handle(None)))
         if self.keep_means_2d_grad:
             self.means_2d_grad = m2
-        return grads
+        return grads, (None if gv is None else gv.view(4, 4).T, gc)
