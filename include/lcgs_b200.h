@@ -322,6 +322,18 @@ LCGS_B200_API int lcgs_b200_render_backward(lcgs_b200_ctx* ctx, const lcgs_b200_
                                             const lcgs_b200_view_params* vp, const lcgs_b200_frame* frame,
                                             const lcgs_b200_grad* grad, lcgs_b200_stream stream);
 
+/* SSIM of a planar image against a reference, and optionally its gradient (no reference counterpart: the reference
+ * renders only; semantics: the 3DGS training loss's ssim(), see DESIGN).  img, ref: [3][H][W] float32, the layout of
+ * target_img.  ssim: device float [1], overwritten with the mean SSIM.  dssim_dimg: optional [3][H][W], overwritten
+ * with d(mean SSIM)/d(img), ready to be scaled into lcgs_b200_grad::dl_dimg.  All 4-byte aligned.  Enqueue only,
+ * except workspace growth on the first call at a larger size; bit-reproducible.
+ *   Window: 11 taps, sigma 1.5, applied separably per channel with zero padding of 5 (pixels outside the image are 0
+ *   in every moment); C1 = 0.01^2, C2 = 0.03^2; the mean over the 3 H W channel pixels.  The reference image is a
+ *   constant: there is no gradient with respect to it.  LCGS_B200_ERR_INVALID (nothing written) for a NULL img, ref
+ *   or ssim, a width or height <= 0, or a misaligned pointer. */
+LCGS_B200_API int lcgs_b200_ssim(lcgs_b200_ctx* ctx, int width, int height, const float* img, const float* ref,
+                                 float* ssim, float* dssim_dimg, lcgs_b200_stream stream);
+
 /* The value GSTileSplatter::forward returns (impl.cpp:179): synchronises `stream` (the one the
  * last whole-frame call was enqueued on) and stores that frame's num_rendered.  Returns LCGS_B200_ERR_CAPACITY if it exceeded
  * list_capacity (the frame's image is then incomplete).  The comparison is made ON THE DEVICE by the

@@ -101,6 +101,7 @@ _PROTOS = {
     "lcgs_b200_splat_forward": (_I, [_VP, _I, _VP, C.POINTER(Frame), _VP]),
     "lcgs_b200_render": (_I, [_VP, C.POINTER(Scene), C.POINTER(ViewParams), C.POINTER(Frame), _VP]),
     "lcgs_b200_render_backward": (_I, [_VP, C.POINTER(Scene), C.POINTER(ViewParams), C.POINTER(Frame), C.POINTER(Grad), _VP]),
+    "lcgs_b200_ssim": (_I, [_VP, _I, _I, _VP, _VP, _VP, _VP, _VP]),
     "lcgs_b200_num_rendered": (_I, [_VP, _VP, C.POINTER(_I)]),
     "lcgs_b200_read_num_rendered_async": (_I, [_VP, _VP, _VP]),
     "lcgs_b200_read_image": (_I, [_VP, C.POINTER(Frame), _VP, _VP]),

@@ -22,8 +22,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 BUILD = os.path.join(CSRC, "build")
 LIB = os.path.join(HERE, "liblcgs_b200.so")
-SOURCES = ["capi.cu", "preprocess.cu", "scan.cu", "binning.cu", "sort.cu", "blend.cu", "backward.cu"]
-HEADERS = ["common.cuh", "frame_plan.cuh", "lcgs_math.cuh", "lcgs_grad.cuh", "lookback.cuh", "blend_walk.cuh", os.path.join("..", "..", "include", "lcgs_b200.h")]
+SOURCES = ["capi.cu", "preprocess.cu", "scan.cu", "binning.cu", "sort.cu", "blend.cu", "backward.cu", "ssim.cu"]
+HEADERS = ["common.cuh", "frame_plan.cuh", "lcgs_math.cuh", "lcgs_grad.cuh", "lookback.cuh", "blend_walk.cuh", "ssim_math.cuh", os.path.join("..", "..", "include", "lcgs_b200.h")]
 
 NVCC = os.environ.get("LCGS_NVCC", "/usr/local/cuda/bin/nvcc")
 NVCC_FLAGS = [

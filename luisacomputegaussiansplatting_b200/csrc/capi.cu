@@ -279,6 +279,7 @@ int lcgs_b200_ctx_destroy(lcgs_b200_ctx* ctx)
     if (ctx->emit_ws.ptr) cudaFree(ctx->emit_ws.ptr);
     if (ctx->grad_ws.ptr) cudaFree(ctx->grad_ws.ptr);
     if (ctx->pose_ws.ptr) cudaFree(ctx->pose_ws.ptr);
+    if (ctx->ssim_ws.ptr) cudaFree(ctx->ssim_ws.ptr);
     for (int i = 0; i < 16; i++)
         if (ctx->ev[i]) cudaEventDestroy(ctx->ev[i]);
     for (int i = 0; i < 3; i++)
@@ -599,6 +600,20 @@ int lcgs_b200_render_backward(lcgs_b200_ctx* ctx, const lcgs_b200_scene* sc, con
     LCGS_REQUIRE(ctx, aligned(gr->grad_view, 4) && aligned(gr->grad_cam_pos, 4),
                  "render_backward: grad_view / grad_cam_pos must be 4-byte aligned");
     return launch_render_backward(ctx, sc, vp, fr, gr, as_stream(stream));
+}
+
+int lcgs_b200_ssim(lcgs_b200_ctx* ctx, int width, int height, const float* img, const float* ref, float* ssim,
+                   float* dssim_dimg, lcgs_b200_stream stream)
+{
+    int rc = enter(ctx);
+    if (rc) return rc;
+    LCGS_REQUIRE(ctx, img && ref && ssim, "ssim: null img / ref / ssim");
+    LCGS_REQUIRE(ctx, width > 0 && height > 0, "ssim: width and height must be positive");
+    LCGS_REQUIRE(ctx, ((size_t)width + 31) / 32 * (((size_t)height + 31) / 32) <= 0x7fffffffu / 3,
+                 "ssim: image too large");
+    LCGS_REQUIRE(ctx, aligned(img, 4) && aligned(ref, 4) && aligned(ssim, 4) && aligned(dssim_dimg, 4),
+                 "ssim: buffers must be 4-byte aligned");
+    return launch_ssim(ctx, width, height, img, ref, ssim, dssim_dimg, as_stream(stream));
 }
 
 int lcgs_b200_num_rendered(lcgs_b200_ctx* ctx, lcgs_b200_stream stream, int* num_rendered)

@@ -55,6 +55,7 @@ struct lcgs_b200_ctx {
     lcgs_b200::Workspace emit_ws;        // emission: entries + pieces of the Gaussians expanded by emit_big_kernel
     lcgs_b200::Workspace grad_ws;        // backward: packed per-Gaussian gradient of the blend's inputs [P][12]
     lcgs_b200::Workspace pose_ws;        // backward: per-CTA partial sums of the pose gradient [15][CTAs] (double)
+    lcgs_b200::Workspace ssim_ws;        // ssim: partial maps [3][3][H][W] (with the gradient) + per-CTA sums (double)
     // per-stage timing
     int          profiling  = 0;
     cudaEvent_t  ev[16];
@@ -156,6 +157,9 @@ int launch_tile_order(lcgs_b200_ctx* ctx, const uint32_t* ranges, int num_tiles,
 // lcgs_b200_render_backward of a whole frame (backward.cu); arguments checked by the caller
 int launch_render_backward(lcgs_b200_ctx* ctx, const lcgs_b200_scene* sc, const lcgs_b200_view_params* vp,
                            const lcgs_b200_frame* fr, const lcgs_b200_grad* gr, cudaStream_t s);
+// lcgs_b200_ssim (ssim.cu); arguments checked by the caller, grad may be null
+int launch_ssim(lcgs_b200_ctx* ctx, int W, int H, const float* img, const float* ref, float* ssim, float* grad,
+                cudaStream_t s);
 int launch_peer_signal(lcgs_b200_ctx* ctx, uint32_t* flag, uint32_t value, cudaStream_t s);
 int launch_peer_wait(lcgs_b200_ctx* ctx, const uint32_t* flag, uint32_t value, uint32_t timeout_ms, cudaStream_t s);
 int launch_checksum_u32(lcgs_b200_ctx* ctx, const void* data, size_t num_words, uint64_t* out, cudaStream_t s);

@@ -823,3 +823,45 @@ class DifferentiableRenderer:
         if self.keep_means_2d_grad:
             self.means_2d_grad = m2
         return grads, (None if gv is None else gv.view(4, 4).T, gc)
+
+
+# --------------------------------------------------------------------------------------------------
+# SSIM loss (extension: no reference counterpart)
+# --------------------------------------------------------------------------------------------------
+
+class _SSIMFunction(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, device: Device, img, ref):
+        H, W = int(img.shape[1]), int(img.shape[2])
+        x = img.detach().contiguous()
+        y = ref.detach().contiguous()
+        out = torch.empty((), dtype=torch.float32, device=x.device)
+        grad = torch.empty_like(x) if ctx.needs_input_grad[1] else None
+        device.check(device.lib.lcgs_b200_ssim(device.ctx, W, H, _ptr(x), _ptr(y), _ptr(out), _ptr(grad),
+                                               _stream_handle(None)))
+        if grad is not None:
+            ctx.save_for_backward(grad)
+        return out
+
+    @staticmethod
+    def backward(ctx, grad_output):
+        (grad,) = ctx.saved_tensors
+        return None, grad_output * grad, None
+
+
+def ssim(device: Device, img: torch.Tensor, ref: torch.Tensor) -> torch.Tensor:
+    """Mean SSIM of the planar image `img` against the reference `ref` (both [3, H, W] float32 on `device`), a 0-dim
+    tensor, as in the 3DGS training loss: an 11-tap Gaussian window of sigma 1.5 per channel with zero padding,
+    C1 = 0.01^2, C2 = 0.03^2.  Differentiable with respect to `img` (lcgs_b200_ssim's CUDA kernels compute the value
+    and the gradient map in one call, no atomics: both are bit-reproducible); `ref` is a constant of the loss and must
+    not require grad, so that no gradient is silently dropped.  The usual loss is
+    `0.8 * (img - ref).abs().mean() + 0.2 * (1 - ssim(dev, img, ref))`."""
+    if ref.requires_grad:
+        raise ValueError("ssim: ref must not require grad (there is no gradient with respect to the reference)")
+    if img.dim() != 3 or img.shape[0] != 3 or tuple(img.shape) != tuple(ref.shape):
+        raise ValueError("ssim: img and ref must both be [3, H, W], got %s and %s" % (tuple(img.shape), tuple(ref.shape)))
+    if img.dtype != torch.float32 or ref.dtype != torch.float32:
+        raise ValueError("ssim: img and ref must be float32")
+    if img.device != device.torch_device or ref.device != device.torch_device:
+        raise ValueError("ssim: img and ref must be on the device's GPU")
+    return _SSIMFunction.apply(device, img, ref)
